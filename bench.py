@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload play_lmp|tacorl|play_lmp_multiview|tacorl_multiview]
                     [--precision bf16|fp32] [--scaling weak|strong] [--batch 64] [--global-batch 512]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): train frames/sec.  A step = one optimiser step (forward + backward + gradient all-reduce +
 Adam[s]) on a synthetic CALVIN-shaped batch of windows x 16 frames of 3x200x200 per GPU.  The headline line is the
@@ -49,6 +50,8 @@ ENC_NCU_TRAFFIC_BYTES = 2.887e9
 PLAYLMP_FLOP_PER_WINDOW = 8.97e9        # BiRNN recogniser, 16 x 200x200 frames
 TACORL_FLOP_PER_WINDOW = 5.89e9         # 27 encoder fwd + 6 bwd frames, PR fwd, decoder fwd+bwd, MLPs
 RNN_H = 2048
+DUMP_SAMPLE = 32768                 # --dump-outputs: elements kept per tensor
+DUMP_MAX_BYTES = 64 << 20
 
 
 def parse():
@@ -75,7 +78,40 @@ def parse():
     ap.add_argument("--no-gpu-eager", action="store_true", help="reference arm: skip the torch-eager-on-GPU timings")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
     ap.add_argument("--cpu-steps", type=int, default=3, help="timed steps of the cpu_baseline leg of our own line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps of the headline workload, write what its last step computed as "
+                         "DIR/<name>.npy (float32): the returned loss, the logged scalars, every floating-point "
+                         "state_dict entry after the update and every parameter's gradient; a tensor of more than "
+                         f"{DUMP_SAMPLE} elements is stored as a fixed, seeded sample of its flattened elements")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, loss, module, opts):
+    """Writes the outputs of the last timed step (see --dump-outputs).  Inputs, initial weights and noise are seeded, so
+    two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    names = {id(p): n for n, p in module.named_parameters()}
+    arrays = {"loss": loss}
+    arrays.update({"logged." + k.replace("/", "."): v for k, v in module.logged.items() if torch.is_tensor(v)})
+    arrays.update({"state." + k: v for k, v in module.state_dict().items() if v.dtype.is_floating_point})
+    for o in opts:
+        for p, g in zip(o.param_groups[0]["params"], o.grad_views):
+            arrays["grad." + names[id(p)]] = g
+    total = sum(4 * min(t.numel(), DUMP_SAMPLE) for t in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE]
+            a = a.reshape(-1)[idx.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def peaks():
@@ -322,8 +358,9 @@ class Ctx:
         return float(ms)
 
 
-def measure_workload(ctx, name, precision, steps, warmup, e2e=True, sample_clocks=False):
-    """Resident and end-to-end timing of one workload.  Returns (result dict, handles for the roofline probes)."""
+def measure_workload(ctx, name, precision, steps, warmup, e2e=True, sample_clocks=False, dump_dir=None):
+    """Resident and end-to-end timing of one workload.  Returns (result dict, handles for the roofline probes).
+    dump_dir: rank 0 writes the outputs of the last resident timed step there (dump_outputs)."""
     from tacorl_b200 import _lib, runtime
     args, dev, world, rank = ctx.args, ctx.dev, ctx.world, ctx.rank
     wl = WORKLOADS[name]
@@ -337,8 +374,10 @@ def measure_workload(ctx, name, precision, steps, warmup, e2e=True, sample_clock
         graphed = runtime.GraphedTrainStep(eager_step, resident, device=dev, warmup=3, buffers=2)
         ctx.graphs.append(graphed)
 
+    last = [None]
+
     def step(_s):
-        return graphed() if graphed is not None else eager_step(resident)
+        last[0] = graphed() if graphed is not None else eager_step(resident)
 
     for s in range(warmup):
         step(s)
@@ -361,6 +400,8 @@ def measure_workload(ctx, name, precision, steps, warmup, e2e=True, sample_clock
     if clk is not None:
         res["clocks"] = clk
     trace(f"{name}/{precision}: resident {ms:.3f} ms/step")
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, last[0], m, opts)
     if ctx.args.timeline and graphed is not None and name == ctx.args.workload:
         from torch.profiler import ProfilerActivity, profile
         ctx.barrier()
@@ -770,7 +811,8 @@ def run_ours(args):
     B = windows_per_gpu(args, world)
     wl = WORKLOADS[args.workload]
 
-    main, h = measure_workload(ctx, args.workload, args.precision, args.steps, args.warmup, sample_clocks=True)
+    main, h = measure_workload(ctx, args.workload, args.precision, args.steps, args.warmup, sample_clocks=True,
+                               dump_dir=args.dump_outputs)
     rooflines = []
     if "rgb_static" in wl["mods"] and args.precision == "bf16" and wl["module"] != "cql":
         try:

@@ -24,7 +24,16 @@ def test_shared_library_exports_every_declared_symbol():
     assert not missing, missing
     assert declared == set(_lib.EXPORTED), declared ^ set(_lib.EXPORTED)
     assert _lib.lib().tacorl_abi_version() == 7
-    assert _lib.launch_count() == 0          # nothing may have launched on a CPU-only box
+    if not torch.cuda.is_available():        # with a GPU, the GPU tests earlier in the session have launched kernels
+        assert _lib.launch_count() == 0      # nothing may have launched on a CPU-only box
+    # the same in a fresh process that sees no device, on every machine: loading the package and refusing CPU tensors
+    # launches nothing
+    code = ("import torch; from tacorl_b200 import _lib, ops\n"
+            "try:\n    ops.linear(torch.randn(2, 3), torch.randn(4, 3), torch.randn(4))\n"
+            "except _lib.TacorlLibraryError:\n    print('LAUNCHES', _lib.launch_count())\n")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=ROOT,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 0 and "LAUNCHES 0" in out.stdout, (out.stdout, out.stderr[-1500:])
 
 
 def test_ops_fail_loudly_without_cuda_tensors():
@@ -210,6 +219,44 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert other.returncode == 0 and other.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_writes_every_output_of_the_step_reproducibly(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: loss, logged scalars, every floating-point state_dict entry and every gradient as float32
+    .npy; tensors above the sample size become the same seeded sample on every call (CPU: no kernels run)."""
+    import numpy as np
+    import bench
+    from tacorl_b200 import configs
+    from tacorl_b200.utils import synthetic
+    from tacorl_b200.utils.config import instantiate
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    m = instantiate(configs.play_lmp_for_rl("tanh_net", rnn_hidden=64))
+    synthetic.init_like_reference(m, seed=0)
+    opt = m.configure_optimizers()
+    opt.flat_grad.copy_(torch.arange(opt.flat_grad.numel(), dtype=torch.float32))
+    m.logged = {"train/total_loss": torch.tensor(0.5), "train/epoch": 3}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor(1.25), m, [opt])
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(os.listdir(tmp_path / "b"))
+    sd = m.state_dict()
+    want = {"loss.npy", "logged.train.total_loss.npy"} | {f"state.{k}.npy" for k in sd} | \
+           {f"grad.{n}.npy" for n, p in m.named_parameters() if p.requires_grad}
+    assert set(files) == want
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b), f
+    assert float(np.load(tmp_path / "a" / "loss.npy")) == 1.25
+    big = max(sd, key=lambda k: sd[k].numel())
+    got = np.load(tmp_path / "a" / f"state.{big}.npy")
+    assert sd[big].numel() > 1000 and got.shape == (1000,)
+    assert np.isin(got, sd[big].reshape(-1).numpy()).all()
+    small = min(sd, key=lambda k: sd[k].numel())
+    assert np.array_equal(np.load(tmp_path / "a" / f"state.{small}.npy"), sd[small].numpy())
+    g0 = opt.grad_views[0]
+    name0 = [n for n, p in m.named_parameters() if p is opt.param_groups[0]["params"][0]][0]
+    got = np.load(tmp_path / "a" / f"grad.{name0}.npy")
+    assert got.size == min(g0.numel(), 1000) and np.isin(got, g0.reshape(-1).numpy()).all()
+
+
 def test_vendored_reference_tree_is_importable_without_the_source_checkout():
     """oracle/vendor_reference.py copies the pure-Python reference package to oracle/_ref (git-ignored, travels to the
     GPU box); the loader must work from that tree alone, as it has to on the box."""
@@ -322,60 +369,67 @@ def test_reference_lightning_checkpoint_resumes_in_the_b200_modules(tmp_path):
     """A run directory as the reference leaves it (`.hydra/config.yaml` with the reference `_target_`, a Lightning-format
     `.ckpt` holding the reference module's state_dict and its torch.optim.Adam state) is picked up by the B200 loader:
     class path remapped, weights identical, Adam moments / step restored into FlatAdam (utils/networks.py:90-117,
-    scripts/train.py:48-66).  CPU only: no kernel runs."""
+    scripts/train.py:48-66).  The reference's layout comes from the golden recorded from it: state_dict keys, order and
+    shapes, and its parameters in named_parameters() order (the gradients it recorded) -- the list its
+    torch.optim.Adam (play_lmp_for_rl.py:362-368) numbers.  CPU only: no kernel runs."""
     import yaml
-    from oracle import ref_loader as R
     from oracle import ref_loader_cfg as RC
     from oracle import synth as S
-    if not R.reference_available():
-        pytest.skip("reference not present")
-    ref = R.build_reference_play_lmp(pr_kind="tanh_net", rnn_hidden=32, dropout_p=0.0, max_window=8)
-    opt = ref.configure_optimizers()
-    batch = S.synth_play_batch(2, 8, 84, 84, 3)
-    for s in range(2):
-        torch.manual_seed(10 + s)
-        opt.zero_grad()
-        ref.training_step(S.clone_batch(batch), s).backward()
+    rec = json.load(open(os.path.join(GOLD, "playlmp_birnn_84.json")))
+    assert rec["pr_kind"] == "tanh_net" and rec["modalities"] == ["rgb_static"]
+    ref_sd = S.synth_state_dict(rec["shapes"], 3)
+    assert list(ref_sd) == list(rec["shapes"])
+    ref_names = list(rec["steps"][0]["grads"])
+    ref_params = [torch.nn.Parameter(ref_sd[k].clone()) for k in ref_names]
+    cfg = RC.play_lmp_cfg(pr_kind="tanh_net", rnn_hidden=rec["rnn_hidden"], dropout_p=0.0, max_window=rec["T"])
+    opt = torch.optim.Adam(ref_params, lr=cfg["lr"])
+    g = torch.Generator().manual_seed(10)
+    for _ in range(2):
+        for p in ref_params:
+            p.grad = torch.randn(p.shape, generator=g)
         opt.step()
+    for k, p in zip(ref_names, ref_params):
+        ref_sd[k] = p.detach().clone()
     run = tmp_path / "run"
     (run / ".hydra").mkdir(parents=True)
     (run / "saved_models").mkdir()
-    cfg = RC.play_lmp_cfg(pr_kind="tanh_net", rnn_hidden=32, dropout_p=0.0, max_window=8)
     cfg["_target_"] = "tacorl.modules.play_lmp.play_lmp_for_rl.PlayLMP"
     cfg["_recursive_"] = False
     yaml.safe_dump({"module": cfg}, open(run / ".hydra" / "config.yaml", "w"))
-    torch.save({"epoch": 3, "global_step": 2, "pytorch-lightning_version": "1.6.5", "state_dict": ref.state_dict(),
+    torch.save({"epoch": 3, "global_step": 2, "pytorch-lightning_version": "1.6.5", "state_dict": ref_sd,
                 "optimizer_states": [opt.state_dict()], "lr_schedulers": []}, run / "saved_models" / "tacorl_epoch_03_.ckpt")
     from tacorl_b200 import trainer as TR
     from tacorl_b200.modules.play_lmp.play_lmp_for_rl import PlayLMP
     from tacorl_b200.utils.networks import get_checkpoint_i_from_dir, load_pl_module_from_checkpoint
     m = load_pl_module_from_checkpoint(run, epoch=3)
     assert type(m) is PlayLMP
-    for k, v in ref.state_dict().items():
+    for k, v in ref_sd.items():
         assert torch.equal(m.state_dict()[k], v), k
     ckpt = TR.restore_checkpoint(m, get_checkpoint_i_from_dir(run, 3))
     assert ckpt["global_step"] == 2 and m.current_epoch == 3
     o = m.optimizers()[0]
     assert o.step_count == 2
-    ref_params = [p for p in ref.parameters() if p.requires_grad]
     mine = o.param_groups[0]["params"]
     assert len(ref_params) == len(mine)
     for i, (rp, off) in enumerate(zip(ref_params, o.pbuf.offsets)):
-        st = opt.state.get(rp)
-        if not st:
-            continue
+        st = opt.state[rp]
         assert torch.equal(o.exp_avg[off:off + rp.numel()].view(rp.shape), st["exp_avg"]), i
         assert torch.equal(o.exp_avg_sq[off:off + rp.numel()].view(rp.shape), st["exp_avg_sq"]), i
     # and back: a checkpoint written by this package has the layout the reference's Lightning run expects
     out = TR.save_checkpoint(m, tmp_path / "out" / "last.ckpt", epoch=4, global_step=7)
     back = torch.load(out, weights_only=False)
     assert set(back) >= {"epoch", "global_step", "state_dict", "optimizer_states", "pytorch-lightning_version"}
-    ref2 = R.build_reference_play_lmp(pr_kind="tanh_net", rnn_hidden=32, dropout_p=0.0, max_window=8)
-    ref2.load_state_dict(back["state_dict"], strict=True)
-    opt2 = ref2.configure_optimizers()
+    assert [(k, list(v.shape)) for k, v in back["state_dict"].items()] == list(rec["shapes"].items())
+    for k, v in ref_sd.items():
+        assert torch.equal(back["state_dict"][k], v), k
+    rp2 = [torch.nn.Parameter(ref_sd[k].clone()) for k in ref_names]
+    opt2 = torch.optim.Adam(rp2, lr=1.0)
     opt2.load_state_dict(back["optimizer_states"][0])
-    rp2 = [p for p in ref2.parameters() if p.requires_grad]
-    assert float(opt2.state[rp2[0]]["step"]) == 2.0
+    assert opt2.param_groups[0]["lr"] == cfg["lr"]
+    for p, rp in zip(rp2, ref_params):
+        assert float(opt2.state[p]["step"]) == 2.0
+        assert torch.equal(opt2.state[p]["exp_avg"], opt.state[rp]["exp_avg"])
+        assert torch.equal(opt2.state[p]["exp_avg_sq"], opt.state[rp]["exp_avg_sq"])
 
 
 def test_launch_side_helpers_numa_and_channel_choice(monkeypatch):
