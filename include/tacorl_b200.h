@@ -273,6 +273,57 @@ int tacorl_actions_gather_pad(const float* store, long long frames, int A, const
 int tacorl_color_jitter_u8(const unsigned char* x, long long N, int H, int W, const int* order, const float* factors,
                            float norm_mean, float norm_std, float* mean_ws, float* out, void* stream);
 
+/* ---- HBM-resident replay (tacorl_b200/replay.py; sampling rules: DESIGN.md section 13).  A step's batch is drawn and
+ * assembled on the device by two graph-capturable launches; nothing is allocated and nothing crosses PCIe.
+ * replay_sample: ONE CTA.  Reads *step_dev, draws with Philox4x32-10 (key = (lo32(seed), hi32(seed) ^ rank * 0x9E3779B9),
+ *   counter = (lo32(step), hi32(step), sample, draw id)), writes the tables and stores *step_dev + 1.
+ *   kind 0 PlayLMP, 1 TACO-RL, 2 flat CQL.  valid: start frames (kinds 0/1: >= min_window frames left in the episode;
+ *   kind 2: frames with a successor in their episode), n_valid entries.  geom_thr: n_geom non-decreasing thresholds of
+ *   Geometric(p) on {1, 2, ...}: thr[k] = floor(2^32 P(d <= k + 1)).  neg_thr: TACO-RL negative goal iff u < neg_thr.
+ *   tab  (4, B) int32: start | window | goal | disp  (kind 2: frame i | 1 | goal | reward);
+ *   out64 (3, B) int64: idx | window_size | disp     (kind 2: rewards | terminals | goal);
+ *   shift (n_mod, B, n_slots, 2) int32 in [0, 2 pad], or NULL for no RandomShiftsAug.
+ *   jitter (optional, NULL = none): ColorJitter of every output frame: jit_order (n_mod, B, n_slots) int32 packed op
+ *   order as tacorl_color_jitter_u8 takes it (a uniform order of the ops enabled in jitter->ops, bit 0 brightness,
+ *   1 contrast, 3 hue), jit_factors (n_mod, B, n_slots, 3) fp32 = lo[i] + span[i] * (u >> 8) * 2^-24 per enabled op
+ *   (1, 1, 0 for disabled ones).  Negative goal iff u < neg_thr (neg_thr = 2^32: always).
+ *   Every index table must hold only in-range frame ids: the host validates them before upload.
+ * replay_gather: ONE launch for every image output of the batch plus the action rows.  images[i].out is
+ *   (B, T, 3, H, W) for TACORL_REPLAY_WINDOW (pad_sequence by repetition), else (B, 3, H, W) with the frame
+ *   start (OBS), start + 1 (NEXT) or goal (GOAL) of `tab`; each frame is shifted by its slot shift_slot (+ t) of the
+ *   modality's shift table (NULL = none), like tacorl_window_gather_u8.
+ * replay_color_jitter: ScaleImageTensor -> ColorJitter -> Normalize of B x nf uint8 frames (the uint8 output of a
+ *   gather) into fp32, frame (b, t) taking entry b * n_slots + slot0 + t of the sampler's jitter tables of its modality.
+ *   mean_ws: B * nf floats.  Two launches (contrast mean, apply), the kernels of tacorl_color_jitter_u8.  act_out: (B, T, A) rows of act_store windowed
+ *   like tacorl_actions_gather_pad (act_role WINDOW) or (B, A) (act_role OBS); NULL = no actions. */
+#define TACORL_REPLAY_MAX_IMAGES 8
+#define TACORL_REPLAY_WINDOW 0
+#define TACORL_REPLAY_OBS 1
+#define TACORL_REPLAY_NEXT 2
+#define TACORL_REPLAY_GOAL 3
+typedef struct tacorl_replay_image {
+  const unsigned char* store;   /* (frames, 3, H, W) uint8 */
+  unsigned char* out;
+  const int* shift;             /* (B, n_slots, 2) shift table of this modality, or NULL */
+  int H; int W;                 /* W % 4 == 0 */
+  int role;                     /* TACORL_REPLAY_* */
+  int shift_slot; int n_slots;
+} tacorl_replay_image;
+typedef struct tacorl_replay_jitter {
+  int ops;                      /* bit 0 brightness, bit 1 contrast, bit 3 hue */
+  float lo[3]; float span[3];   /* factor ranges of brightness, contrast, hue */
+} tacorl_replay_jitter;
+int tacorl_replay_sample(int kind, int B, int min_window, int max_window, int n_mod, int n_slots, int pad,
+                         unsigned long long neg_thr, unsigned long long seed, int rank, long long* step_dev,
+                         const int* ep_end, long long frames, const int* valid, long long n_valid,
+                         const unsigned* geom_thr, int n_geom, int* tab, int* shift, long long* out64,
+                         const tacorl_replay_jitter* jitter, int* jit_order, float* jit_factors, void* stream);
+int tacorl_replay_gather(int B, int T, int pad, const int* tab, int n_images, const tacorl_replay_image* images,
+                         const float* act_store, int A, int act_role, int zero_pad, float* act_out, void* stream);
+int tacorl_replay_color_jitter(const unsigned char* x, int B, int nf, int H, int W, const int* order,
+                               const float* factors, int n_slots, int slot0, float norm_mean, float norm_std,
+                               float* mean_ws, float* out, void* stream);
+
 /* ---- fused small-MLP chains (fp32): a whole Linear -> act -> Linear ... stack in ONE launch, forward or backward.
  * Replaces the per-layer launches behind VisualGoalEncoder.forward (goal_encoder.py:29-33), MLPPolicy.forward
  * (actor.py:252-270: 3 x Linear+SiLU, then fc_mean | fc_log_std as ONE layer of two weight segments) and

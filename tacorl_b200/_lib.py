@@ -76,6 +76,10 @@ _SIGS = {
     "tacorl_window_gather_u8": [_vp, _ll, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tacorl_actions_gather_pad": [_vp, _ll, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tacorl_color_jitter_u8": [_vp, _ll, _i, _i, _vp, _vp, _f, _f, _vp, _vp, _vp],
+    "tacorl_replay_sample": [_i, _i, _i, _i, _i, _i, _i, ctypes.c_ulonglong, ctypes.c_ulonglong, _i, _vp, _vp, _ll, _vp,
+                             _ll, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tacorl_replay_gather": [_i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "tacorl_replay_color_jitter": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _f, _f, _vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],
     "tacorl_mlp_chain_fwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp],
     "tacorl_mlp_chain_bwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _sz, _vp],
@@ -108,6 +112,21 @@ class MlpLayer(ctypes.Structure):
     _fields_ = [("W0", _vp), ("b0", _vp), ("n0", _i), ("W1", _vp), ("b1", _vp), ("n1", _i),
                 ("W2", _vp), ("b2", _vp), ("n2", _i), ("in_", _i), ("act", _i),
                 ("dW0", _vp), ("db0", _vp), ("dW1", _vp), ("db1", _vp), ("dW2", _vp), ("db2", _vp)]
+
+
+class ReplayImage(ctypes.Structure):
+    """tacorl_replay_image (include/tacorl_b200.h)."""
+    _fields_ = [("store", _vp), ("out", _vp), ("shift", _vp), ("H", _i), ("W", _i), ("role", _i),
+                ("shift_slot", _i), ("n_slots", _i)]
+
+
+class ReplayJitter(ctypes.Structure):
+    """tacorl_replay_jitter (include/tacorl_b200.h)."""
+    _fields_ = [("ops", _i), ("lo", _f * 3), ("span", _f * 3)]
+
+
+REPLAY_WINDOW, REPLAY_OBS, REPLAY_NEXT, REPLAY_GOAL = 0, 1, 2, 3
+REPLAY_MAX_IMAGES = 8
 
 
 def lib():

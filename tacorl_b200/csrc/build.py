@@ -5,7 +5,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIBDIR = os.path.join(os.path.dirname(HERE), "lib")
-SOURCES = ["api.cu", "gemm_f32.cu", "gemm_tc.cu", "conv_tc.cu", "conv_f32.cu", "encoder.cu", "rnn.cu", "losses.cu", "optim.cu", "cql.cu", "transformer.cu", "mlp_chain.cu", "data_pipeline.cu", "dp_nccl.cu", "gripper.cu"]
+SOURCES = ["api.cu", "gemm_f32.cu", "gemm_tc.cu", "conv_tc.cu", "conv_f32.cu", "encoder.cu", "rnn.cu", "losses.cu", "optim.cu", "cql.cu", "transformer.cu", "mlp_chain.cu", "data_pipeline.cu", "dp_nccl.cu", "gripper.cu", "replay.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-cudart", "static"]
 

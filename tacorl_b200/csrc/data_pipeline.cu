@@ -109,15 +109,24 @@ __device__ __forceinline__ void cj_apply(float& r, float& g, float& b, int order
   }
 }
 
+// Frame n of the batch reads its op order / factors at entry (n / nf) * n_slots + slot0 + n % nf of the tables: frames
+// come in groups of nf (a window), each group's parameters in a row of n_slots entries (tacorl_replay_color_jitter).
+// nf = n_slots = 1, slot0 = 0: entry n.
+__device__ __forceinline__ long long cj_entry(long long n, int nf, int n_slots, int slot0) {
+  return (n / nf) * n_slots + slot0 + n % nf;
+}
+
 // pre-pass: mean over the frame of the grayscale of the image as it is when the contrast op runs
 __global__ void color_jitter_mean_kernel(const unsigned char* __restrict__ x, int H, int W, const int* __restrict__ order,
-                                         const float* __restrict__ factors, float* __restrict__ mean) {
+                                         const float* __restrict__ factors, int nf, int n_slots, int slot0,
+                                         float* __restrict__ mean) {
   __shared__ float red[32];
   const int n = blockIdx.x;
   const long long plane = (long long)H * W;
   const unsigned char* xp = x + (long long)n * 3 * plane;
-  const int ord = order[n];
-  const float fb = factors[n * 3], fc = factors[n * 3 + 1], fh = factors[n * 3 + 2];
+  const long long q = cj_entry(n, nf, n_slots, slot0);
+  const int ord = order[q];
+  const float fb = factors[q * 3], fc = factors[q * 3 + 1], fh = factors[q * 3 + 2];
   float s = 0.f;
   for (long long p = threadIdx.x; p < plane; p += blockDim.x) {
     float r = xp[p] * (1.f / 255.f), g = xp[plane + p] * (1.f / 255.f), b = xp[2 * plane + p] * (1.f / 255.f);
@@ -135,15 +144,19 @@ __global__ void color_jitter_mean_kernel(const unsigned char* __restrict__ x, in
 }
 
 __global__ void color_jitter_kernel(const unsigned char* __restrict__ x, long long N, int H, int W,
-                                    const int* __restrict__ order, const float* __restrict__ factors,
-                                    const float* __restrict__ mean, float norm_mean, float norm_std, float* __restrict__ out) {
+                                    const int* __restrict__ order, const float* __restrict__ factors, int nf,
+                                    int n_slots, int slot0, const float* __restrict__ mean, float norm_mean,
+                                    float norm_std, float* __restrict__ out) {
   const long long plane = (long long)H * W, total = N * plane;
   const float inv_std = 1.f / norm_std;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const long long n = i / plane, p = i - n * plane;
     const unsigned char* xp = x + n * 3 * plane;
     float r = xp[p] * (1.f / 255.f), g = xp[plane + p] * (1.f / 255.f), b = xp[2 * plane + p] * (1.f / 255.f);
-    if (order) cj_apply(r, g, b, order[n], factors[n * 3], factors[n * 3 + 1], factors[n * 3 + 2], mean[n], false);
+    if (order) {
+      const long long q = cj_entry(n, nf, n_slots, slot0);
+      cj_apply(r, g, b, order[q], factors[q * 3], factors[q * 3 + 1], factors[q * 3 + 2], mean[n], false);
+    }
     float* op = out + n * 3 * plane;
     op[p] = (r - norm_mean) * inv_std; op[plane + p] = (g - norm_mean) * inv_std; op[2 * plane + p] = (b - norm_mean) * inv_std;
   }
@@ -187,12 +200,31 @@ int tacorl_color_jitter_u8(const unsigned char* x, long long N, int H, int W, co
   if (N == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   if (order) {
-    color_jitter_mean_kernel<<<(int)N, 256, 0, st>>>(x, H, W, order, factors, mean_ws);
+    color_jitter_mean_kernel<<<(int)N, 256, 0, st>>>(x, H, W, order, factors, 1, 1, 0, mean_ws);
     TACORL_LAUNCH_CHECK();
   }
   const long long total = N * H * W;
-  color_jitter_kernel<<<(int)min((long long)148 * 16, (total + 255) / 256), 256, 0, st>>>(x, N, H, W, order, factors, mean_ws,
-                                                                                        norm_mean, norm_std, out);
+  color_jitter_kernel<<<(int)min((long long)148 * 16, (total + 255) / 256), 256, 0, st>>>(x, N, H, W, order, factors, 1, 1, 0,
+                                                                                        mean_ws, norm_mean, norm_std, out);
+  TACORL_LAUNCH_CHECK();
+  return 0;
+}
+
+int tacorl_replay_color_jitter(const unsigned char* x, int B, int nf, int H, int W, const int* order,
+                               const float* factors, int n_slots, int slot0, float norm_mean, float norm_std,
+                               float* mean_ws, float* out, void* stream) {
+  TACORL_REQUIRE(x && order && factors && mean_ws && out, "replay_color_jitter: null pointer");
+  TACORL_REQUIRE(norm_std != 0.f, "replay_color_jitter: std must not be zero");
+  TACORL_REQUIRE(nf > 0 && slot0 >= 0 && slot0 + nf <= n_slots, "replay_color_jitter: slots %d + %d > %d", slot0, nf,
+                 n_slots);
+  const long long N = (long long)B * nf;
+  if (N == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  color_jitter_mean_kernel<<<(int)N, 256, 0, st>>>(x, H, W, order, factors, nf, n_slots, slot0, mean_ws);
+  TACORL_LAUNCH_CHECK();
+  const long long total = N * H * W;
+  color_jitter_kernel<<<(int)min((long long)148 * 16, (total + 255) / 256), 256, 0, st>>>(
+      x, N, H, W, order, factors, nf, n_slots, slot0, mean_ws, norm_mean, norm_std, out);
   TACORL_LAUNCH_CHECK();
   return 0;
 }

@@ -60,18 +60,39 @@ class GraphedTrainStep:
     tensors a step mutates: they are saved before the warm-up steps a capture needs and restored afterwards, so
     building a graph does not train on the example batch."""
 
-    def __init__(self, step_fn, example_batch, device=None, warmup=3, mode_key=None, preserve=None, buffers=1):
+    def __init__(self, step_fn, example_batch, device=None, warmup=3, mode_key=None, preserve=None, buffers=1,
+                 source=None):
         """buffers=2: two sets of static input buffers, one captured graph per set (sharing one memory pool), used
         alternately: `prefetch()` copies the next batch host->device straight into the set the running step is NOT
-        reading, so a host-fed loop needs no staging->static device copy between replays."""
+        reading, so a host-fed loop needs no staging->static device copy between replays.
+        source: a tacorl_b200.replay.DeviceReplay.  Every capture records `source.sample()` ahead of the step, so a
+        replay draws, assembles and trains with no host work and no host->device copy; `example_batch` may be None and
+        calls take no batch.  The source's step counter joins `preserve`: the warm-up steps consume no draws."""
         device = device or torch.device("cuda", torch.cuda.current_device())
         self.device = device
-        self.statics = [_clone_to_static(example_batch, device) for _ in range(max(1, int(buffers)))]
+        self.source = source
+        if source is not None:
+            if int(buffers) != 1:
+                raise ValueError("a replay source fills its own buffers: buffers must be 1")
+            self.statics = [source.batch()]
+            inner = step_fn
+
+            def step_fn(static, _inner=inner):
+                source.sample()
+                return _inner(static)
+            for attr in ("mode_key", "preserve"):
+                if hasattr(inner, attr):
+                    setattr(step_fn, attr, getattr(inner, attr))
+        else:
+            self.statics = [_clone_to_static(example_batch, device) for _ in range(max(1, int(buffers)))]
         self._cur = 0
         self.step_fn = step_fn
         self.warmup = warmup
         self.mode_key = mode_key if mode_key is not None else getattr(step_fn, "mode_key", None)
         self.preserve = preserve if preserve is not None else getattr(step_fn, "preserve", None)
+        if source is not None:
+            inner_preserve = self.preserve
+            self.preserve = lambda: (list(inner_preserve()) if inner_preserve is not None else []) + source.preserve()
         self._graphs = {}
         self._pool = None
         self.replays = 0
@@ -121,6 +142,8 @@ class GraphedTrainStep:
     def __call__(self, batch=None):
         """Returns the step's output tensor; with buffers > 1 it is only valid until the next call (shared pool)."""
         main = torch.cuda.current_stream()
+        if batch is not None and self.source is not None:
+            raise ValueError("this step samples its batch from its replay source: call it without a batch")
         if batch is not None:
             _copy_into(self.static, batch)
         elif self._staged:

@@ -60,7 +60,8 @@ def restore_checkpoint(module, path, strict=True):
 
 class Trainer:
     """fit(module, batches) with the reference Trainer's knobs that matter on the hot path.
-    batches: an iterable of batch dicts (host or device tensors) or a callable step -> batch; the loop runs one
+    batches: an iterable of batch dicts (host or device tensors), a callable step -> batch, or a DeviceReplay
+    (tacorl_b200.replay: the batch is drawn and assembled on the device inside the step's graph); the loop runs one
     optimisation step per batch: `loss = training_step(batch, i); backward; optimizer.step()` for automatic optimisation
     (PlayLMP), `training_step(batch)` alone for manual optimisation (TACORL steps its own optimisers).
     Under torchrun (WORLD_SIZE > 1) every FlatAdam averages its gradient over the ranks (NCCL), overlapped with the
@@ -99,10 +100,21 @@ class Trainer:
         return runtime.tacorl_step_fn(module)
 
     def fit(self, module, batches, ckpt_path=None):
+        """batches: an iterable of batch dicts, a callable step -> batch, or a tacorl_b200.replay.DeviceReplay, which
+        then samples every step's batch on the device (inside the step's CUDA graph).  With a replay, an epoch is
+        `replay.steps_per_epoch` steps unless `steps_per_epoch` says otherwise, and checkpoints carry its step counter."""
+        from .replay import DeviceReplay
+        replay = batches if isinstance(batches, DeviceReplay) else None
+        if replay is not None:
+            self._check_replay(replay)
         step_fn = self._setup(module)
         if ckpt_path is not None and Path(ckpt_path).is_file():
             ckpt = restore_checkpoint(module, ckpt_path)
             self.global_step = int(ckpt.get("global_step", 0))
+            if replay is not None and "replay" in ckpt:
+                replay.load_state_dict(ckpt["replay"])
+        if replay is not None:
+            return self._fit_replay(module, step_fn, replay)
         get = batches if callable(batches) else None
         it = None if get else iter(batches)
         graphed = None
@@ -137,6 +149,48 @@ class Trainer:
                                     module.current_epoch, self.global_step)
         if self.root and self.rank == 0:
             save_checkpoint(module, self.root / "saved_models" / "last.ckpt", module.current_epoch, self.global_step)
+        torch.cuda.synchronize(self.device)
+        return self
+
+    def _check_replay(self, replay):
+        """A replay feeds the rank whose device holds it, with that rank's shard and random stream."""
+        if torch.device(replay.device) != torch.device(self.device):
+            raise ValueError(f"the replay lives on {replay.device} but this rank trains on {self.device}: build it with "
+                             "device=cuda:LOCAL_RANK (the default under torchrun)")
+        ix = replay.index
+        if (ix.rank, ix.world_size) != (self.rank, self.world):
+            raise ValueError(f"the replay holds shard {ix.rank} of {ix.world_size} but this is rank {self.rank} of "
+                             f"{self.world}: build its ReplayIndex with rank=RANK, world_size=WORLD_SIZE")
+
+    def _fit_replay(self, module, step_fn, replay):
+        spe = self.steps_per_epoch or replay.steps_per_epoch
+        graphed = None
+        epoch0 = int(getattr(module, "current_epoch", 0))
+        done_in_epoch = 0
+
+        def save(name):
+            if self.root and self.rank == 0:
+                save_checkpoint(module, self.root / "saved_models" / name, module.current_epoch, self.global_step,
+                                extra={"replay": replay.state_dict()})
+        while not (self.max_steps >= 0 and self.global_step >= self.max_steps):
+            if self.max_steps < 0 and module.current_epoch - epoch0 >= self.max_epochs:
+                break
+            if self.use_cuda_graph:
+                if graphed is None:
+                    graphed = runtime.GraphedTrainStep(step_fn, None, device=self.device, warmup=2, source=replay)
+                out = graphed()
+            else:
+                out = step_fn(replay.sample())
+            if torch.is_tensor(out):
+                self.losses.append(out.detach().clone())
+            self.global_step += 1
+            done_in_epoch += 1
+            if done_in_epoch >= spe:
+                done_in_epoch = 0
+                module.current_epoch += 1
+                if module.current_epoch % self.save_every_n_epochs == 0:
+                    save(f"tacorl_epoch_{module.current_epoch:02d}_.ckpt")
+        save("last.ckpt")
         torch.cuda.synchronize(self.device)
         return self
 
