@@ -324,6 +324,29 @@ int tacorl_replay_color_jitter(const unsigned char* x, int B, int nf, int H, int
                                const float* factors, int n_slots, int slot0, float norm_mean, float norm_std,
                                float* mean_ws, float* out, void* stream);
 
+/* ---- validation sweeps of an HBM-resident split (tacorl_b200/replay.py mode="sweep"; rules: DESIGN.md section 14).
+ * replay_sweep: replay_sample's kernel in sweep mode.  *cursor_dev is an item cursor: row b < n of the B-row tables
+ *   takes item i = (cursor + b) mod n_valid, start valid[i], and draws its window / goal / disp / CQL goal with the laws
+ *   of replay_sample from counter (lo32(i), hi32(i), 0, draw id); then *cursor_dev += n.  No shift and no jitter.
+ * replay_gather_rows: replay_gather over rows [0, n) of the B-row tables (images[i].out and act_out: prefixes of the
+ *   B-row buffers).  replay_gather is replay_gather_rows with n = B.
+ * metrics_accumulate: ONE launch, one thread per slot: acc[i] += n * (double)*value[i] for i < k, acc[k] += n.
+ *   The struct travels by value, so a call needs no host-to-device copy. */
+#define TACORL_METRICS_MAX 32
+typedef struct tacorl_metrics {
+  const float* value[TACORL_METRICS_MAX];   /* device fp32 scalars */
+  int k;                                    /* number of metrics */
+  int n;                                    /* items of the batch */
+} tacorl_metrics;
+int tacorl_replay_sweep(int kind, int B, int n, int min_window, int max_window, unsigned long long neg_thr,
+                        unsigned long long seed, int rank, long long* cursor_dev, const int* ep_end, long long frames,
+                        const int* valid, long long n_valid, const unsigned* geom_thr, int n_geom, int* tab,
+                        long long* out64, void* stream);
+int tacorl_replay_gather_rows(int B, int n, int T, int pad, const int* tab, int n_images,
+                              const tacorl_replay_image* images, const float* act_store, int A, int act_role,
+                              int zero_pad, float* act_out, void* stream);
+int tacorl_metrics_accumulate(const tacorl_metrics* m, double* acc, void* stream);
+
 /* ---- fused small-MLP chains (fp32): a whole Linear -> act -> Linear ... stack in ONE launch, forward or backward.
  * Replaces the per-layer launches behind VisualGoalEncoder.forward (goal_encoder.py:29-33), MLPPolicy.forward
  * (actor.py:252-270: 3 x Linear+SiLU, then fc_mean | fc_log_std as ONE layer of two weight segments) and

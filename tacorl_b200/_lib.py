@@ -80,6 +80,10 @@ _SIGS = {
                              _ll, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tacorl_replay_gather": [_i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tacorl_replay_color_jitter": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _f, _f, _vp, _vp, _vp],
+    "tacorl_replay_sweep": [_i, _i, _i, _i, _i, ctypes.c_ulonglong, ctypes.c_ulonglong, _i, _vp, _vp, _ll, _vp, _ll, _vp,
+                            _i, _vp, _vp, _vp],
+    "tacorl_replay_gather_rows": [_i, _i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "tacorl_metrics_accumulate": [_vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],
     "tacorl_mlp_chain_fwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp],
     "tacorl_mlp_chain_bwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _sz, _vp],
@@ -127,6 +131,12 @@ class ReplayJitter(ctypes.Structure):
 
 REPLAY_WINDOW, REPLAY_OBS, REPLAY_NEXT, REPLAY_GOAL = 0, 1, 2, 3
 REPLAY_MAX_IMAGES = 8
+METRICS_MAX = 32
+
+
+class Metrics(ctypes.Structure):
+    """tacorl_metrics (include/tacorl_b200.h)."""
+    _fields_ = [("value", _vp * METRICS_MAX), ("k", _i), ("n", _i)]
 
 
 def lib():
@@ -201,6 +211,9 @@ def int_array(values):
 
 
 _WS = {}
+# outgrown scratch buffers stay allocated: a CUDA graph captured earlier (a training step) still reads and writes them
+# when a larger call (a validation batch bigger than the training batch) has moved on to a new buffer
+_WS_RETIRED = []
 
 
 def workspace(nbytes, device, tag="main"):
@@ -210,6 +223,8 @@ def workspace(nbytes, device, tag="main"):
     key = (device.index if device.index is not None else torch.cuda.current_device(), tag)
     buf = _WS.get(key)
     if buf is None or buf.numel() < nbytes:
+        if buf is not None:
+            _WS_RETIRED.append(buf)
         buf = torch.empty(int(nbytes * 1.25) + 4096, dtype=torch.uint8, device=device)
         _WS[key] = buf
     return buf

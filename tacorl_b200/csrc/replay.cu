@@ -3,6 +3,9 @@
 //   replay_sample_kernel   one CTA: reads the device step counter, draws every random quantity of the batch with
 //                          counter-based Philox4x32-10 (key = seed with the rank folded in, counter = (step, sample, draw
 //                          id)), writes int32 index tables and the int64 batch scalars, then advances the counter;
+//                          in sweep mode (DESIGN.md section 14) it reads an item cursor instead, takes rows [0, n) from
+//                          the items cursor .. cursor + n - 1 of the start table in order, draws with counter = (item, 0,
+//                          draw id) and advances the cursor by n;
 //   replay_gather_kernel   one block per output image plane (every modality and role of the batch in one grid, driven by
 //                          a small descriptor array) plus one block per sample for the action rows.
 // The gather keeps window_gather_u8_kernel's semantics (data_pipeline.cu): pad_sequence by repetition of the last frame,
@@ -57,8 +60,12 @@ __constant__ int kJitterPerms[6][3] = {{0, 1, 3}, {0, 3, 1}, {1, 0, 3}, {1, 3, 0
 
 struct JitterParams { int ops; float lo[3], span[3]; };
 
-__global__ void replay_sample_kernel(int kind, int B, int min_window, int max_window, int n_mod, int n_slots, int pad,
-                                     unsigned long long neg_thr, unsigned k0, unsigned k1,
+// rows: rows [0, rows) of the B-row tables are written (rows = B when training).  sweep: *step_dev is an item cursor;
+// row b takes item (cursor + b) mod n_valid of the start table and draws with counter (lo32(item), hi32(item), 0, draw
+// id); the cursor advances by rows.  Otherwise row b draws its start with counter (lo32(step), hi32(step), b, draw id)
+// and the step advances by one.
+__global__ void replay_sample_kernel(int kind, int B, int rows, int sweep, int min_window, int max_window, int n_mod,
+                                     int n_slots, int pad, unsigned long long neg_thr, unsigned k0, unsigned k1,
                                      long long* __restrict__ step_dev,
                                      const int* __restrict__ ep_end, long long frames, const int* __restrict__ valid,
                                      long long n_valid, const unsigned* __restrict__ geom_thr, int n_geom,
@@ -72,9 +79,11 @@ __global__ void replay_sample_kernel(int kind, int B, int min_window, int max_wi
   int* t_window = tab + B;
   int* t_goal = tab + 2 * B;
   int* t_disp = tab + 3 * B;
-  for (int b = threadIdx.x; b < B; b += blockDim.x) {
-    const U4 r = philox4x32_10(U4{c0, c1, (unsigned)b, DRAW_SAMPLE}, k0, k1);
-    const int s = valid[uniform_below(r.x, n_valid)];
+  for (int b = threadIdx.x; b < rows; b += blockDim.x) {
+    const unsigned long long item = sweep ? (s_step + b) % (unsigned long long)n_valid : 0ull;
+    const U4 ctr = sweep ? U4{(unsigned)item, (unsigned)(item >> 32), 0u, 0u} : U4{c0, c1, (unsigned)b, 0u};
+    const U4 r = philox4x32_10(U4{ctr.x, ctr.y, ctr.z, DRAW_SAMPLE}, k0, k1);
+    const int s = valid[sweep ? (long long)item : uniform_below(r.x, n_valid)];
     const int end = ep_end[s];
     if (kind == KIND_CQL) {
       // transition (s, s + 1); goal = min(s + k, ep_end[s]), k ~ Geometric; reward = terminal = [goal is the successor]
@@ -90,7 +99,7 @@ __global__ void replay_sample_kernel(int kind, int B, int min_window, int max_wi
     int goal = s + w - 1, disp = 1;
     if (kind == KIND_TACORL) {
       if ((unsigned long long)r.z < neg_thr) {
-        const U4 g = philox4x32_10(U4{c0, c1, (unsigned)b, DRAW_NEG_GOAL}, k0, k1);
+        const U4 g = philox4x32_10(U4{ctr.x, ctr.y, ctr.z, DRAW_NEG_GOAL}, k0, k1);
         goal = (int)uniform_below(g.x, frames);
         disp = -1;
       } else {
@@ -136,7 +145,14 @@ __global__ void replay_sample_kernel(int kind, int B, int min_window, int max_wi
     }
   }
   __syncthreads();
-  if (threadIdx.x == 0) *step_dev = (long long)(s_step + 1);
+  if (threadIdx.x == 0) *step_dev = (long long)(s_step + (sweep ? (unsigned long long)rows : 1ull));
+}
+
+// acc[i] += n * value[i] for i < k, acc[k] += n: one thread per slot, so every sum is taken in a fixed order
+__global__ void metrics_accumulate_kernel(const __grid_constant__ tacorl_metrics m, double* __restrict__ acc) {
+  const int i = threadIdx.x;
+  if (i < m.k) acc[i] += (double)m.n * (double)*m.value[i];
+  else if (i == m.k) acc[i] += (double)m.n;
 }
 
 constexpr int kMaxImages = TACORL_REPLAY_MAX_IMAGES;
@@ -226,14 +242,15 @@ using namespace tacorl;
 
 extern "C" {
 
-int tacorl_replay_sample(int kind, int B, int min_window, int max_window, int n_mod, int n_slots, int pad,
-                         unsigned long long neg_thr, unsigned long long seed, int rank, long long* step_dev,
+static int launch_sample(int kind, int B, int rows, int sweep, int min_window, int max_window, int n_mod, int n_slots,
+                         int pad, unsigned long long neg_thr, unsigned long long seed, int rank, long long* step_dev,
                          const int* ep_end, long long frames, const int* valid, long long n_valid,
                          const unsigned* geom_thr, int n_geom, int* tab, int* shift, long long* out64,
                          const tacorl_replay_jitter* jitter, int* jit_order, float* jit_factors, void* stream) {
   TACORL_REQUIRE(kind >= KIND_PLAY_LMP && kind <= KIND_CQL, "replay_sample: unknown kind %d", kind);
   TACORL_REQUIRE(step_dev && ep_end && valid && tab && out64, "replay_sample: null pointer");
   TACORL_REQUIRE(B > 0 && frames > 0 && n_valid > 0, "replay_sample: empty batch, store or start table");
+  TACORL_REQUIRE(rows > 0 && rows <= B, "replay_sample: %d rows for a batch of %d", rows, B);
   TACORL_REQUIRE(kind == KIND_CQL || (min_window >= 1 && max_window >= min_window),
                  "replay_sample: window bounds %d..%d", min_window, max_window);
   TACORL_REQUIRE(kind == KIND_PLAY_LMP || (geom_thr && n_geom > 0), "replay_sample: geometric table missing");
@@ -246,16 +263,36 @@ int tacorl_replay_sample(int kind, int B, int min_window, int max_window, int n_
     for (int i = 0; i < 3; ++i) { jit.lo[i] = jitter->lo[i]; jit.span[i] = jitter->span[i]; }
   }
   replay_sample_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(
-      kind, B, min_window, max_window, n_mod, n_slots, pad, neg_thr, (unsigned)seed,
+      kind, B, rows, sweep, min_window, max_window, n_mod, n_slots, pad, neg_thr, (unsigned)seed,
       (unsigned)(seed >> 32) ^ ((unsigned)rank * 0x9E3779B9u), step_dev, ep_end, frames, valid, n_valid, geom_thr, n_geom,
       tab, shift, out64, jit, jitter ? jit_order : nullptr, jitter ? jit_factors : nullptr);
   TACORL_LAUNCH_CHECK();
   return 0;
 }
 
-int tacorl_replay_gather(int B, int T, int pad, const int* tab, int n_images, const tacorl_replay_image* images,
-                         const float* act_store, int A, int act_role, int zero_pad, float* act_out, void* stream) {
+int tacorl_replay_sample(int kind, int B, int min_window, int max_window, int n_mod, int n_slots, int pad,
+                         unsigned long long neg_thr, unsigned long long seed, int rank, long long* step_dev,
+                         const int* ep_end, long long frames, const int* valid, long long n_valid,
+                         const unsigned* geom_thr, int n_geom, int* tab, int* shift, long long* out64,
+                         const tacorl_replay_jitter* jitter, int* jit_order, float* jit_factors, void* stream) {
+  return launch_sample(kind, B, B, 0, min_window, max_window, n_mod, n_slots, pad, neg_thr, seed, rank, step_dev, ep_end,
+                       frames, valid, n_valid, geom_thr, n_geom, tab, shift, out64, jitter, jit_order, jit_factors,
+                       stream);
+}
+
+int tacorl_replay_sweep(int kind, int B, int n, int min_window, int max_window, unsigned long long neg_thr,
+                        unsigned long long seed, int rank, long long* cursor_dev, const int* ep_end, long long frames,
+                        const int* valid, long long n_valid, const unsigned* geom_thr, int n_geom, int* tab,
+                        long long* out64, void* stream) {
+  return launch_sample(kind, B, n, 1, min_window, max_window, 0, 0, 0, neg_thr, seed, rank, cursor_dev, ep_end, frames,
+                       valid, n_valid, geom_thr, n_geom, tab, nullptr, out64, nullptr, nullptr, nullptr, stream);
+}
+
+int tacorl_replay_gather_rows(int B, int n, int T, int pad, const int* tab, int n_images,
+                              const tacorl_replay_image* images, const float* act_store, int A, int act_role,
+                              int zero_pad, float* act_out, void* stream) {
   TACORL_REQUIRE(tab && B > 0 && T > 0, "replay_gather: null table / empty batch");
+  TACORL_REQUIRE(n > 0 && n <= B, "replay_gather: %d rows for a batch of %d", n, B);
   TACORL_REQUIRE(n_images >= 0 && n_images <= kMaxImages, "replay_gather: %d images (at most %d)", n_images, kMaxImages);
   TACORL_REQUIRE(!act_out || (act_store && A > 0), "replay_gather: action store missing");
   GatherArgs a{};
@@ -272,15 +309,32 @@ int tacorl_replay_gather(int B, int T, int pad, const int* tab, int n_images, co
     TACORL_REQUIRE(!im.shift || (im.shift_slot >= 0 && im.shift_slot + nf <= im.n_slots),
                    "replay_gather: image %d: shift slots %d + %d > %d", i, im.shift_slot, nf, im.n_slots);
     a.img[i] = GatherImage{im.store, im.out, im.shift, im.H, im.W, im.role, nf, im.shift_slot, im.n_slots, (int)planes};
-    planes += (long long)B * nf * 3;
+    planes += (long long)n * nf * 3;
   }
   TACORL_REQUIRE(planes < (1LL << 30), "replay_gather: batch too large");
   a.n_img = n_images; a.n_planes = (int)planes;
   a.B = B; a.T = T; a.pad = pad; a.tab = tab;
   a.act_store = act_store; a.act_out = act_out; a.A = A; a.act_role = act_role; a.zero_pad = zero_pad;
-  const long long blocks = planes + (act_out ? B : 0);
+  const long long blocks = planes + (act_out ? n : 0);
   if (blocks == 0) return 0;
   replay_gather_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(a);
+  TACORL_LAUNCH_CHECK();
+  return 0;
+}
+
+int tacorl_replay_gather(int B, int T, int pad, const int* tab, int n_images, const tacorl_replay_image* images,
+                         const float* act_store, int A, int act_role, int zero_pad, float* act_out, void* stream) {
+  return tacorl_replay_gather_rows(B, B, T, pad, tab, n_images, images, act_store, A, act_role, zero_pad, act_out,
+                                   stream);
+}
+
+int tacorl_metrics_accumulate(const tacorl_metrics* m, double* acc, void* stream) {
+  TACORL_REQUIRE(m && acc, "metrics_accumulate: null pointer");
+  TACORL_REQUIRE(m->k >= 0 && m->k <= TACORL_METRICS_MAX, "metrics_accumulate: %d metrics (at most %d)", m->k,
+                 TACORL_METRICS_MAX);
+  TACORL_REQUIRE(m->n > 0, "metrics_accumulate: batch of %d items", m->n);
+  for (int i = 0; i < m->k; ++i) TACORL_REQUIRE(m->value[i], "metrics_accumulate: metric %d: null pointer", i);
+  metrics_accumulate_kernel<<<1, 32 * ((m->k + 32) / 32), 0, (cudaStream_t)stream>>>(*m, acc);
   TACORL_LAUNCH_CHECK();
   return 0;
 }

@@ -672,6 +672,10 @@ class ReluRNN2Fn(Function):
 
 
 def relu_rnn(x_tm, weights, num_layers, bidirectional, last_only=False, h0=None, grad_rows=None):
+    if not torch.is_grad_enabled():
+        # no backward will follow (validation, frozen encoders): keep no BPTT operands and fork no W_hh^T preparation
+        # onto the prep stream, whose work only a backward joins (a captured graph would end with it unjoined)
+        x_tm, weights = x_tm.detach(), [w.detach() for w in weights]
     if h0 is None and _STATE["prec"] == L.PREC_BF16 and x_tm.is_cuda and weights[1].shape[0] % 8 == 0:
         return ReluRNN2Fn.apply(x_tm, num_layers, bidirectional, last_only, grad_rows, *weights)
     return ReluRNNFn.apply(x_tm, h0, num_layers, bidirectional, last_only, *weights)

@@ -10,7 +10,14 @@ crosses PCIe after start-up.
 frame of f's episode) and the lookup tables the sampler draws from.  `DeviceReplay` holds the store on one device and
 fills persistent output buffers in place; `sample()` returns the batch dict the modules consume (oracle/synth.py layout).
 The sampling rules are DESIGN.md section 13: i.i.d. with replacement at every step, reproducible bit for bit from
-(seed, rank, step)."""
+(seed, rank, step).
+
+`DeviceReplay(..., mode="sweep")` holds a validation split instead: every sweep visits each item of the rank's store
+once, in store order, with per-item draws that depend on (seed, rank, item) only (DESIGN.md section 14).
+
+    val = DeviceReplay(ReplayIndex.from_calvin("task_D_D/validation", ...), batch_size=64, kind="play_lmp",
+                       min_window=8, max_window=16, seed=0, mode="sweep")
+    Trainer(max_epochs=30).fit(module, replay, val=val)"""
 import ctypes
 import os
 
@@ -143,6 +150,11 @@ class ReplayIndex:
         """Transition starts: frames with a successor in their episode."""
         return np.nonzero(self.ep_end > np.arange(self.num_frames))[0].astype(np.int32)
 
+    def items(self, kind, min_window=1):
+        """The start table a replay of `kind` draws from, and a sweep visits in order: window starts (play_lmp,
+        tacorl) or transition starts (cql)."""
+        return self.valid_transitions() if kind == "cql" else self.valid_starts(min_window)
+
     def geometric_thresholds(self, p):
         return geometric_thresholds(p)
 
@@ -177,6 +189,15 @@ def _jitter_params(jitter):
             "lo": [cs.lo[i] for i in range(3)], "span": [cs.span[i] for i in range(3)]}
 
 
+def sweep_shape(items, batch_size):
+    """(full batches, tail rows) of a sweep over `items` items: every item once, the tail neither padded nor dropped."""
+    return int(items) // int(batch_size), int(items) % int(batch_size)
+
+
+def _prefix(batch, n):
+    return {k: (_prefix(v, n) if isinstance(v, dict) else v[:n]) for k, v in batch.items()}
+
+
 def _validate(index, valid):
     F = index.num_frames
     f = np.arange(F)
@@ -200,12 +221,21 @@ class DeviceReplay:
     ColorTransform of rl_train.yaml on every frame with its own op order and factors (torchvision ColorJitter ranges
     [max(0, 1 - b), 1 + b], [max(0, 1 - c), 1 + c], [-h, h]), then Normalize(mean, std): frames come out float32.
     The step counter lives on the device and advances inside sample().  device defaults to cuda:LOCAL_RANK under
-    torchrun (else the current device); sample() always launches on that device's current stream."""
+    torchrun (else the current device); sample() always launches on that device's current stream.
+
+    mode="sweep": a validation split.  The items (window starts; CQL: transitions) form `batches_per_sweep` full
+    batches and a `tail` of `items % batch_size` rows; `reset()` puts the device item cursor at 0 and `sample(n)` fills
+    rows [0, n) from the next n items and returns prefix views.  No augmentation: pad must be 0 and jitter None."""
 
     def __init__(self, index, batch_size, kind="play_lmp", min_window=8, max_window=16, pad=0, goal_p=0.3,
-                 neg_frac=0.1, jitter=None, seed=0, device=None):
+                 neg_frac=0.1, jitter=None, seed=0, device=None, mode="train"):
         if kind not in KINDS:
             raise ValueError(f"kind must be one of {sorted(KINDS)}, got {kind!r}")
+        if mode not in ("train", "sweep"):
+            raise ValueError(f"mode must be 'train' or 'sweep', got {mode!r}")
+        if mode == "sweep" and (int(pad) > 0 or _jitter_params(jitter) is not None):
+            raise ValueError("a validation sweep does not augment: build it with pad=0 and jitter=None")
+        self.mode = mode
         if kind != "cql" and not 1 <= min_window <= max_window:
             raise ValueError(f"window bounds {min_window}..{max_window}")
         if not 0.0 <= neg_frac <= 1.0:
@@ -225,7 +255,7 @@ class DeviceReplay:
         self.jitter = _jitter_params(jitter)
         mods = index.modalities
         self.n_slots = {"play_lmp": self.T, "tacorl": self.T + 1, "cql": 3}[kind]
-        valid = index.valid_transitions() if kind == "cql" else index.valid_starts(self.min_window)
+        valid = index.items(kind, self.min_window)
         # goals and CQL offsets draw from the geometric table; PlayLMP never reads it
         geom = geometric_thresholds(self.goal_p) if kind != "play_lmp" else np.full(1, 2 ** 32 - 1, np.uint32)
         _validate(index, valid)
@@ -327,8 +357,13 @@ class DeviceReplay:
         self._n_images = len(jobs)
 
     # ---- the step
-    def sample(self):
-        """Draw and assemble the next batch on the current stream (two launches); returns the batch dict."""
+    def sample(self, n=None):
+        """Draw and assemble the next batch on the current stream (two launches); returns the batch dict.
+        Sweep mode: rows [0, n) (default: the whole batch) from the next n items; the batch dict holds prefix views."""
+        if self.mode == "sweep":
+            return self._sweep(self.B if n is None else int(n))
+        if n is not None:
+            raise ValueError("a training replay always draws whole batches: call sample() without n")
         with torch.cuda.device(self.device):
             s = L.stream()
             jit = None if self.jitter is None else ctypes.byref(self.jitter["c"])
@@ -349,13 +384,32 @@ class DeviceReplay:
                        L.ptr(ws), L.ptr(out), s)
         return self.batch()
 
+    def _sweep(self, n):
+        if not 1 <= n <= self.B:
+            raise ValueError(f"a sweep batch holds 1..{self.B} rows, got {n}")
+        with torch.cuda.device(self.device):
+            s = L.stream()
+            L.call("tacorl_replay_sweep", KINDS[self.kind], self.B, n, self.min_window, self.max_window, self.neg_thr,
+                   self.seed & 0xFFFFFFFFFFFFFFFF, self.rank, L.ptr_any(self._step), L.ptr_any(self.ep_end),
+                   self.index.num_frames, L.ptr_any(self.valid), self.n_valid, L.ptr_any(self.geom), self.n_geom,
+                   L.ptr_any(self.tab), L.ptr_any(self.out64), s)
+            act_role = L.REPLAY_OBS if self.kind == "cql" else L.REPLAY_WINDOW
+            L.call("tacorl_replay_gather_rows", self.B, n, self.T, 0, L.ptr_any(self.tab), self._n_images,
+                   ctypes.cast(self._images, ctypes.c_void_p), L.ptr_any(self.actions_store), self.actions.shape[-1],
+                   act_role, 1 if self.action_zero_pad else 0, L.ptr_any(self.actions), s)
+        return self.batch(n)
+
     @property
     def action_zero_pad(self):
         """Relative actions pad with zeros (gripper repeated); absolute ones repeat the last step."""
         return self.index.action_key.startswith("rel")
 
-    def batch(self):
-        """The batch dict over the persistent buffers (a fresh dict each call: modules may rebind its entries)."""
+    def batch(self, n=None):
+        """The batch dict over the persistent buffers (a fresh dict each call: modules may rebind its entries).
+        n: views of the first n rows only (a sweep's tail)."""
+        if n is not None:
+            full = self.batch()
+            return _prefix(full, int(n))
         if self.kind == "cql":
             return {"observations": {"observation": dict(self.obs), "goal": dict(self.goal)}, "actions": self.actions,
                     "next_observations": {"observation": dict(self.next_obs), "goal": dict(self.goal)},
@@ -378,8 +432,32 @@ class DeviceReplay:
         return int(self._step.item())
 
     def preserve(self):
-        """Tensors sample() mutates that a graph capture must restore (GraphedTrainStep)."""
+        """Tensors sample() mutates that a graph capture must restore (GraphedTrainStep): the step counter, or in
+        sweep mode the item cursor."""
         return [self._step]
+
+    # ---- sweep mode
+    @property
+    def items(self):
+        """Items of one sweep: valid window starts (CQL: transitions) on this rank."""
+        return self.n_valid
+
+    @property
+    def batches_per_sweep(self):
+        """Full batches of one sweep."""
+        return sweep_shape(self.n_valid, self.B)[0]
+
+    @property
+    def tail(self):
+        """Rows of the sweep's last, partial batch (0: none)."""
+        return sweep_shape(self.n_valid, self.B)[1]
+
+    def reset(self):
+        """Put the sweep's item cursor at the first item (on the device's current stream)."""
+        if self.mode != "sweep":
+            raise ValueError("reset() rewinds a validation sweep; a training replay resumes with load_state_dict()")
+        with torch.cuda.device(self.device):
+            self._step.zero_()
 
     @property
     def steps_per_epoch(self):

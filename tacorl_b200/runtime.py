@@ -4,6 +4,8 @@ The step issues several hundred small launches (per-timestep recurrent GEMMs, pe
 kernels); replaying them from one captured graph removes the host launch / ctypes / autograd overhead that would
 otherwise dominate a ~ms step (SURVEY.md §7 "Host overhead").  Noise keeps advancing between replays (the torch
 CUDA generator is graph-aware) and the Adam bias correction reads a device-resident step counter."""
+import ctypes
+
 import torch
 
 
@@ -228,4 +230,80 @@ def tacorl_step_fn(module):
     step.mode_key = lambda: (module.current_epoch < module.bc_epochs, bool(getattr(module, "finetune_action_decoder", False)),
                              tuple(float(o.param_groups[0]["lr"]) for o in opts), bool(module.training))
     step.preserve = lambda: list(opts) + [b.flat for b in (module._target_bufs or ())]
+    return step
+
+
+def item_weighted_means(keys, totals):
+    """Epoch value of every logged validation scalar: `totals` holds one (sums, count) vector per rank, sums[i] =
+    sum over the rank's batches of n_b * mean_b of keys[i], count = sum of n_b.  Ranks are added before dividing, as
+    Lightning aggregates `self.log(..., on_epoch=True, sync_dist=True)`.  Pure host function."""
+    rows = [[float(x) for x in t] for t in totals]
+    if not rows or any(len(r) != len(keys) + 1 for r in rows):
+        raise ValueError(f"expected (sums, count) vectors of {len(keys) + 1} entries")
+    total = [sum(col) for col in zip(*rows)]
+    count = total[-1]
+    if count <= 0:
+        raise ValueError("no validation item was evaluated")
+    return {k: total[i] / count for i, k in enumerate(keys)}
+
+
+class MetricsAccumulator:
+    """Device fp64 (sums, count) of the `prefix` scalars a module logs: `add(logged, n)` is one launch
+    (tacorl_metrics_accumulate, graph-capturable, no host copy) that adds n * value to each sum and n to the count.
+    The keys are fixed by the first add().  `read()` is the only device-to-host copy."""
+
+    def __init__(self, device, prefix="validation/"):
+        from . import _lib
+        device = torch.device(device)
+        self.device = device if device.index is not None else torch.device("cuda", torch.cuda.current_device())
+        self.prefix = prefix
+        self.keys = None
+        self.acc = torch.zeros(_lib.METRICS_MAX + 1, dtype=torch.float64, device=self.device)
+
+    def reset(self):
+        self.acc.zero_()
+
+    def add(self, logged, n):
+        from . import _lib
+        if self.keys is None:
+            self.keys = sorted(k for k in logged if k.startswith(self.prefix))
+            if not self.keys:
+                raise ValueError(f"the step logged no '{self.prefix}*' scalar")
+            if len(self.keys) > _lib.METRICS_MAX:
+                raise ValueError(f"{len(self.keys)} metrics; at most {_lib.METRICS_MAX} are accumulated")
+        m = _lib.Metrics()
+        for i, k in enumerate(self.keys):
+            v = logged.get(k)
+            if not torch.is_tensor(v) or v.numel() != 1 or v.device != self.device:
+                raise ValueError(f"{k}: expected a one-element tensor on {self.device}, got {v!r}")
+            if v.dtype != torch.float32:
+                v = v.float()
+                logged[k] = v                         # keeps the converted value alive while the launch reads it
+            m.value[i] = v.data_ptr()
+        m.k, m.n = len(self.keys), int(n)
+        _lib.call("tacorl_metrics_accumulate", ctypes.byref(m), _lib.ptr_any(self.acc), _lib.stream())
+
+    def totals(self):
+        """The (sums, count) vector on the device."""
+        return self.acc[:len(self.keys or ()) + 1]
+
+    def read(self, totals=None):
+        """{key: item-weighted mean} from the device vector (one device-to-host copy)."""
+        if self.keys is None:
+            raise ValueError("no validation batch was evaluated")
+        t = (self.totals() if totals is None else totals).cpu().tolist()
+        return item_weighted_means(self.keys, [t])
+
+
+def validation_step_fn(module, accumulator):
+    """One validation batch: `module.validation_step(batch)` under no_grad, then the accumulate launch with the batch's
+    item count (its rows).  Same contract as play_lmp_step_fn / tacorl_step_fn, so GraphedTrainStep replays it."""
+    def step(batch):
+        with torch.no_grad():
+            module.validation_step(batch, 0)
+        accumulator.add(module.logged, batch["actions"].shape[0])
+    # host state the validation forward reads: TACO-RL's BC actor loss below bc_epochs, PlayLMP's kl_beta by value
+    step.mode_key = lambda: (module.current_epoch < getattr(module, "bc_epochs", 0), float(getattr(module, "kl_beta", 0.0)),
+                             bool(getattr(module, "finetune_action_decoder", False)), bool(module.training))
+    step.preserve = lambda: [accumulator.acc]
     return step

@@ -16,6 +16,8 @@ import torch.distributed as dist
 from . import ops, parallel, runtime
 
 CKPT_VERSION = "1.6.5"      # the reference pins pytorch-lightning < 1.7 (setup.cfg:17)
+# the CUDA generator's seed during a validation sweep (restored afterwards): the same weights give the same metrics
+VALIDATION_SEED = 0x7A11D
 
 
 def _to_device(batch, device):
@@ -65,10 +67,15 @@ class Trainer:
     optimisation step per batch: `loss = training_step(batch, i); backward; optimizer.step()` for automatic optimisation
     (PlayLMP), `training_step(batch)` alone for manual optimisation (TACORL steps its own optimisers).
     Under torchrun (WORLD_SIZE > 1) every FlatAdam averages its gradient over the ranks (NCCL), overlapped with the
-    encoder backward; rank r must be fed its own shard (parallel.shard_batch)."""
+    encoder backward; rank r must be fed its own shard (parallel.shard_batch).
+
+    Validation (`fit(..., val=)`, `validate`): every `check_val_every_n_epoch`-th epoch ends with a sweep of `val`, a
+    DeviceReplay(mode="sweep") or a re-iterable of host batches, through the module's `validation_step`.  Each logged
+    `validation/*` scalar becomes its item-weighted mean over the sweep (summed over ranks), in `callback_metrics` and
+    `val_history`.  A sweep runs in eval mode under a fixed generator seed and leaves the training run untouched."""
 
     def __init__(self, max_steps=-1, max_epochs=1, precision="bf16", use_cuda_graph=True, default_root_dir=None,
-                 steps_per_epoch=None, save_every_n_epochs=1, device=None):
+                 steps_per_epoch=None, save_every_n_epochs=1, device=None, check_val_every_n_epoch=1):
         self.max_steps, self.max_epochs = max_steps, max_epochs
         self.precision = {"16": "bf16", 16: "bf16", "bf16": "bf16", "32": "fp32", 32: "fp32", "fp32": "fp32"}[precision]
         self.use_cuda_graph = use_cuda_graph
@@ -81,8 +88,14 @@ class Trainer:
         self.device = device or torch.device("cuda", self.local)
         self.global_step = 0
         self.losses = []
+        if int(check_val_every_n_epoch) < 1:
+            raise ValueError(f"check_val_every_n_epoch must be >= 1, got {check_val_every_n_epoch}")
+        self.check_val_every_n_epoch = int(check_val_every_n_epoch)
+        self.callback_metrics = {}
+        self.val_history = []                 # (epoch, global_step, metrics) per sweep of fit()
+        self._val_states = {}
 
-    def _setup(self, module):
+    def _setup_device(self, module):
         torch.cuda.set_device(self.device)
         ops.set_precision(self.precision)
         if self.world > 1 and not dist.is_initialized():
@@ -90,6 +103,9 @@ class Trainer:
             os.environ.setdefault("NCCL_MIN_NCHANNELS", str(parallel.collective_channels(self.world)))
             dist.init_process_group("nccl", device_id=self.device)
         module.to(self.device)
+
+    def _setup(self, module):
+        self._setup_device(module)
         module.train()
         opts = _optimizers_of(module)
         if self.world > 1:
@@ -99,22 +115,31 @@ class Trainer:
             return runtime.play_lmp_step_fn(module, opts[0])
         return runtime.tacorl_step_fn(module)
 
-    def fit(self, module, batches, ckpt_path=None):
+    def fit(self, module, batches, ckpt_path=None, val=None):
         """batches: an iterable of batch dicts, a callable step -> batch, or a tacorl_b200.replay.DeviceReplay, which
         then samples every step's batch on the device (inside the step's CUDA graph).  With a replay, an epoch is
-        `replay.steps_per_epoch` steps unless `steps_per_epoch` says otherwise, and checkpoints carry its step counter."""
+        `replay.steps_per_epoch` steps unless `steps_per_epoch` says otherwise, and checkpoints carry its step counter.
+        val: validation data (see `validate`), swept at the end of every `check_val_every_n_epoch`-th epoch before
+        that epoch's checkpoint is written; checkpoints then carry the results under "validation"."""
         from .replay import DeviceReplay
         replay = batches if isinstance(batches, DeviceReplay) else None
         if replay is not None:
+            if replay.mode != "train":
+                raise ValueError("a sweep-mode DeviceReplay is a validation split: pass it as val=, not as the batches")
             self._check_replay(replay)
+        if val is not None:
+            self._check_val(val)
         step_fn = self._setup(module)
         if ckpt_path is not None and Path(ckpt_path).is_file():
             ckpt = restore_checkpoint(module, ckpt_path)
             self.global_step = int(ckpt.get("global_step", 0))
             if replay is not None and "replay" in ckpt:
                 replay.load_state_dict(ckpt["replay"])
+            if "validation" in ckpt:
+                self.val_history = list(ckpt["validation"]["history"])
+                self.callback_metrics = dict(ckpt["validation"]["metrics"])
         if replay is not None:
-            return self._fit_replay(module, step_fn, replay)
+            return self._fit_replay(module, step_fn, replay, val)
         get = batches if callable(batches) else None
         it = None if get else iter(batches)
         graphed = None
@@ -143,12 +168,14 @@ class Trainer:
             done_in_epoch += 1
             if self.steps_per_epoch and done_in_epoch >= self.steps_per_epoch:
                 done_in_epoch = 0
+                self._end_of_epoch(module, val)
                 module.current_epoch += 1          # (a graph captured for the BC epochs is swapped when bc_epochs is crossed)
                 if self.root and self.rank == 0 and module.current_epoch % self.save_every_n_epochs == 0:
                     save_checkpoint(module, self.root / "saved_models" / f"tacorl_epoch_{module.current_epoch:02d}_.ckpt",
-                                    module.current_epoch, self.global_step)
+                                    module.current_epoch, self.global_step, extra=self._val_extra(val))
         if self.root and self.rank == 0:
-            save_checkpoint(module, self.root / "saved_models" / "last.ckpt", module.current_epoch, self.global_step)
+            save_checkpoint(module, self.root / "saved_models" / "last.ckpt", module.current_epoch, self.global_step,
+                            extra=self._val_extra(val))
         torch.cuda.synchronize(self.device)
         return self
 
@@ -162,7 +189,89 @@ class Trainer:
             raise ValueError(f"the replay holds shard {ix.rank} of {ix.world_size} but this is rank {self.rank} of "
                              f"{self.world}: build its ReplayIndex with rank=RANK, world_size=WORLD_SIZE")
 
-    def _fit_replay(self, module, step_fn, replay):
+    def _check_val(self, val):
+        from .replay import DeviceReplay
+        if isinstance(val, DeviceReplay):
+            if val.mode != "sweep":
+                raise ValueError("val= takes a DeviceReplay built with mode='sweep' (or an iterable of batches)")
+            self._check_replay(val)
+        elif callable(val) or not hasattr(val, "__iter__"):
+            raise ValueError("val= takes a sweep-mode DeviceReplay or a re-iterable of batch dicts")
+
+    def _val_extra(self, val):
+        if val is None:
+            return None
+        return {"validation": {"metrics": dict(self.callback_metrics), "history": list(self.val_history)}}
+
+    def _end_of_epoch(self, module, val):
+        """Lightning's rule: validate after epoch e when (e + 1) % check_val_every_n_epoch == 0 (current_epoch = e)."""
+        if val is None or (module.current_epoch + 1) % self.check_val_every_n_epoch:
+            return
+        metrics = self._sweep(module, val)
+        self.callback_metrics = dict(metrics)
+        self.val_history.append((int(module.current_epoch), int(self.global_step), dict(metrics)))
+
+    def validate(self, module, val):
+        """One validation sweep of `module` over `val`: a DeviceReplay(mode="sweep") of this rank's split (full batches
+        replayed from one CUDA graph, the tail run eagerly on prefix views) or a re-iterable of batch dicts (copied to
+        the device, run eagerly).  Returns [{"validation/...": item-weighted mean}] like pl.Trainer.validate."""
+        self._check_val(val)
+        self._setup_device(module)
+        metrics = self._sweep(module, val)
+        self.callback_metrics = dict(metrics)
+        return [metrics]
+
+    def _sweep(self, module, val):
+        """eval mode, the generator saved and seeded with VALIDATION_SEED, cursor and sums reset, every batch through
+        validation_step_fn, one read-back of the (sums, count) vector (all-reduced over ranks first), then the
+        generator and every submodule's train/eval flag restored."""
+        from .replay import DeviceReplay
+        key = (id(module), id(val))
+        if key not in self._val_states:
+            acc = runtime.MetricsAccumulator(self.device)
+            self._val_states[key] = {"acc": acc, "step": runtime.validation_step_fn(module, acc), "graph": None}
+        st = self._val_states[key]
+        acc, step_fn = st["acc"], st["step"]
+        flags = [(m, m.training) for m in module.modules()]
+        with torch.cuda.device(self.device):
+            rng = torch.cuda.get_rng_state()
+            module.eval()
+            try:
+                if isinstance(val, DeviceReplay):
+                    graphed = None
+                    if self.use_cuda_graph and val.batches_per_sweep:
+                        graphed = st["graph"]
+                        if graphed is None:
+                            graphed = st["graph"] = runtime.GraphedTrainStep(step_fn, None, device=self.device,
+                                                                             warmup=2, source=val)
+                        elif (graphed._key(), graphed._cur) != graphed._active_key:
+                            graphed._select(graphed._key())     # capture a new host mode now, before the seed is set
+                    torch.cuda.manual_seed(VALIDATION_SEED)
+                    acc.reset()
+                    val.reset()
+                    for _ in range(val.batches_per_sweep):
+                        if graphed is not None:
+                            graphed()
+                        else:
+                            step_fn(val.sample())
+                    if val.tail:
+                        step_fn(val.sample(val.tail))
+                else:
+                    torch.cuda.manual_seed(VALIDATION_SEED)
+                    acc.reset()
+                    for batch in val:
+                        step_fn(_to_device(batch, self.device))
+                totals = acc.totals()
+                if self.world > 1:
+                    totals = totals.clone()
+                    dist.all_reduce(totals)
+                return acc.read(totals)
+            finally:
+                torch.cuda.set_rng_state(rng)
+                for m, training in flags:
+                    m.training = training
+
+    def _fit_replay(self, module, step_fn, replay, val=None):
         spe = self.steps_per_epoch or replay.steps_per_epoch
         graphed = None
         epoch0 = int(getattr(module, "current_epoch", 0))
@@ -170,8 +279,10 @@ class Trainer:
 
         def save(name):
             if self.root and self.rank == 0:
+                extra = {"replay": replay.state_dict()}
+                extra.update(self._val_extra(val) or {})
                 save_checkpoint(module, self.root / "saved_models" / name, module.current_epoch, self.global_step,
-                                extra={"replay": replay.state_dict()})
+                                extra=extra)
         while not (self.max_steps >= 0 and self.global_step >= self.max_steps):
             if self.max_steps < 0 and module.current_epoch - epoch0 >= self.max_epochs:
                 break
@@ -187,6 +298,7 @@ class Trainer:
             done_in_epoch += 1
             if done_in_epoch >= spe:
                 done_in_epoch = 0
+                self._end_of_epoch(module, val)
                 module.current_epoch += 1
                 if module.current_epoch % self.save_every_n_epochs == 0:
                     save(f"tacorl_epoch_{module.current_epoch:02d}_.ckpt")
