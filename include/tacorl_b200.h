@@ -347,6 +347,14 @@ int tacorl_replay_gather_rows(int B, int n, int T, int pad, const int* tab, int 
                               int zero_pad, float* act_out, void* stream);
 int tacorl_metrics_accumulate(const tacorl_metrics* m, double* acc, void* stream);
 
+/* ---- per-step training metrics (tacorl_b200/runtime.py TrainMetricsRecorder; DESIGN.md section 15).
+ * metrics_record: ONE launch, one CTA of 32 threads, graph-capturable.  slot = *step_dev % ring_rows; thread i writes
+ *   *value[i] to ring[slot * 32 + i] and adds it to the fp64 sum acc[i] and 1 to the count acc[32 + i].  A NULL
+ *   value[i] (a key not logged in this mode) and every slot i >= k write NaN to the ring and leave acc alone.  Then
+ *   *step_dev += 1.  m->n is not read.  ring: ring_rows x 32 fp32; acc: 64 fp64. */
+int tacorl_metrics_record(const tacorl_metrics* m, float* ring, int ring_rows, long long* step_dev, double* acc,
+                          void* stream);
+
 /* ---- fused small-MLP chains (fp32): a whole Linear -> act -> Linear ... stack in ONE launch, forward or backward.
  * Replaces the per-layer launches behind VisualGoalEncoder.forward (goal_encoder.py:29-33), MLPPolicy.forward
  * (actor.py:252-270: 3 x Linear+SiLU, then fc_mean | fc_log_std as ONE layer of two weight segments) and

@@ -84,6 +84,7 @@ _SIGS = {
                             _i, _vp, _vp, _vp],
     "tacorl_replay_gather_rows": [_i, _i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tacorl_metrics_accumulate": [_vp, _vp, _vp],
+    "tacorl_metrics_record": [_vp, _vp, _i, _vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],
     "tacorl_mlp_chain_fwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp],
     "tacorl_mlp_chain_bwd": [_i, _i, _vp, _vp, _i, _ll, _vp, _i, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _sz, _vp],

@@ -155,6 +155,25 @@ __global__ void metrics_accumulate_kernel(const __grid_constant__ tacorl_metrics
   else if (i == m.k) acc[i] += (double)m.n;
 }
 
+// one training step's scalars into row (*step_dev % ring_rows) of the ring; acc[i] += value, acc[32 + i] += 1 for every
+// logged key.  32 threads always write the whole row (NaN for a null or unused slot), so a graph captured before a
+// later mode added a column leaves no stale entry behind.  One launch per step: every sum is taken in step order.
+__global__ void metrics_record_kernel(const __grid_constant__ tacorl_metrics m, float* __restrict__ ring, int ring_rows,
+                                      long long* __restrict__ step_dev, double* __restrict__ acc) {
+  const int i = threadIdx.x;
+  const long long slot = *step_dev % ring_rows;
+  const float* p = i < m.k ? m.value[i] : nullptr;
+  float v = __int_as_float(0x7fc00000);
+  if (p) {
+    v = *p;
+    acc[i] += (double)v;
+    acc[TACORL_METRICS_MAX + i] += 1.0;
+  }
+  ring[slot * TACORL_METRICS_MAX + i] = v;
+  __syncthreads();
+  if (i == 0) *step_dev += 1;
+}
+
 constexpr int kMaxImages = TACORL_REPLAY_MAX_IMAGES;
 
 struct GatherImage {
@@ -335,6 +354,17 @@ int tacorl_metrics_accumulate(const tacorl_metrics* m, double* acc, void* stream
   TACORL_REQUIRE(m->n > 0, "metrics_accumulate: batch of %d items", m->n);
   for (int i = 0; i < m->k; ++i) TACORL_REQUIRE(m->value[i], "metrics_accumulate: metric %d: null pointer", i);
   metrics_accumulate_kernel<<<1, 32 * ((m->k + 32) / 32), 0, (cudaStream_t)stream>>>(*m, acc);
+  TACORL_LAUNCH_CHECK();
+  return 0;
+}
+
+int tacorl_metrics_record(const tacorl_metrics* m, float* ring, int ring_rows, long long* step_dev, double* acc,
+                          void* stream) {
+  TACORL_REQUIRE(m && ring && step_dev && acc, "metrics_record: null pointer");
+  TACORL_REQUIRE(m->k >= 0 && m->k <= TACORL_METRICS_MAX, "metrics_record: %d metrics (at most %d)", m->k,
+                 TACORL_METRICS_MAX);
+  TACORL_REQUIRE(ring_rows >= 1, "metrics_record: %d ring rows", ring_rows);
+  metrics_record_kernel<<<1, TACORL_METRICS_MAX, 0, (cudaStream_t)stream>>>(*m, ring, ring_rows, step_dev, acc);
   TACORL_LAUNCH_CHECK();
   return 0;
 }

@@ -4,9 +4,13 @@ The step issues several hundred small launches (per-timestep recurrent GEMMs, pe
 kernels); replaying them from one captured graph removes the host launch / ctypes / autograd overhead that would
 otherwise dominate a ~ms step (SURVEY.md §7 "Host overhead").  Noise keeps advancing between replays (the torch
 CUDA generator is graph-aware) and the Adam bias correction reads a device-resident step counter."""
+import csv
 import ctypes
+from pathlib import Path
 
+import numpy as np
 import torch
+import torch.distributed as dist
 
 
 def _clone_to_static(batch, device):
@@ -307,3 +311,278 @@ def validation_step_fn(module, accumulator):
                              bool(getattr(module, "finetune_action_decoder", False)), bool(module.training))
     step.preserve = lambda: [accumulator.acc]
     return step
+
+
+def assign_columns(keys, names):
+    """Appends to `keys` (in place) every name it lacks, in order: a key keeps its column for good, because captured
+    graphs hold the ring's pointers.  Refuses more than METRICS_MAX keys.  Pure host function."""
+    from . import _lib
+    for k in names:
+        if k not in keys:
+            if len(keys) == _lib.METRICS_MAX:
+                raise ValueError(f"the step logs more than {_lib.METRICS_MAX} 'train/*' scalars ({k!r} is one too "
+                                 f"many); at most {_lib.METRICS_MAX} are recorded")
+            keys.append(k)
+    return keys
+
+
+def epoch_means(keys, totals):
+    """Epoch mean of every recorded training scalar.  `totals` holds one vector per rank: METRICS_MAX fp64 sums, then
+    METRICS_MAX counts (sums[i]: the values of keys[i] over the steps that logged it; counts[i]: those steps).  Ranks
+    are added before dividing, as Lightning aggregates `self.log(..., on_epoch=True, sync_dist=True)`; a key no step of
+    the epoch logged has no mean.  Pure host function."""
+    from . import _lib
+    M = _lib.METRICS_MAX
+    rows = [[float(x) for x in t] for t in totals]
+    if not rows or any(len(r) != 2 * M for r in rows):
+        raise ValueError(f"expected (sums, counts) vectors of {2 * M} entries")
+    total = [sum(col) for col in zip(*rows)]
+    return {k: total[i] / total[M + i] for i, k in enumerate(keys) if total[M + i] > 0}
+
+
+class RingBook:
+    """Host side of the metrics ring: the device counter puts the n-th recorded step (n counts from 0 since the ring
+    was made) in row n % (2 * half).  `advance` notes each step's (global step, epoch) and hands over a range when its
+    step fills a half; `take` hands over whatever is not handed over yet (epoch and fit end).  A range never spans two
+    halves, since a half boundary always ends one.  Pure host class."""
+
+    def __init__(self, half):
+        self.half, self.rows = int(half), 2 * int(half)
+        self.n = 0               # steps recorded
+        self.taken = 0           # steps handed over for read-back
+        self._steps, self._epochs = [], []
+
+    def advance(self, global_step, epoch):
+        """One more recorded step; returns `take()` when it filled a half, else None."""
+        self._steps.append(int(global_step))
+        self._epochs.append(int(epoch))
+        self.n += 1
+        return self.take() if self.n % self.half == 0 else None
+
+    def take(self):
+        """(first ring row, global steps, epochs) of steps [taken, n), or None when there are none."""
+        if self.taken == self.n:
+            return None
+        row0 = self.taken % self.rows
+        out = (row0, np.asarray(self._steps, np.int64), np.asarray(self._epochs, np.int32))
+        self._steps, self._epochs = [], []
+        self.taken = self.n
+        return out
+
+
+class TrainHistory:
+    """One row per training step, as numpy blocks in the order they were read back: `steps` (global step), `epochs`
+    and `values` (len(steps) x len(keys) fp32, NaN where the step did not log the key).  Pure host class."""
+
+    def __init__(self):
+        self.keys = []
+        self._blocks = []        # (steps, epochs, column index of each value column, values)
+
+    def append(self, keys, steps, epochs, values):
+        assign_columns(self.keys, keys)
+        cols = np.asarray([self.keys.index(k) for k in keys], np.int64)
+        self._blocks.append((np.asarray(steps, np.int64), np.asarray(epochs, np.int32), cols,
+                             np.asarray(values, np.float32)[:, :len(keys)]))
+
+    def __len__(self):
+        return sum(len(b[0]) for b in self._blocks)
+
+    @property
+    def steps(self):
+        return np.concatenate([b[0] for b in self._blocks]) if self._blocks else np.zeros(0, np.int64)
+
+    @property
+    def epochs(self):
+        return np.concatenate([b[1] for b in self._blocks]) if self._blocks else np.zeros(0, np.int32)
+
+    @property
+    def values(self):
+        out = np.full((len(self), len(self.keys)), np.nan, np.float32)
+        r = 0
+        for steps, _, cols, vals in self._blocks:
+            out[r:r + len(steps), cols] = vals
+            r += len(steps)
+        return out
+
+    def column(self, key):
+        return self.values[:, self.keys.index(key)]
+
+
+class MetricsCSV:
+    """`metrics.csv` in Lightning CSVLogger's layout: a header, then one row per logged step.  Columns: `step`,
+    `epoch`, every key (the step's values) and `<key>_epoch` for every key (the epoch means, in one row per epoch at the
+    epoch's last step).  Rows of steps >= `start_step` left by an earlier run are dropped (the run resumes from a
+    checkpoint written before them) and new rows are appended; a key that is new to the file rewrites it with the
+    wider header.  Pure host class."""
+
+    def __init__(self, path, start_step=0):
+        self.path = Path(path)
+        self.keys, rows = [], []
+        if self.path.is_file():
+            with open(self.path, newline="") as f:
+                r = csv.DictReader(f)
+                header = r.fieldnames or []
+                rows = list(r)
+            self.keys = [k for k in header if k not in ("step", "epoch") and not k.endswith("_epoch")]
+            keep = [row for row in rows if row.get("step") not in (None, "") and int(row["step"]) < int(start_step)]
+            if len(keep) != len(rows) or header != self._header():
+                self._rewrite(keep)
+        else:
+            self.path.parent.mkdir(parents=True, exist_ok=True)
+
+    def _header(self):
+        return ["step", "epoch"] + self.keys + [k + "_epoch" for k in self.keys]
+
+    def _rewrite(self, rows):
+        with open(self.path, "w", newline="") as f:
+            w = csv.DictWriter(f, fieldnames=self._header(), restval="")
+            w.writeheader()
+            w.writerows(rows)
+
+    def write(self, rows):
+        """rows: dicts of step, epoch and key (or `<key>_epoch`) -> value."""
+        if not rows:
+            return
+        new = [k for row in rows for k in row if k not in ("step", "epoch") and not k.endswith("_epoch")]
+        new += [k[:-len("_epoch")] for row in rows for k in row if k.endswith("_epoch")]
+        if [k for k in new if k not in self.keys] or not self.path.is_file():
+            old = []
+            if self.path.is_file():
+                with open(self.path, newline="") as f:
+                    old = list(csv.DictReader(f))
+            assign_columns(self.keys, new)
+            self._rewrite(old + [self._fmt(r) for r in rows])
+            return
+        with open(self.path, "a", newline="") as f:
+            csv.DictWriter(f, fieldnames=self._header(), restval="").writerows([self._fmt(r) for r in rows])
+
+    @staticmethod
+    def _fmt(row):
+        return {k: (v if k in ("step", "epoch") else repr(float(v))) for k, v in row.items()}
+
+
+def logging_rows(keys, steps, epochs, values, every):
+    """The CSV rows of a read-back block: the steps s with (s + 1) % every == 0, as Lightning's
+    `log_every_n_steps` logs them.  Pure host function."""
+    rows = []
+    for j in np.flatnonzero((np.asarray(steps) + 1) % int(every) == 0):
+        row = {"step": int(steps[j]), "epoch": int(epochs[j])}
+        row.update({k: float(values[j, i]) for i, k in enumerate(keys)})
+        rows.append(row)
+    return rows
+
+
+class TrainMetricsRecorder:
+    """Every training step's logged `train/*` scalars, recorded on the device with no host sync (DESIGN.md section 15).
+
+    `record(logged)` runs inside the step (and so inside its CUDA graph): one launch of tacorl_metrics_record writes the
+    step's values to row (counter % ring_rows) of a ring_rows x 32 fp32 ring, adds each to an fp64 sum and a per-key
+    count and advances the device counter.  Columns are the `train/*` keys in order of first appearance (at most 32); a
+    key a later mode adds takes the next column and a key the step did not log is NaN in its row.  A plain Python
+    number logged under `train/` is not recorded: it is a host value a captured graph would freeze.
+
+    `step_done(global_step, epoch)` runs on the host after each step.  When a half of the ring fills, the rows are
+    all-reduced to their mean over ranks on the training stream (between replays, in the same order on every rank), a
+    side stream copies them to a pinned buffer, and the training stream waits for the previous copy out of the other
+    half before it writes that half again.  Copies are read on the host at the next read-back, or by `flush()` (epoch and
+    fit end), into `history` and, when given, `csv`.  `end_epoch()` also returns the epoch means from the rank-summed
+    sums and counts.  `preserve()` lists the device state a step changes, so the warm-up steps of a capture record
+    nothing."""
+
+    def __init__(self, device, ring_rows, world=1, history=None, csv=None, log_every_n_steps=None):
+        from . import _lib
+        if int(ring_rows) < 2 or int(ring_rows) % 2:
+            raise ValueError(f"ring_rows must be an even number >= 2, got {ring_rows}")
+        device = torch.device(device)
+        self.device = device if device.index is not None else torch.device("cuda", torch.cuda.current_device())
+        self.ring_rows, self.half = int(ring_rows), int(ring_rows) // 2
+        self.world = int(world)
+        self.keys = []
+        M = _lib.METRICS_MAX
+        self.ring = torch.full((self.ring_rows, M), float("nan"), dtype=torch.float32, device=self.device)
+        self.acc = torch.zeros(2 * M, dtype=torch.float64, device=self.device)
+        self.counter = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self.pinned = [torch.empty((self.half, M), dtype=torch.float32, pin_memory=True) for _ in range(2)]
+        self.side = torch.cuda.Stream(device=self.device)
+        self._filled = [torch.cuda.Event() for _ in range(2)]
+        self._copied = [torch.cuda.Event() for _ in range(2)]
+        self._queue = []         # copies not read yet, oldest first: (half, first row in the half, steps, epochs, keys)
+        self.book = RingBook(self.half)
+        self.history = history if history is not None else TrainHistory()
+        self.csv = csv
+        self.every = int(log_every_n_steps or self.half)
+        self._hold = []
+
+    def record(self, logged):
+        from . import _lib
+        names = [k for k, v in logged.items() if k.startswith("train/") and torch.is_tensor(v)]
+        assign_columns(self.keys, names)
+        m = _lib.Metrics()
+        hold = []
+        for k in names:
+            v = logged[k]
+            if v.numel() != 1 or v.device != self.device:
+                raise ValueError(f"{k}: expected a one-element tensor on {self.device}, got {v!r}")
+            if v.dtype != torch.float32 or not v.is_contiguous():
+                v = v.float().contiguous()
+                hold.append(v)           # keeps the converted value alive while the launch reads it
+            m.value[self.keys.index(k)] = v.data_ptr()
+        m.k, m.n = len(self.keys), 1
+        self._hold = hold
+        _lib.call("tacorl_metrics_record", ctypes.byref(m), _lib.ptr(self.ring), self.ring_rows,
+                  _lib.ptr_any(self.counter), _lib.ptr_any(self.acc), _lib.stream())
+
+    def preserve(self):
+        return [self.counter, self.acc, self.ring]
+
+    def step_done(self, global_step, epoch):
+        got = self.book.advance(global_step, epoch)
+        if got is not None:
+            self._readback(got)
+
+    def _readback(self, got):
+        row0, steps, epochs = got
+        h, off, n = row0 // self.half, row0 % self.half, len(steps)
+        while any(q[0] == h for q in self._queue):       # the host has not read this half's previous copy yet
+            self._read_oldest()
+        main = torch.cuda.current_stream(self.device)
+        rows = self.ring[row0:row0 + n]
+        if self.world > 1:
+            dist.all_reduce(rows)                        # training stream, between replays: every rank in one order
+            rows.div_(self.world)
+        self._filled[h].record(main)
+        self.side.wait_event(self._filled[h])
+        with torch.cuda.stream(self.side):
+            self.pinned[h][off:off + n].copy_(rows, non_blocking=True)
+            self._copied[h].record(self.side)
+        self._queue.append((h, off, steps, epochs, list(self.keys)))
+        main.wait_event(self._copied[1 - h])             # the training stream writes the other half next
+        while self._queue and self._queue[0][0] != h and self._copied[self._queue[0][0]].query():
+            self._read_oldest(wait=False)                # copies already done: read without waiting
+
+    def _read_oldest(self, wait=True):
+        h, off, steps, epochs, keys = self._queue.pop(0)
+        if wait:
+            self._copied[h].synchronize()
+        vals = self.pinned[h][off:off + len(steps), :len(keys)].numpy().copy()
+        self.history.append(keys, steps, epochs, vals)
+        if self.csv is not None:
+            self.csv.write(logging_rows(keys, steps, epochs, vals, self.every))
+
+    def flush(self):
+        """Reads everything recorded so far back to the host (waits for it)."""
+        got = self.book.take()
+        if got is not None:
+            self._readback(got)
+        while self._queue:
+            self._read_oldest()
+
+    def end_epoch(self):
+        """flush(), then {key: epoch mean} from the sums and counts (summed over ranks), which are then zeroed."""
+        self.flush()
+        totals = self.acc.clone()
+        if self.world > 1:
+            dist.all_reduce(totals)
+        means = epoch_means(self.keys, [totals.cpu().tolist()])
+        self.acc.zero_()
+        return means

@@ -60,6 +60,20 @@ def restore_checkpoint(module, path, strict=True):
     return ckpt
 
 
+def _recording(step_fn, module, recorder):
+    """step(batch), then the record launch of the `train/*` tensors that step logged.  A key whose tensor is the very
+    object that was there before the step (`log` stores a new detached tensor each call) was not logged by it."""
+    def step(batch):
+        before = dict(module.logged)
+        out = step_fn(batch)
+        recorder.record({k: v for k, v in module.logged.items() if before.get(k) is not v})
+        return out
+    inner_preserve = step_fn.preserve
+    step.mode_key = step_fn.mode_key
+    step.preserve = lambda: list(inner_preserve()) + recorder.preserve()
+    return step
+
+
 class Trainer:
     """fit(module, batches) with the reference Trainer's knobs that matter on the hot path.
     batches: an iterable of batch dicts (host or device tensors), a callable step -> batch, or a DeviceReplay
@@ -72,10 +86,17 @@ class Trainer:
     Validation (`fit(..., val=)`, `validate`): every `check_val_every_n_epoch`-th epoch ends with a sweep of `val`, a
     DeviceReplay(mode="sweep") or a re-iterable of host batches, through the module's `validation_step`.  Each logged
     `validation/*` scalar becomes its item-weighted mean over the sweep (summed over ranks), in `callback_metrics` and
-    `val_history`.  A sweep runs in eval mode under a fixed generator seed and leaves the training run untouched."""
+    `val_history`.  A sweep runs in eval mode under a fixed generator seed and leaves the training run untouched.
+
+    Training metrics: every step's logged `train/*` tensors are recorded on the device inside the step (its CUDA graph
+    included) and read back every `log_every_n_steps` steps without a host sync (runtime.TrainMetricsRecorder,
+    DESIGN.md section 15).  `train_history` holds one row per step (mean over ranks), `train_epoch_metrics` the means of
+    the last finished epoch and `train_epoch_history` one (epoch, global_step, means) entry per finished epoch; with
+    `default_root_dir`, rank 0 also writes `metrics.csv`.  Python numbers logged under `train/` are not recorded."""
 
     def __init__(self, max_steps=-1, max_epochs=1, precision="bf16", use_cuda_graph=True, default_root_dir=None,
-                 steps_per_epoch=None, save_every_n_epochs=1, device=None, check_val_every_n_epoch=1):
+                 steps_per_epoch=None, save_every_n_epochs=1, device=None, check_val_every_n_epoch=1,
+                 log_every_n_steps=50):
         self.max_steps, self.max_epochs = max_steps, max_epochs
         self.precision = {"16": "bf16", 16: "bf16", "bf16": "bf16", "32": "fp32", 32: "fp32", "fp32": "fp32"}[precision]
         self.use_cuda_graph = use_cuda_graph
@@ -94,6 +115,14 @@ class Trainer:
         self.callback_metrics = {}
         self.val_history = []                 # (epoch, global_step, metrics) per sweep of fit()
         self._val_states = {}
+        if int(log_every_n_steps) < 1:
+            raise ValueError(f"log_every_n_steps must be >= 1, got {log_every_n_steps}")
+        self.log_every_n_steps = int(log_every_n_steps)
+        self.train_history = runtime.TrainHistory()
+        self.train_epoch_metrics = {}
+        self.train_epoch_history = []         # (epoch, global_step, {key: mean}) per finished epoch
+        self._recorder = None
+        self._train_graph = None
 
     def _setup_device(self, module):
         torch.cuda.set_device(self.device)
@@ -120,7 +149,9 @@ class Trainer:
         then samples every step's batch on the device (inside the step's CUDA graph).  With a replay, an epoch is
         `replay.steps_per_epoch` steps unless `steps_per_epoch` says otherwise, and checkpoints carry its step counter.
         val: validation data (see `validate`), swept at the end of every `check_val_every_n_epoch`-th epoch before
-        that epoch's checkpoint is written; checkpoints then carry the results under "validation"."""
+        that epoch's checkpoint is written; checkpoints then carry the results under "validation".
+        Checkpoints carry the training epoch means under "training"; a resume restores them and appends to
+        metrics.csv (dropping rows of steps at or after the checkpoint's)."""
         from .replay import DeviceReplay
         replay = batches if isinstance(batches, DeviceReplay) else None
         if replay is not None:
@@ -138,8 +169,16 @@ class Trainer:
             if "validation" in ckpt:
                 self.val_history = list(ckpt["validation"]["history"])
                 self.callback_metrics = dict(ckpt["validation"]["metrics"])
+            if "training" in ckpt:
+                self.train_epoch_history = list(ckpt["training"]["epoch_history"])
+                self.train_epoch_metrics = dict(ckpt["training"]["metrics"])
+        rec = self._recorder = runtime.TrainMetricsRecorder(
+            self.device, 2 * self.log_every_n_steps, world=self.world, history=self.train_history,
+            csv=runtime.MetricsCSV(self.root / "metrics.csv", self.global_step) if self.root and self.rank == 0 else None,
+            log_every_n_steps=self.log_every_n_steps)
+        step_fn = _recording(step_fn, module, rec)
         if replay is not None:
-            return self._fit_replay(module, step_fn, replay, val)
+            return self._fit_replay(module, step_fn, replay, val, rec)
         get = batches if callable(batches) else None
         it = None if get else iter(batches)
         graphed = None
@@ -158,24 +197,27 @@ class Trainer:
                 break
             if self.use_cuda_graph:
                 if graphed is None:
-                    graphed = runtime.GraphedTrainStep(step_fn, batch, device=self.device, warmup=2)
+                    graphed = self._train_graph = runtime.GraphedTrainStep(step_fn, batch, device=self.device, warmup=2)
                 out = graphed(batch)
             else:
                 out = step_fn(_to_device(batch, self.device))
             if torch.is_tensor(out):
                 self.losses.append(out.detach().clone())
+            rec.step_done(self.global_step, module.current_epoch)
             self.global_step += 1
             done_in_epoch += 1
             if self.steps_per_epoch and done_in_epoch >= self.steps_per_epoch:
                 done_in_epoch = 0
+                self._train_epoch_end(module, rec)
                 self._end_of_epoch(module, val)
                 module.current_epoch += 1          # (a graph captured for the BC epochs is swapped when bc_epochs is crossed)
                 if self.root and self.rank == 0 and module.current_epoch % self.save_every_n_epochs == 0:
                     save_checkpoint(module, self.root / "saved_models" / f"tacorl_epoch_{module.current_epoch:02d}_.ckpt",
-                                    module.current_epoch, self.global_step, extra=self._val_extra(val))
+                                    module.current_epoch, self.global_step, extra=self._ckpt_extra(val))
+        rec.flush()
         if self.root and self.rank == 0:
             save_checkpoint(module, self.root / "saved_models" / "last.ckpt", module.current_epoch, self.global_step,
-                            extra=self._val_extra(val))
+                            extra=self._ckpt_extra(val))
         torch.cuda.synchronize(self.device)
         return self
 
@@ -198,10 +240,21 @@ class Trainer:
         elif callable(val) or not hasattr(val, "__iter__"):
             raise ValueError("val= takes a sweep-mode DeviceReplay or a re-iterable of batch dicts")
 
-    def _val_extra(self, val):
-        if val is None:
-            return None
-        return {"validation": {"metrics": dict(self.callback_metrics), "history": list(self.val_history)}}
+    def _ckpt_extra(self, val):
+        extra = {"training": {"metrics": dict(self.train_epoch_metrics), "epoch_history": list(self.train_epoch_history)}}
+        if val is not None:
+            extra["validation"] = {"metrics": dict(self.callback_metrics), "history": list(self.val_history)}
+        return extra
+
+    def _train_epoch_end(self, module, rec):
+        """The finished epoch's means of every recorded `train/*` key (rank-summed sums over rank-summed counts)."""
+        means = rec.end_epoch()
+        self.train_epoch_metrics = means
+        self.train_epoch_history.append((int(module.current_epoch), int(self.global_step), dict(means)))
+        if rec.csv is not None and means:
+            row = {"step": self.global_step - 1, "epoch": int(module.current_epoch)}
+            row.update({k + "_epoch": v for k, v in means.items()})
+            rec.csv.write([row])
 
     def _end_of_epoch(self, module, val):
         """Lightning's rule: validate after epoch e when (e + 1) % check_val_every_n_epoch == 0 (current_epoch = e)."""
@@ -271,7 +324,7 @@ class Trainer:
                 for m, training in flags:
                     m.training = training
 
-    def _fit_replay(self, module, step_fn, replay, val=None):
+    def _fit_replay(self, module, step_fn, replay, val, rec):
         spe = self.steps_per_epoch or replay.steps_per_epoch
         graphed = None
         epoch0 = int(getattr(module, "current_epoch", 0))
@@ -280,7 +333,7 @@ class Trainer:
         def save(name):
             if self.root and self.rank == 0:
                 extra = {"replay": replay.state_dict()}
-                extra.update(self._val_extra(val) or {})
+                extra.update(self._ckpt_extra(val))
                 save_checkpoint(module, self.root / "saved_models" / name, module.current_epoch, self.global_step,
                                 extra=extra)
         while not (self.max_steps >= 0 and self.global_step >= self.max_steps):
@@ -288,20 +341,24 @@ class Trainer:
                 break
             if self.use_cuda_graph:
                 if graphed is None:
-                    graphed = runtime.GraphedTrainStep(step_fn, None, device=self.device, warmup=2, source=replay)
+                    graphed = self._train_graph = runtime.GraphedTrainStep(step_fn, None, device=self.device, warmup=2,
+                                                                           source=replay)
                 out = graphed()
             else:
                 out = step_fn(replay.sample())
             if torch.is_tensor(out):
                 self.losses.append(out.detach().clone())
+            rec.step_done(self.global_step, module.current_epoch)
             self.global_step += 1
             done_in_epoch += 1
             if done_in_epoch >= spe:
                 done_in_epoch = 0
+                self._train_epoch_end(module, rec)
                 self._end_of_epoch(module, val)
                 module.current_epoch += 1
                 if module.current_epoch % self.save_every_n_epochs == 0:
                     save(f"tacorl_epoch_{module.current_epoch:02d}_.ckpt")
+        rec.flush()
         save("last.ckpt")
         torch.cuda.synchronize(self.device)
         return self
