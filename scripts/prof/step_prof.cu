@@ -115,5 +115,53 @@ int main(int argc, char** argv) {
     for (int i = 0; i < 11; ++i) printf("  %-26s t=%6lld cyc (+%lld)\n", nm[i], h[i] - h[0], i ? h[i] - h[i - 1] : 0);
 #endif
   }
+  for (int n_lanes = 1; n_lanes <= 2; ++n_lanes) {  // two-lane persistent recurrence at batch 64: STEPS steps per lane
+    const int MW = 64, T = STEPS + 1;
+    __nv_bfloat16* hb[2]; float* Cs[2]; unsigned* flags[2];
+    WaveLaneHost lanes[2];
+    for (int l = 0; l < n_lanes; ++l) {
+      cudaMalloc(&hb[l], (size_t)T * MW * N * 2); cudaMalloc(&Cs[l], (size_t)T * MW * N * 4); cudaMalloc(&flags[l], 256);
+      cudaMemset(hb[l], 0, (size_t)T * MW * N * 2); cudaMemset(Cs[l], 0, (size_t)T * MW * N * 4);
+      WaveLaneHost& h = lanes[l];
+      h.Ab = hb[l]; h.lda = K; h.a_ts = (long long)MW * K; h.W = W; h.ldw = K;
+      h.tau0 = l ? T - 2 : 1; h.dtau = l ? -1 : 1; h.n_steps = STEPS; h.beta = 1.f;
+      h.C = Cs[l]; h.ldc = N; h.c_ts = (long long)MW * N; h.Cb = hb[l]; h.ldcb = N; h.cb_ts = (long long)MW * N;
+      h.act = ACT_RELU; h.flags = flags[l];
+    }
+    auto run = [&]() {
+      int rc = rnn_wave_tc(lanes, n_lanes, T, MW, N, K, st);
+      if (rc) { printf("rnn_wave_tc rc=%d %s\n", rc, tacorl_last_error()); exit(1); }
+    };
+    run(); cudaStreamSynchronize(st);
+    for (int i = 0; i < 3; ++i) run();
+    cudaEventRecord(e0, st);
+    for (int i = 0; i < 10; ++i) run();
+    cudaEventRecord(e1, st);
+    cudaStreamSynchronize(st);
+    float ms; cudaEventElapsedTime(&ms, e0, e1);
+    printf("wave %d-lane (M=%d): %.2f us per dependent step (%d steps per launch), timeouts %u, %s\n", n_lanes, MW,
+           ms * 1000 / (10 * STEPS), STEPS, rnn_seq_timeouts(), cudaGetErrorString(cudaGetLastError()));
+#ifdef TACORL_STEP_PROFILE
+    long long h[48];
+    cudaMemcpyFromSymbol(h, g_wave_prof, sizeof(h));
+    const char* nm[12] = {"issuer: step start", "flags ok", "all TMA issued", "epi: previous S free",
+                          "mma issued+commit", "epi: mma done", "S stored", "cluster sync", "dsmem summed + arrive",
+                          "bf16 stored + fence", "flag released", "fp32 stored"};
+    printf("  stage stamps of CTA (1, 3) at step 32, cycles after the issuer's step start:\n");
+    for (int i = 0; i < 48; ++i) {
+      if (i > 0 && h[i] == 0) continue;
+      char buf[64];
+      if (i < 12) snprintf(buf, sizeof(buf), "%s", nm[i]);
+      else if (i >= 16 && i < 24) snprintf(buf, sizeof(buf), "K block %d landed", i - 16);
+      else if (i >= 24 && i < 32) snprintf(buf, sizeof(buf), "K block %d counters seen", i - 24);
+      else if (i >= 32 && i < 40) snprintf(buf, sizeof(buf), "K block %d TMA issued", i - 32);
+      else snprintf(buf, sizeof(buf), "stamp %d", i);
+      printf("  %-26s t=%6lld cyc\n", buf, h[i] - h[0]);
+    }
+    const long long zero[48] = {};
+    cudaMemcpyToSymbol(g_wave_prof, zero, sizeof(zero));
+#endif
+    for (int l = 0; l < n_lanes; ++l) { cudaFree(hb[l]); cudaFree(Cs[l]); cudaFree(flags[l]); }
+  }
   return 0;
 }

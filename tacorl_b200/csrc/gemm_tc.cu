@@ -650,6 +650,16 @@ __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
 __device__ __forceinline__ void red_release_gpu_add(unsigned* p, unsigned v) {
   asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
+// Spins until the arrival counters flags[j_lo..j_hi] have all reached `want` (acquire, gpu scope).  Returns false after a
+// bounded wait (counted in g_rnn_seq_timeouts) so that a violated co-residency assumption cannot hang the launch.
+__device__ __forceinline__ bool rnn_wait_tiles(const unsigned* flags, int j_lo, int j_hi, unsigned want) {
+  for (int j = j_lo; j <= j_hi; ++j) {
+    unsigned spins = 0;
+    while (ld_acquire_gpu(flags + j) < want)
+      if (++spins > (1u << 21)) { atomicAdd(&g_rnn_seq_timeouts, 1u); return false; }
+  }
+  return true;
+}
 
 __global__ void __cluster_dims__(RS_KS, 1, 1) __launch_bounds__(RS_THREADS, 1)
 rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, const SeqArgs sa,
@@ -692,8 +702,6 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     for (int s = 0; s < kb_per_cta; ++s)
       tma_load_2d(smem_u32(w_smem + (size_t)s * W_STAGE), &tmW, k_begin + s * TC_BK, n0, w_bar);
   }
-  // tiles whose columns intersect my K slab [k_begin, k_begin + kb*64)
-  const int j_lo = k_begin / NT, j_hi = min(tiles - 1, (k_begin + kb_per_cta * TC_BK - 1) / NT);
   const int NT4 = NT >> 2, elems = per * NT4;
   bool dead = false;                                                    // a flag wait timed out: stop waiting
 
@@ -702,29 +710,22 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const uint32_t ph = (uint32_t)step & 1u;
     float4 cold[RS_MAXE], gt[RS_MAXE];
     if (warp == RS_EPI / 32) {
-      if (step > 0 && !dead) {      // one lane per producing tile, polled in parallel
-        const unsigned want = (unsigned)(RS_KS * step);
-        bool bad = false;
-        for (int j = j_lo + lane; j <= j_hi; j += 32) {
-          unsigned spins = 0;
-          while (ld_acquire_gpu(&g_rnn_flags[0][j]) < want) {
-            if (++spins > (1u << 21)) { bad = true; atomicAdd(&g_rnn_seq_timeouts, 1u); break; }
-          }
-        }
-        if (__any_sync(0xffffffffu, bad)) dead = true;
-        __threadfence();
-        __syncwarp();
-      }
-      if (lane == 0) {
-        SQ_STAMP(0)
-        if (step == 0) mbar_wait(w_bar, 0);
-        SQ_STAMP(1)
+      // lane s waits for the (one or two) tiles producing K block s and loads that block (as in rnn_wave_kernel)
+      if (lane == 0) { SQ_STAMP(0) }
+      bool bad = false;
+      if (lane < kb_per_cta) {
+        const int k0 = k_begin + lane * TC_BK;
+        if (step > 0 && !dead)
+          bad = !rnn_wait_tiles(g_rnn_flags[0], k0 / NT, min(tiles - 1, (k0 + TC_BK - 1) / NT), (unsigned)(RS_KS * step));
         asm volatile("fence.proxy.async.global;" ::: "memory");
-        for (int s = 0; s < kb_per_cta; ++s) {
-          const uint32_t bar = smem_u32(bars + s);
-          mbar_expect_tx(bar, (uint32_t)Mpad * 128);
-          tma_load_3d(smem_u32(a_smem + (size_t)s * A_TILE), &tmA, k_begin + s * TC_BK, 0, tau - sa.dtau, bar);
-        }
+        const uint32_t bar = smem_u32(bars + lane);
+        mbar_expect_tx(bar, (uint32_t)Mpad * 128);
+        tma_load_3d(smem_u32(a_smem + (size_t)lane * A_TILE), &tmA, k0, 0, tau - sa.dtau, bar);
+      }
+      if (__any_sync(0xffffffffu, bad)) dead = true;
+      if (lane == 0) {
+        SQ_STAMP(1)
+        if (step == 0) mbar_wait(w_bar, 0);
         const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
         SQ_STAMP(2)
         for (int s = 0; s < kb_per_cta; ++s) {
@@ -847,7 +848,8 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       asm volatile("fence.proxy.async.global;" ::: "memory");
       if (tid == 0) { SQ_STAMP(9) }
       asm volatile("bar.sync 1, %0;" ::"n"(RS_EPI) : "memory");
-      if (tid == 0) { __threadfence(); red_release_gpu_add(&g_rnn_flags[0][tile], 1u); SQ_STAMP(10) }
+      // (the release is cumulative over the stores bar.sync ordered before it: no separate fence)
+      if (tid == 0) { red_release_gpu_add(&g_rnn_flags[0][tile], 1u); SQ_STAMP(10) }
 #pragma unroll
       for (int i = 0; i < RS_MAXE; ++i) {
         const int e = tid + i * RS_EPI;
@@ -889,6 +891,12 @@ struct WaveLane {
   unsigned* flags;                        // [tiles] arrival counters, zero before the launch
 };
 struct WaveArgs { WaveLane lane[2]; };
+#ifdef TACORL_STEP_PROFILE                    // stage stamps of one CTA at step 32 (scripts/prof/step_prof.cu)
+__device__ long long g_wave_prof[48];
+#define WV_STAMP(i) if (step == 32 && blockIdx.x == 1 && blockIdx.y == 3 && blockIdx.z == 0) g_wave_prof[i] = clock64();
+#else
+#define WV_STAMP(i)
+#endif
 
 __global__ void __launch_bounds__(RS_THREADS, 1)
 rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmW0,
@@ -936,8 +944,6 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     for (int s = 0; s < kb_per_cta; ++s)
       tma_load_2d(smem_u32(w_smem + (size_t)s * W_STAGE), tmW, k_begin + s * TC_BK, n0, w_bar);
   }
-  // tiles whose columns intersect my K slab [k_begin, k_begin + kb*64)
-  const int j_lo = k_begin / NT, j_hi = min(tiles - 1, (k_begin + kb_per_cta * TC_BK - 1) / NT);
   const int NT4 = NT >> 2, elems = per * NT4;
   bool dead = false;                                                    // a flag wait timed out: stop waiting
 
@@ -946,33 +952,31 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     const uint32_t ph = (uint32_t)step & 1u;
     float4 cold[RS_MAXE], gt[RS_MAXE];
     if (warp == RS_EPI / 32) {
-      // the producing tiles' arrival counters are polled by one lane each, in parallel (a dependent chain of up to four
-      // L2 round trips by a single lane cost ~1 us per step)
-      if (step > 0 && !dead) {
-        const unsigned want = (unsigned)(RW_KS * step);
-        bool bad = false;
-        for (int j = j_lo + lane; j <= j_hi; j += 32) {
-          unsigned spins = 0;
-          while (ld_acquire_gpu(&g_rnn_flags[blockIdx.z][j]) < want) {
-            if (++spins > (1u << 21)) { bad = true; atomicAdd(&g_rnn_seq_timeouts, 1u); break; }
-          }
-        }
-        if (__any_sync(0xffffffffu, bad)) dead = true;
-        __threadfence();          // the lanes' acquires, made cumulative for lane 0's TMA issue below
-        __syncwarp();
-      }
-      if (lane == 0) {
-        if (step == 0) mbar_wait(w_bar, 0);
+      // K block s of the h slab is loaded by lane s as soon as the tiles that produce it have all arrived: when the
+      // slowest producer arrives, only its own blocks are still to be fetched.  Each lane's TMA read is ordered after
+      // its own acquire by the proxy fence.
+      if (lane == 0) { WV_STAMP(0) }
+      bool bad = false;
+      if (lane < kb_per_cta) {
+        const int k0 = k_begin + lane * TC_BK;
+        if (step > 0 && !dead)
+          bad = !rnn_wait_tiles(g_rnn_flags[blockIdx.z], k0 / NT, min(tiles - 1, (k0 + TC_BK - 1) / NT), (unsigned)(RW_KS * step));
+        WV_STAMP(24 + lane)
         asm volatile("fence.proxy.async.global;" ::: "memory");
-        for (int s = 0; s < kb_per_cta; ++s) {
-          const uint32_t bar = smem_u32(bars + s);
-          mbar_expect_tx(bar, A_PITCH);
-          tma_load_3d(smem_u32(a_smem + (size_t)s * A_PITCH), tmA, k_begin + s * TC_BK, 0, tau - sa.dtau, bar);
-        }
+        const uint32_t bar = smem_u32(bars + lane);
+        mbar_expect_tx(bar, A_PITCH);
+        tma_load_3d(smem_u32(a_smem + (size_t)lane * A_PITCH), tmA, k0, 0, tau - sa.dtau, bar);
+        WV_STAMP(32 + lane)
+      }
+      if (__any_sync(0xffffffffu, bad)) dead = true;
+      if (lane == 0) {
+        WV_STAMP(2)
+        if (step == 0) mbar_wait(w_bar, 0);
         const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
         for (int s = 0; s < kb_per_cta; ++s) {
           mbar_wait(smem_u32(bars + s), ph);
           tc_fence_after();
+          WV_STAMP(16 + s)
           const uint32_t a_src = smem_u32(a_smem + (size_t)s * A_PITCH), w_src = smem_u32(w_smem + (size_t)s * W_STAGE);
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
@@ -980,6 +984,7 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
                         (s > 0 || k > 0) ? 1u : 0u);
         }
         tc_commit(done_bar);
+        WV_STAMP(4)
       }
       __syncwarp();
     } else {
@@ -1002,8 +1007,10 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       for (int i = 0; i < RS_MAXE; ++i) gt[i] = Gt ? *reinterpret_cast<const float4*>(Gt + offg[i]) : one;
       mbar_wait(done_bar, ph);
       tc_fence_after();
+      if (tid == 0) { WV_STAMP(5) }
     }
     if (step > 0) asm volatile("barrier.cluster.wait.aligned;" ::: "memory");   // peers finished reading my previous S
+    if (tid == 0) { WV_STAMP(3) }
     if (warp < RS_EPI / 32) {
       const int q = warp & 3;
       if (q * 32 < Mpad) {
@@ -1028,8 +1035,10 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       }
     }
     tc_fence_before();
+    if (tid == 0) { WV_STAMP(6) }
     cluster_sync_all();
     tc_fence_after();
+    if (tid == 0) { WV_STAMP(7) }
     float4 acc[RS_MAXE];
     if (warp < RS_EPI / 32) {
       float4 part[RS_MAXE][RW_KS];
@@ -1052,6 +1061,7 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
 #pragma unroll
       for (int i = 0; i < RS_MAXE; ++i) dep += acc[i].x + acc[i].y + acc[i].z + acc[i].w;
       asm volatile("barrier.cluster.arrive.release.aligned;" ::"f"(dep) : "memory");
+      if (tid == 0) { WV_STAMP(8) }
       // epilogue: the bf16 copy (the next step's operand) first, then the arrival, then the fp32 store
       float* Ct = sa.C + (long long)tau * sa.c_ts;
       __nv_bfloat16* Bt = sa.Cb + (long long)tau * sa.cb_ts;
@@ -1079,14 +1089,17 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         }
       }
       asm volatile("fence.proxy.async.global;" ::: "memory");
+      if (tid == 0) { WV_STAMP(9) }
       asm volatile("bar.sync 1, %0;" ::"n"(RS_EPI) : "memory");
-      if (tid == 0) { __threadfence(); red_release_gpu_add(&g_rnn_flags[blockIdx.z][tile], 1u); }
+      // (the release is cumulative over the stores bar.sync ordered before it: no separate fence)
+      if (tid == 0) { red_release_gpu_add(&g_rnn_flags[blockIdx.z][tile], 1u); WV_STAMP(10) }
 #pragma unroll
       for (int i = 0; i < RS_MAXE; ++i) {
         const int e = tid + i * RS_EPI;
         const int bi = e / NT4, n = (e - bi * NT4) * 4, b = (int)rank * per + bi, col = n0 + n;
         if (okv[i]) *reinterpret_cast<float4*>(Ct + (long long)b * sa.ldc + col) = outv[i];
       }
+      if (tid == 0) { WV_STAMP(11) }
     } else {
       asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     }
