@@ -397,6 +397,32 @@ int tacorl_adam_step(long long n, float* p, const float* g, float* m, float* v, 
 int tacorl_adam_step_range(long long n, float* p, const float* g, float* m, float* v, float lr, float beta1,
                            float beta2, float eps, int step, int* step_dev, int increment_step, int background,
                            float grad_scale, const float* sqnorm, float max_norm, void* shadow_bf16, void* stream);
+
+/* ---- batched rollout: one control step of ActionDecoderLogistic.act (action_decoder_logistic.py:116-122) for n
+ * independent environments, 1 <= n <= 64 (tacorl_b200/rollout.py, DESIGN.md section 16).  Three graph-capturable
+ * launches (layer 0, layer 1, heads + sample); no allocation, no host synchronisation.
+ *   plan (n, P), emb (n, E): the decoder input [plan | emb], fp32, P and E multiples of 4;
+ *   hidden (2, n, H): the recurrent state, read and updated in place; H a multiple of 8;
+ *   restart (n) int32: a non-zero row starts from h = 0 (clear_hidden_state()); the call does not clear it;
+ *   w: 16 fp32 tensors, rnn.{weight_ih_l0, weight_hh_l0, bias_ih_l0, bias_hh_l0, weight_ih_l1, weight_hh_l1, bias_ih_l1,
+ *      bias_hh_l1}, {prob_fc, mean_fc, log_scale_fc, gripper_fc}.{weight, bias}, 16-byte aligned;
+ *   w_bf16: NULL or 8 bf16 operand copies (entries may be NULL) of weight_ih_l0, weight_hh_l0, weight_ih_l1,
+ *      weight_hh_l1, prob_fc, mean_fc, log_scale_fc, gripper_fc weights; PREC_BF16 reads them instead of rounding the
+ *      fp32 weights itself (the same values);
+ *   noise: counter-based Philox4x32-10 with key (lo32(seed), hi32(seed)); row r's uniform i < 66 is word i mod 4 of
+ *      the draw with counter (lo32(t[r]), hi32(t[r]), env_id[r], i div 4), as (w >> 8) 2^-24; i < 60 is u1[i / 10][i %
+ *      10], i >= 60 is u2[i - 60]; then tacorl_dlm_sample's transforms.  t (n) int64 is incremented by the call;
+ *   actions (n, 7); logits: NULL or (n, 182) [prob 60 | mean 60 | log_scale 60 | gripper 2];
+ *   ws: tacorl_rollout_ws_bytes(n, H) bytes, ZERO-FILLED before its first use (it holds a completion counter that
+ *      every call leaves at zero).  Calls that share a ws must be stream-ordered.
+ *   prec: PREC_F32 = fp32 FFMA; PREC_BF16 = operands rounded to bf16 (nearest even), fp32 accumulation.
+ * Every output element is reduced in an order that depends neither on n nor on the other rows: a row's hidden state,
+ * logits and action are bit-identical whether it runs alone or in a batch. */
+size_t tacorl_rollout_ws_bytes(int n, int H);
+int tacorl_rollout_decoder_step(int n, int P, int E, int H, const float* plan, const float* emb, float* hidden,
+                                const int* restart, const float* const* w, const void* const* w_bf16,
+                                unsigned long long seed, const int* env_id, long long* t, float grip_lo, float grip_hi,
+                                float* actions, float* logits, void* ws, size_t ws_bytes, int prec, void* stream);
 int tacorl_polyak_update(long long n, float* target, const float* source, float tau, void* stream);
 int tacorl_sqnorm(long long n, const float* x, float* out, float* ws, void* stream);
 

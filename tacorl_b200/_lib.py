@@ -83,6 +83,9 @@ _SIGS = {
     "tacorl_replay_sweep": [_i, _i, _i, _i, _i, ctypes.c_ulonglong, ctypes.c_ulonglong, _i, _vp, _vp, _ll, _vp, _ll, _vp,
                             _i, _vp, _vp, _vp],
     "tacorl_replay_gather_rows": [_i, _i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "tacorl_rollout_ws_bytes": [_i, _i],
+    "tacorl_rollout_decoder_step": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp, _f, _f,
+                                    _vp, _vp, _vp, _sz, _i, _vp],
     "tacorl_metrics_accumulate": [_vp, _vp, _vp],
     "tacorl_metrics_record": [_vp, _vp, _i, _vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],
@@ -101,7 +104,7 @@ _SIGS = {
 }
 _RESTYPES = {
     "tacorl_lmp_encoder_ws_bytes": _sz, "tacorl_rnn_layer_ws_bytes": _sz, "tacorl_rnn_layer2_ws_bytes": _sz,
-    "tacorl_mlp_chain_ws_bytes": _sz,
+    "tacorl_mlp_chain_ws_bytes": _sz, "tacorl_rollout_ws_bytes": _sz,
     "tacorl_last_error": ctypes.c_char_p, "tacorl_launch_count": ctypes.c_ulonglong,
     "tacorl_rnn_seq_timeouts": ctypes.c_uint,
 }

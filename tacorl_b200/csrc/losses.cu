@@ -4,12 +4,10 @@
 // Citations are into /root/reference/src/tacorl/.
 #include "common.cuh"
 #include "internal.h"
+#include "dlm_sample.cuh"
 #include "../../include/tacorl_b200.h"
 
 namespace tacorl {
-
-constexpr int kMix = 10;    // n_mixtures (config/networks/action_decoder/logistic.yaml:2)
-constexpr float kLogSigMin = -5.f;
 
 __device__ __forceinline__ float sigmoid_acc(float x) { return 1.f / (1.f + expf(-x)); }
 __device__ __forceinline__ float softplus_acc(float x) { return x > 20.f ? x : log1pf(expf(x)); }
@@ -109,20 +107,10 @@ __global__ void dlm_sample_kernel(int rows, int A, const float* __restrict__ log
   if (idx >= rows * A) return;
   const int r = idx / A, d = idx % A;
   const float* L = logits + (long long)r * ld;
-  const float r1 = 1e-5f, r2 = 1.f - 1e-5f;
-  int best = 0; float bv = -INFINITY;
-#pragma unroll
-  for (int k = 0; k < kMix; ++k) {
-    const float t = (r1 - r2) * u1[((long long)r * A + d) * kMix + k] + r2;
-    const float v = L[d * kMix + k] - logf(-logf(t));
-    if (v > bv) { bv = v; best = k; }
-  }
-  const float mu = L[A * kMix + d * kMix + best];
-  const float s = fmaxf(L[2 * A * kMix + d * kMix + best], kLogSigMin);
-  const float u = (r1 - r2) * u2[(long long)r * A + d] + r2;
-  pred[(long long)r * (A + 1) + d] = mu + expf(s) * (logf(u) - logf(1.f - u));
+  const float* u1d = u1 + ((long long)r * A + d) * kMix;
+  pred[(long long)r * (A + 1) + d] = dlm_sample_dim(L, A, d, [&](int k) { return u1d[k]; }, u2[(long long)r * A + d]);
   if (d == 0) {
-    const float g = (L[3 * A * kMix + 1] > L[3 * A * kMix]) ? grip_hi : grip_lo;
+    const float g = dlm_gripper(L, A, grip_lo, grip_hi);
     pred[(long long)r * (A + 1) + A] = g;
     if (hit && actions) hit[r] = ((g > 0.f ? 1.f : -1.f) == actions[(long long)r * lda + A]) ? 1.f : 0.f;
   }

@@ -1,0 +1,290 @@
+"""Batched rollout policy of a trained TACO-RL agent: many environments, one CUDA-graph replay per control step.
+
+The reference's policy entry is single-environment and stateful (rollout_manager.py:364-386): a deterministic latent
+plan from the visual actor, `clear_hidden_state()`, then one `act()` per control step, with ONE hidden state and one
+`torch.rand` draw for the whole batch.  `RolloutPolicy` keeps per-environment plans, hidden states, goals and step
+counters on the device, so environments reset, change subtask and replan independently, and draws each environment's
+sampling noise from its own counter (Philox4x32-10 keyed by the seed, counter = (step, env_id, draw)): an
+environment's noise depends only on the seed, its env_id and its own step count, never on which other environments
+share the batch, and the decoder step is batch-invariant.  DESIGN.md section 16 states the rules.
+
+    policy = RolloutPolicy(tacorl_module, n_envs, seed=0)
+    policy.reset(rows, goal)        # goal images of these environments; their step counters restart at 0
+    actions = policy.step(obs)      # {modality: (n_envs, 3, H, W)} uint8 or normalised fp32 -> (n_envs, 7)
+
+The decoder step is `tacorl_rollout_decoder_step` (csrc/rollout.cu); the encoders and the actor run through the same
+library kernels as training.  Nothing here changes the module: `act()`, `clear_hidden_state()` and training are
+untouched."""
+import ctypes
+
+import numpy as np
+import torch
+
+from . import _lib as L
+from . import ops
+
+MAX_ENVS = 64
+
+
+def _rows_list(rows, n):
+    if torch.is_tensor(rows):
+        rows = rows.detach().cpu().reshape(-1).tolist()
+    elif isinstance(rows, (int, np.integer)):
+        rows = [rows]
+    out = []
+    for r in rows:
+        if isinstance(r, (bool, np.bool_)) or not isinstance(r, (int, np.integer)):
+            raise ValueError(f"rows must be integers, got {r!r}")
+        if not 0 <= int(r) < n:
+            raise ValueError(f"row {int(r)} out of range for {n} environments")
+        out.append(int(r))
+    if not out:
+        raise ValueError("no rows given")
+    if len(set(out)) != len(out):
+        raise ValueError(f"duplicate rows {out}")
+    return out
+
+
+def decoder_weights(decoder):
+    """The 16 fp32 tensors of tacorl_rollout_decoder_step, in the order of include/tacorl_b200.h."""
+    rnn = decoder.rnn
+    w = [getattr(rnn, f"{k}_l{l}") for l in range(2) for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")]
+    for fc in (decoder.prob_fc, decoder.mean_fc, decoder.log_scale_fc, decoder.gripper_fc):
+        w += [fc.weight, fc.bias]
+    return [t.detach() for t in w]
+
+
+def decoder_step(decoder, plan, emb, hidden, restart, seed, env_id, t, actions, logits=None, ws=None):
+    """One control step of `decoder` (an ActionDecoderLogistic) for n = plan.shape[0] environments, in the current
+    precision mode: hidden (2, n, H) and t (n, int64) are updated in place, actions (n, 7) and logits (n, 182, optional)
+    are written.  ws: a zero-filled uint8 buffer of tacorl_rollout_ws_bytes(n, H) bytes kept between calls (a fresh one
+    is allocated when None)."""
+    n, P = plan.shape
+    E, H = emb.shape[1], hidden.shape[2]
+    w = decoder_weights(decoder)
+    for x in w:
+        if not x.is_contiguous():
+            raise ValueError("decoder weights must be contiguous")
+    shadows = [ops.shadow_of(w[i]) for i in (0, 1, 4, 5, 8, 10, 12, 14)]
+    if ws is None:
+        ws = torch.zeros(int(L.query("tacorl_rollout_ws_bytes", n, H)), dtype=torch.uint8, device=plan.device)
+    L.call("tacorl_rollout_decoder_step", n, P, E, H, L.ptr(plan), L.ptr(emb), L.ptr(hidden), L.ptr_any(restart),
+           L.ptr_array(w), L.ptr_array(shadows), ctypes.c_ulonglong(int(seed) & 0xFFFFFFFFFFFFFFFF), L.ptr_any(env_id),
+           L.ptr_any(t), float(decoder._grip[0]), float(decoder._grip[1]), L.ptr(actions), L.ptr(logits),
+           ctypes.c_void_p(ws.data_ptr()), ws.numel(), ops._STATE["prec"], L.stream())
+    return actions
+
+
+class RolloutPolicy:
+    """Batched deterministic-plan rollout of a TACO-RL module (eval mode, on its CUDA device) for 1..64 environments.
+
+    reset(rows, goal)    new episode: goal images for these rows, step counter 0, replan at their next step
+    set_goal(rows, goal) next subtask: new goal, replan at the next step, step counter kept
+    replan(rows)         new plan and zero hidden state at the next step (every plan_duration steps)
+    step(obs)            one control step of every environment -> (n_envs, 7) actions
+
+    A replanning row takes the plan of the reference's deterministic actor call, tanh(mean) of the actor on its encoder
+    embedding of the current observation and the goal embedding goal_encoder(encoder(goal)) (computed once, at
+    reset / set_goal); its hidden state restarts at zero and its first decoder step uses the same frame.  The decoder
+    consumes perceptual_encoder.get_state_from_observation(obs, action_decoder_modalities), as `act()` does.
+
+    Each step is one CUDA-graph replay of one of two graphs, with and without a replan (the replan graph runs the actor
+    for every row and keeps the plan of the flagged rows only); the host picks it from its own bookkeeping.  `step`
+    copies the observation into `static_obs`; a caller may instead write there and call `step()` with no argument.
+    The returned actions tensor is the policy's output buffer: it is overwritten by the next step.  The policy reads the
+    module's live parameters: an optimiser step, `load_state_dict` or a torch-side edit between steps is seen by the
+    next step, and a step whose parameters or bf16 shadows moved since the capture (an optimiser built or dropped
+    since) captures its graphs again."""
+
+    def __init__(self, module, n_envs, seed=0, env_ids=None, use_graphs=True):
+        for attr in ("actor", "action_decoder", "perceptual_encoder", "action_decoder_modalities"):
+            if not hasattr(module, attr):
+                raise ValueError(f"RolloutPolicy needs a TACO-RL module (no `{attr}`)")
+        dec = module.action_decoder
+        if not hasattr(dec, "_grip") or getattr(dec.rnn, "num_layers", None) != 2 or dec.rnn.bidirectional:
+            raise ValueError("RolloutPolicy covers the two-layer ActionDecoderLogistic")
+        if isinstance(n_envs, bool) or not isinstance(n_envs, (int, np.integer)) or not 1 <= int(n_envs) <= MAX_ENVS:
+            raise ValueError(f"n_envs must be an integer in 1..{MAX_ENVS} (got {n_envs!r}); build several policies for more")
+        if module.training:
+            raise ValueError("put the module in eval mode (module.eval()) before building a RolloutPolicy")
+        n = int(n_envs)
+        if env_ids is None:
+            env_ids = list(range(n))
+        env_ids = [int(e) for e in (env_ids.tolist() if torch.is_tensor(env_ids) else env_ids)]
+        if len(env_ids) != n or any(not 0 <= e < 2 ** 31 for e in env_ids):
+            raise ValueError(f"env_ids must be {n} integers in [0, 2^31)")
+        dev = next(module.parameters()).device
+        if dev.type != "cuda":
+            raise L.TacorlLibraryError("RolloutPolicy runs on a CUDA device (there is no CPU path)")
+        self.module, self.n, self.seed, self.device = module, n, int(seed), dev
+        self.use_graphs = bool(use_graphs)
+        actor = module.actor
+        self.P = dec.latent_plan_dim
+        self.H = dec.rnn.hidden_size
+        self.E = dec.rnn.input_size - self.P
+        self.dec_mods = list(module.action_decoder_modalities)
+        self.obs_mods = list(dict.fromkeys(self.dec_mods + list(actor.env_modalities)))
+        self.goal_mods = list(actor.goal_modalities)
+        if self.P % 4 or self.E % 4 or self.H % 8:
+            raise ValueError(f"decoder sizes plan {self.P} / embedding {self.E} / hidden {self.H} are not supported")
+        f32 = dict(device=dev, dtype=torch.float32)
+        self.plan = torch.zeros(n, self.P, **f32)
+        self.hidden = torch.zeros(2, n, self.H, **f32)
+        self.goal_emb = torch.zeros(n, actor.actor.goal_dim, **f32)
+        self.restart = torch.zeros(n, device=dev, dtype=torch.int32)
+        self.env_id = torch.tensor(env_ids, device=dev, dtype=torch.int32)
+        self.t = torch.zeros(n, device=dev, dtype=torch.int64)
+        self.actions = torch.zeros(n, 7, **f32)
+        self.logits = torch.zeros(n, 182, **f32)
+        self.ws = torch.zeros(int(L.query("tacorl_rollout_ws_bytes", n, self.H)), dtype=torch.uint8, device=dev)
+        self.static_obs = None
+        self._replan = np.zeros(n, dtype=np.int32)
+        self._has_goal = np.zeros(n, dtype=bool)
+        self._graphs = {}
+        self._pool = None
+        self.launches = {}            # (replan, precision) -> library launches recorded in that graph
+        self._tensors = [x for mod in (module.perceptual_encoder, actor, dec)
+                         for x in list(mod.parameters()) + list(mod.buffers())]
+        self.captures = 0
+
+    # ------------------------------------------------------------------------------------------------ validation
+    def _check_images(self, imgs, mods, rows, what):
+        if not isinstance(imgs, dict) or set(imgs) != set(mods):
+            got = sorted(imgs) if isinstance(imgs, dict) else type(imgs).__name__
+            raise ValueError(f"{what} must be a dict with the modalities {sorted(mods)} (got {got})")
+        for m in mods:
+            x = imgs[m]
+            if not torch.is_tensor(x) or x.dim() != 4 or x.shape[0] != rows or x.shape[1] != 3:
+                shape = tuple(x.shape) if torch.is_tensor(x) else type(x).__name__
+                raise ValueError(f"{what}[{m!r}] must be ({rows}, 3, H, W), got {shape}")
+            if x.dtype not in (torch.uint8, torch.float32):
+                raise ValueError(f"{what}[{m!r}] must be uint8 frames or normalised float32, got {x.dtype}")
+
+    # ------------------------------------------------------------------------------------------------ episode control
+    @torch.no_grad()
+    def _set_goal(self, rows, goal):
+        rows = _rows_list(rows, self.n)
+        self._check_images(goal, self.goal_mods, len(rows), "goal")
+        actor = self.module.actor
+        g = {m: goal[m].to(self.device) for m in self.goal_mods}
+        emb = actor.encoder.get_state_from_observation(observation=g, modalities=self.goal_mods).reshape(len(rows), -1)
+        if actor.goal_encoder is not None:
+            emb = actor.goal_encoder(emb)
+        self.goal_emb[rows] = emb.reshape(len(rows), -1)
+        self._has_goal[rows] = True
+        self._replan[rows] = 1
+        return rows
+
+    def reset(self, rows, goal):
+        """New episode for `rows`: goal images, step counter 0, replan (plan + zero hidden state) at the next step."""
+        rows = self._set_goal(rows, goal)
+        self.t[rows] = 0
+
+    def set_goal(self, rows, goal):
+        """Next subtask for `rows`: new goal, replan at the next step; the step counter keeps counting."""
+        self._set_goal(rows, goal)
+
+    def replan(self, rows):
+        """New plan and zero hidden state for `rows` at the next step."""
+        rows = _rows_list(rows, self.n)
+        self._replan[rows] = 1
+
+    # ------------------------------------------------------------------------------------------------ stepping
+    def _run(self, replan):
+        """The work of one step on the static buffers (what a graph captures)."""
+        m = self.module
+        with torch.no_grad():
+            emb = m.perceptual_encoder.get_state_from_observation(observation=self.static_obs,
+                                                                  modalities=self.dec_mods).reshape(self.n, -1)
+            if replan:
+                actor = m.actor
+                e = actor.encoder.get_state_from_observation(observation=self.static_obs,
+                                                             modalities=actor.env_modalities).reshape(self.n, -1)
+                new_plan = torch.tanh(actor.actor(e, self.goal_emb)[0])
+                self.plan.copy_(torch.where(self.restart.unsqueeze(1) != 0, new_plan, self.plan))
+            decoder_step(m.action_decoder, self.plan, emb.contiguous(), self.hidden, self.restart, self.seed,
+                         self.env_id, self.t, self.actions, self.logits, self.ws)
+
+    def _signature(self):
+        """What decides the device addresses a captured step reads.  A graph bakes them in: an optimiser built later
+        moves the parameters into its flat buffer, and a dropped optimiser takes its bf16 shadows with it, so a step
+        whose signature differs from its graph's captures again.  The parameters' and buffers' addresses, the live
+        optimisers' shadow buffers (a parameter's shadow is its owner's buffer at the parameter's offset) and the cached
+        shadows of frozen parameters determine every address `ops.shadow_of` can hand the kernels."""
+        return (ops.get_precision(), tuple(x.data_ptr() for x in self._tensors),
+                frozenset((id(o), o.shadow.data_ptr()) for o in ops._SHADOW_OWNERS),
+                frozenset(id(v[2]) for v in ops._FROZEN_SHADOWS.values()))
+
+    def _operands(self):
+        """The tensors a graph reads: every parameter and buffer of the encoders, the actor and the decoder, and the
+        bf16 shadow of each parameter.  A graph keeps them alive for as long as it exists."""
+        keep = []
+        for x in self._tensors:
+            keep.append(x.detach())
+            if isinstance(x, torch.nn.Parameter):
+                keep.append(ops.shadow_of(x))
+        return keep
+
+    def _capture(self, replan):
+        # warm-up on a side stream against copies of the state the step mutates, then restore it
+        saved = [x.clone() for x in (self.plan, self.hidden, self.t)]
+        side = torch.cuda.Stream(device=self.device)
+        side.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(side):
+            self._run(replan)
+        torch.cuda.current_stream(self.device).wait_stream(side)
+        torch.cuda.synchronize(self.device)
+        graph = torch.cuda.CUDAGraph()
+        if self._pool is None:
+            self._pool = torch.cuda.graph_pool_handle()
+        n0 = L.launch_count()
+        with torch.cuda.graph(graph, pool=self._pool):
+            self._run(replan)
+        launches = L.launch_count() - n0
+        with torch.no_grad():
+            for x, s in zip((self.plan, self.hidden, self.t), saved):
+                x.copy_(s)
+        torch.cuda.synchronize(self.device)
+        return graph, launches
+
+    def step(self, obs=None):
+        """One control step of every environment.  obs: {modality: (n_envs, 3, H, W)} uint8 frames or normalised
+        float32, the same shapes and dtype at every step (None: `static_obs` already holds the observation)."""
+        if not self._has_goal.all():
+            missing = np.flatnonzero(~self._has_goal).tolist()
+            raise ValueError(f"environments {missing} have no goal yet: reset(rows, goal) them before the first step")
+        if obs is not None:
+            self._check_images(obs, self.obs_mods, self.n, "obs")
+            if self.static_obs is None:
+                self.static_obs = {k: torch.empty(obs[k].shape, dtype=obs[k].dtype, device=self.device) for k in self.obs_mods}
+            for k in self.obs_mods:
+                s = self.static_obs[k]
+                if obs[k].shape != s.shape or obs[k].dtype != s.dtype:
+                    raise ValueError(f"obs[{k!r}] is {tuple(obs[k].shape)} {obs[k].dtype}; this policy's static buffer "
+                                     f"is {tuple(s.shape)} {s.dtype}")
+                s.copy_(obs[k], non_blocking=True)
+        elif self.static_obs is None:
+            raise ValueError("no observation: pass obs to the first step")
+        replan = bool(self._replan.any())
+        self.restart.copy_(torch.from_numpy(self._replan))
+        ops.refresh_shadows()          # parameters edited through torch since the last step (checkpoint load, ...)
+        if self.use_graphs:
+            key = (replan, ops.get_precision())
+            sig = self._signature()
+            entry = self._graphs.get(key)
+            if entry is not None and entry[2] != sig:
+                self._graphs.clear()      # every graph reads the same operands: none of them is valid any more
+                entry = None
+            if entry is None:
+                keep = self._operands()          # (creates any frozen shadow before the capture reads it)
+                sig = self._signature()
+                graph, launches = self._capture(replan)
+                # the graph holds raw pointers: keep what it reads alive for as long as the graph exists
+                entry = self._graphs[key] = (graph, launches, sig, keep)
+                self.captures += 1
+            graph, self.launches[key] = entry[:2]
+            graph.replay()
+        else:
+            self._run(replan)
+        self._replan[:] = 0
+        return self.actions
