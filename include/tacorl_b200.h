@@ -423,6 +423,18 @@ int tacorl_rollout_decoder_step(int n, int P, int E, int H, const float* plan, c
                                 const int* restart, const float* const* w, const void* const* w_bf16,
                                 unsigned long long seed, const int* env_id, long long* t, float grip_lo, float grip_hi,
                                 float* actions, float* logits, void* ws, size_t ws_bytes, int prec, void* stream);
+/* ---- the rollout policy's own sampling (sampled latent plans, the flat-CQL actor), one graph-capturable launch for n
+ * rows, 1 <= n <= 64; fp32 arithmetic in both precision modes.  mean, std (n, A): ops.gauss_head's output; grip_logits:
+ * NULL or (n, 2); mask: NULL or (n) int32, rows whose mask is 0 are not written.  Draw j of row r is the Philox4x32-10
+ * block with key (lo32(seed), hi32(seed)) and counter (lo32(t[r]), hi32(t[r]), env_id[r], j); its words 0 and 1 give
+ * u_a = (w0 >> 8) 2^-24 and u_b = (w1 >> 8) 2^-24.  Dimension d < A uses draw 32 + d:
+ * out[r][d] = tanh(mean + std sqrt(-2 ln(1 - u_a)) cos(2 pi u_b)).  The gripper uses draw 32 + A:
+ * out[r][A] = 2 argmax_c(normalised logit_c - log(-log(u_c))) - 1 with u_0 = u_a, u_1 = u_b (ties -> class 0).
+ * (Draws 0..16 are tacorl_rollout_decoder_step's.)  advance_t = 1: every row's t is incremented after sampling.
+ * out has row stride ldo floats.  Each row is computed on its own: bit-identical alone or among 64 rows. */
+int tacorl_rollout_policy_sample(int n, int A, const float* mean, const float* std, const float* grip_logits,
+                                 const int* mask, unsigned long long seed, const int* env_id, long long* t, int advance_t,
+                                 float* out, long long ldo, void* stream);
 int tacorl_polyak_update(long long n, float* target, const float* source, float tau, void* stream);
 int tacorl_sqnorm(long long n, const float* x, float* out, float* ws, void* stream);
 

@@ -86,6 +86,7 @@ _SIGS = {
     "tacorl_rollout_ws_bytes": [_i, _i],
     "tacorl_rollout_decoder_step": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp, _f, _f,
                                     _vp, _vp, _vp, _sz, _i, _vp],
+    "tacorl_rollout_policy_sample": [_i, _i, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp, _i, _vp, _ll, _vp],
     "tacorl_metrics_accumulate": [_vp, _vp, _vp],
     "tacorl_metrics_record": [_vp, _vp, _i, _vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],

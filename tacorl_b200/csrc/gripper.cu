@@ -6,17 +6,10 @@
 // Noise (the uniforms) is an input, like every other random quantity of this library.
 #include "common.cuh"
 #include "internal.h"
+#include "gripper.cuh"
 #include "../../include/tacorl_b200.h"
 
 namespace tacorl {
-
-// torch: Categorical-family `logits` are stored normalised, logits - logsumexp(logits) (max-shifted)
-__device__ __forceinline__ void gr_normalise(float l0, float l1, float& n0, float& n1) {
-  const float m = fmaxf(l0, l1);
-  const float lse = m + logf(expf(l0 - m) + expf(l1 - m));
-  n0 = l0 - lse;
-  n1 = l1 - lse;
-}
 
 // index[r] = argmax_c(norm_logits[r % rows0][c] - log(-log(u[r][c]))); ties -> class 0 (torch.argmax: first maximum).
 // clamp_u: u clamped to [eps, 1 - eps] first (torch.distributions.utils.clamp_probs, the rsample path).

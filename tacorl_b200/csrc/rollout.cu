@@ -10,10 +10,13 @@
 // one column; lane l accumulates k = chunk + 128 h + 4 l + q (h < 2, q < 4) in that order, chunk after chunk, and the
 // 32 lane partials are summed by a fixed shuffle-down tree.  Nothing in that order depends on the number of rows or on
 // any other row, so a row's result is bit-identical alone or in a batch of 64.
+// tacorl_rollout_policy_sample draws the policy's own samples (a sampled latent plan, the flat-CQL actor's TanhNormal
+// arm and GumbelSoftmax gripper) from the same counter-based stream, in one launch.
 #include "common.cuh"
 #include "internal.h"
 #include "philox.cuh"
 #include "dlm_sample.cuh"
+#include "gripper.cuh"
 #include "../../include/tacorl_b200.h"
 #include <cuda_bf16.h>
 
@@ -190,6 +193,43 @@ static int launch_gemv(const GemvArgs& a, int prec, cudaStream_t st) {
   return bf ? launch_gemv_nr<kMaxRows, true>(a, st) : launch_gemv_nr<kMaxRows, false>(a, st);
 }
 
+// The policy's own draws (sampled plans, the flat-CQL actor) start at draw 32: the decoder step above uses draws 0..16
+// of the same counter, so both can sample in one step with the same t and still read disjoint noise.
+constexpr int kPolicyDraw0 = 32;
+
+// Row r, continuous dimension d < A: words 0 / 1 of draw 32 + d are u_a / u_b, z = sqrt(-2 ln(1 - u_a)) cos(2 pi u_b)
+// and out = tanh(mean + std z) (TanhNormal.sample()).  Gripper (logits given): words 0 / 1 of draw 32 + A are u_0 / u_1
+// and out[A] = 2 argmax_c(normalised logit_c - log(-log(u_c))) - 1 (GumbelSoftmax.sample(), as gripper_gumbel_kernel
+// computes it unclamped: u = 0 scores -inf, ties go to class 0).  One CTA, so that the step counters are advanced
+// after every element has read them; each element is computed on its own, so a row's output does not depend on n.
+__global__ void __launch_bounds__(256) rollout_policy_sample_kernel(
+    int n, int A, const float* __restrict__ mean, const float* __restrict__ stdv, const float* __restrict__ grip,
+    const int* __restrict__ mask, unsigned k0, unsigned k1, const int* __restrict__ env_id, long long* t, int advance_t,
+    float* __restrict__ out, long long ldo) {
+  const int per_row = A + (grip ? 1 : 0);
+  for (int i = threadIdx.x; i < n * per_row; i += blockDim.x) {
+    const int r = i / per_row, d = i % per_row;
+    if (mask && mask[r] == 0) continue;
+    const unsigned long long tt = (unsigned long long)t[r];
+    const U4 w = philox4x32_10(U4{(unsigned)tt, (unsigned)(tt >> 32), (unsigned)env_id[r], (unsigned)(kPolicyDraw0 + d)},
+                               k0, k1);
+    const float ua = __fmul_rn((float)(w.x >> 8), 5.9604644775390625e-08f);
+    const float ub = __fmul_rn((float)(w.y >> 8), 5.9604644775390625e-08f);
+    if (d < A) {
+      const float z = sqrtf(-2.f * logf(1.f - ua)) * cosf(6.28318530717958647692f * ub);
+      out[r * ldo + d] = tanhf(fmaf(stdv[r * A + d], z, mean[r * A + d]));
+    } else {
+      float n0, n1;
+      gr_normalise(grip[2 * r], grip[2 * r + 1], n0, n1);
+      const float s0 = n0 - logf(-logf(ua)), s1 = n1 - logf(-logf(ub));
+      out[r * ldo + A] = s1 > s0 ? 1.f : -1.f;
+    }
+  }
+  if (!advance_t) return;
+  __syncthreads();
+  for (int r = threadIdx.x; r < n; r += blockDim.x) t[r] += 1;
+}
+
 static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 static bool aligned8(const void* p) { return ((uintptr_t)p & 7) == 0; }
 
@@ -266,6 +306,20 @@ int tacorl_rollout_decoder_step(int n, int P, int E, int H, const float* plan, c
   a.k0 = (unsigned)seed; a.k1 = (unsigned)(seed >> 32);
   a.grip_lo = grip_lo; a.grip_hi = grip_hi;
   return launch_gemv(a, prec, st);
+}
+
+int tacorl_rollout_policy_sample(int n, int A, const float* mean, const float* std, const float* grip_logits,
+                                 const int* mask, unsigned long long seed, const int* env_id, long long* t, int advance_t,
+                                 float* out, long long ldo, void* stream) {
+  TACORL_REQUIRE(n >= 1 && n <= kMaxRows, "rollout_policy_sample: n = %d rows (1..%d)", n, kMaxRows);
+  TACORL_REQUIRE(A >= 1, "rollout_policy_sample: A = %d continuous dimensions", A);
+  TACORL_REQUIRE(ldo >= A + (grip_logits ? 1 : 0), "rollout_policy_sample: output row stride %lld < %d", ldo,
+                 A + (grip_logits ? 1 : 0));
+  TACORL_REQUIRE(mean && std && env_id && t && out, "rollout_policy_sample: null pointer");
+  rollout_policy_sample_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(n, A, mean, std, grip_logits, mask, (unsigned)seed,
+                                                                    (unsigned)(seed >> 32), env_id, t, advance_t, out, ldo);
+  TACORL_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // extern "C"

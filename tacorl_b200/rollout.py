@@ -1,4 +1,5 @@
-"""Batched rollout policy of a trained TACO-RL agent: many environments, one CUDA-graph replay per control step.
+"""Batched rollout policy of a trained TACO-RL, PlayLMP or flat-CQL agent: many environments, one CUDA-graph replay
+per control step.
 
 The reference's policy entry is single-environment and stateful (rollout_manager.py:364-386): a deterministic latent
 plan from the visual actor, `clear_hidden_state()`, then one `act()` per control step, with ONE hidden state and one
@@ -8,13 +9,13 @@ sampling noise from its own counter (Philox4x32-10 keyed by the seed, counter = 
 environment's noise depends only on the seed, its env_id and its own step count, never on which other environments
 share the batch, and the decoder step is batch-invariant.  DESIGN.md section 16 states the rules.
 
-    policy = RolloutPolicy(tacorl_module, n_envs, seed=0)
+    policy = RolloutPolicy(module, n_envs, seed=0)
     policy.reset(rows, goal)        # goal images of these environments; their step counters restart at 0
     actions = policy.step(obs)      # {modality: (n_envs, 3, H, W)} uint8 or normalised fp32 -> (n_envs, 7)
 
-The decoder step is `tacorl_rollout_decoder_step` (csrc/rollout.cu); the encoders and the actor run through the same
-library kernels as training.  Nothing here changes the module: `act()`, `clear_hidden_state()` and training are
-untouched."""
+The decoder step is `tacorl_rollout_decoder_step` and sampled plans and flat-CQL actions are drawn by
+`tacorl_rollout_policy_sample` (csrc/rollout.cu); the encoders and the actor run through the same library kernels as
+training.  Nothing here changes the module: `act()`, `clear_hidden_state()` and training are untouched."""
 import ctypes
 
 import numpy as np
@@ -75,34 +76,89 @@ def decoder_step(decoder, plan, emb, hidden, restart, seed, env_id, t, actions, 
     return actions
 
 
+def policy_sample(mean, std, logits, mask, seed, env_id, t, out, advance_t=False):
+    """Sample n = mean.shape[0] rows of a TanhNormal(mean, std) (n, A) arm, plus a GumbelSoftmax gripper when logits
+    (n, 2) are given, from each row's counter-based noise (Philox draws 32 + d, DESIGN.md section 16), into out (n, >= A
+    [+ 1]): tanh(mean + std z) and the gripper as 2 class - 1.  mask: None or (n,) int32, rows whose mask is 0 are not
+    written.  advance_t: t (n, int64) is incremented after sampling.  fp32 in both precision modes."""
+    n, A = mean.shape
+    if std.shape != mean.shape or (logits is not None and logits.shape != (n, 2)):
+        raise ValueError(f"policy_sample: mean {tuple(mean.shape)}, std {tuple(std.shape)}, logits "
+                         f"{None if logits is None else tuple(logits.shape)}")
+    if out.dim() != 2 or out.shape[0] != n or out.stride(1) != 1:
+        raise ValueError(f"policy_sample: out must be ({n}, >= {A}) with unit column stride")
+    if env_id.dtype != torch.int32 or t.dtype != torch.int64 or (mask is not None and mask.dtype != torch.int32):
+        raise ValueError("policy_sample: env_id and mask are int32, t is int64")
+    L.call("tacorl_rollout_policy_sample", n, A, L.ptr(mean.contiguous()), L.ptr(std.contiguous()),
+           L.ptr(None if logits is None else logits.contiguous()), L.ptr_any(mask),
+           ctypes.c_ulonglong(int(seed) & 0xFFFFFFFFFFFFFFFF), L.ptr_any(env_id), L.ptr_any(t), int(bool(advance_t)),
+           L.ptr(out), out.stride(0), L.stream())
+    return out
+
+
+def _module_kind(module):
+    """"play_lmp", "cql" (flat CQL: a CQL_Offline without an action decoder) or "tacorl" (everything else, checked as
+    a TACO-RL module)."""
+    from .modules.cql.cql_offline_lightning import CQL_Offline
+    from .modules.play_lmp.play_lmp_for_rl import PlayLMP
+    if isinstance(module, PlayLMP):
+        return "play_lmp"
+    if isinstance(module, CQL_Offline) and not hasattr(module, "action_decoder"):
+        return "cql"
+    return "tacorl"
+
+
+def _check_decoder(dec):
+    if not hasattr(dec, "_grip") or getattr(dec.rnn, "num_layers", None) != 2 or dec.rnn.bidirectional:
+        raise ValueError("RolloutPolicy covers the two-layer ActionDecoderLogistic")
+
+
+def _cat(ts):
+    return ts[0] if len(ts) == 1 else torch.cat(ts, dim=-1)
+
+
 class RolloutPolicy:
-    """Batched deterministic-plan rollout of a TACO-RL module (eval mode, on its CUDA device) for 1..64 environments.
+    """Batched rollout of a TACO-RL, PlayLMP or flat-CQL module (eval mode, on its CUDA device) for 1..64 environments.
 
     reset(rows, goal)    new episode: goal images for these rows, step counter 0, replan at their next step
     set_goal(rows, goal) next subtask: new goal, replan at the next step, step counter kept
-    replan(rows)         new plan and zero hidden state at the next step (every plan_duration steps)
+    replan(rows)         new plan and zero hidden state at the next step (every plan_duration steps; not flat CQL)
     step(obs)            one control step of every environment -> (n_envs, 7) actions
 
-    A replanning row takes the plan of the reference's deterministic actor call, tanh(mean) of the actor on its encoder
-    embedding of the current observation and the goal embedding goal_encoder(encoder(goal)) (computed once, at
-    reset / set_goal); its hidden state restarts at zero and its first decoder step uses the same frame.  The decoder
-    consumes perceptual_encoder.get_state_from_observation(obs, action_decoder_modalities), as `act()` does.
+    TACO-RL and PlayLMP: a replanning row takes a plan from the high-level policy (TACO-RL's actor, PlayLMP's
+    plan_proposal) on its encoder embedding of the current observation and the goal embedding
+    goal_encoder(encoder(goal)) (computed once, at reset / set_goal): tanh(mean) with deterministic=True (the
+    reference's deterministic actor call), a TanhNormal sample drawn from the row's own noise otherwise (PlayLMP's
+    `pp_dist.sample()`).  Its hidden state restarts at zero and its first decoder step uses the same frame.  The decoder
+    consumes perceptual_encoder.get_state_from_observation(obs, action_decoder_modalities), as `act()` does; PlayLMP's
+    plan proposal reads the same encoder, so each modality is encoded once per step.
+    Flat CQL: every step is the actor on cat(encoder(obs), goal embedding): Actor.get_actions(deterministic=True)
+    (tanh(mean), argmax gripper), or with deterministic=False a TanhNormal arm and GumbelSoftmax gripper sample.
 
     Each step is one CUDA-graph replay of one of two graphs, with and without a replan (the replan graph runs the actor
-    for every row and keeps the plan of the flagged rows only); the host picks it from its own bookkeeping.  `step`
+    for every row and keeps the plan of the flagged rows only; flat CQL has one graph); the host picks it from its own
+    bookkeeping.  `step`
     copies the observation into `static_obs`; a caller may instead write there and call `step()` with no argument.
     The returned actions tensor is the policy's output buffer: it is overwritten by the next step.  The policy reads the
     module's live parameters: an optimiser step, `load_state_dict` or a torch-side edit between steps is seen by the
     next step, and a step whose parameters or bf16 shadows moved since the capture (an optimiser built or dropped
     since) captures its graphs again."""
 
-    def __init__(self, module, n_envs, seed=0, env_ids=None, use_graphs=True):
-        for attr in ("actor", "action_decoder", "perceptual_encoder", "action_decoder_modalities"):
-            if not hasattr(module, attr):
-                raise ValueError(f"RolloutPolicy needs a TACO-RL module (no `{attr}`)")
-        dec = module.action_decoder
-        if not hasattr(dec, "_grip") or getattr(dec.rnn, "num_layers", None) != 2 or dec.rnn.bidirectional:
-            raise ValueError("RolloutPolicy covers the two-layer ActionDecoderLogistic")
+    def __init__(self, module, n_envs, seed=0, env_ids=None, use_graphs=True, deterministic=True):
+        kind = _module_kind(module)
+        if kind == "tacorl":
+            for attr in ("actor", "action_decoder", "perceptual_encoder", "action_decoder_modalities"):
+                if not hasattr(module, attr):
+                    raise ValueError(f"RolloutPolicy needs a TACO-RL, PlayLMP or flat-CQL module (no `{attr}`)")
+            _check_decoder(module.action_decoder)
+        elif kind == "play_lmp":
+            _check_decoder(module.action_decoder)
+            if not hasattr(module.plan_proposal, "policy") or module.plan_proposal.discrete_gripper:
+                raise ValueError("RolloutPolicy covers a PlayLMP whose plan proposal is a continuous Actor")
+        elif not module.actor.discrete_gripper:
+            raise ValueError("RolloutPolicy covers flat CQL with a discrete (GumbelSoftmax) gripper")
+        if not isinstance(deterministic, bool):
+            raise ValueError(f"deterministic must be a bool (got {deterministic!r})")
         if isinstance(n_envs, bool) or not isinstance(n_envs, (int, np.integer)) or not 1 <= int(n_envs) <= MAX_ENVS:
             raise ValueError(f"n_envs must be an integer in 1..{MAX_ENVS} (got {n_envs!r}); build several policies for more")
         if module.training:
@@ -117,34 +173,50 @@ class RolloutPolicy:
         if dev.type != "cuda":
             raise L.TacorlLibraryError("RolloutPolicy runs on a CUDA device (there is no CPU path)")
         self.module, self.n, self.seed, self.device = module, n, int(seed), dev
+        self.kind, self.deterministic = kind, deterministic
         self.use_graphs = bool(use_graphs)
-        actor = module.actor
-        self.P = dec.latent_plan_dim
-        self.H = dec.rnn.hidden_size
-        self.E = dec.rnn.input_size - self.P
-        self.dec_mods = list(module.action_decoder_modalities)
-        self.obs_mods = list(dict.fromkeys(self.dec_mods + list(actor.env_modalities)))
-        self.goal_mods = list(actor.goal_modalities)
-        if self.P % 4 or self.E % 4 or self.H % 8:
-            raise ValueError(f"decoder sizes plan {self.P} / embedding {self.E} / hidden {self.H} are not supported")
+        # what the step reads: the encoder of the actor's (plan proposal's) input, its goal encoder and policy, and the
+        # decoder with its encoder (None for flat CQL)
+        if kind == "play_lmp":
+            self._enc, self._goal_enc, self._net = module.perceptual_encoder, module.goal_encoder, module.plan_proposal
+            self.env_mods = list(module.plan_proposal_obs_modalities)
+            self.goal_mods = list(module.plan_proposal_goal_modalities)
+            nets = (module.perceptual_encoder, module.goal_encoder, module.plan_proposal, module.action_decoder)
+        else:
+            actor = module.actor
+            self._enc, self._goal_enc, self._net = actor.encoder, actor.goal_encoder, actor.actor
+            self.env_mods, self.goal_mods = list(actor.env_modalities), list(actor.goal_modalities)
+            nets = ((module.perceptual_encoder, actor, module.action_decoder) if kind == "tacorl"
+                    else tuple(m for m in (actor.encoder, actor.goal_encoder, actor.actor) if m is not None))
+        self._dec = None if kind == "cql" else module.action_decoder
+        self.dec_mods = [] if kind == "cql" else list(module.action_decoder_modalities)
+        self.obs_mods = list(dict.fromkeys(self.dec_mods + self.env_mods))
         f32 = dict(device=dev, dtype=torch.float32)
-        self.plan = torch.zeros(n, self.P, **f32)
-        self.hidden = torch.zeros(2, n, self.H, **f32)
-        self.goal_emb = torch.zeros(n, actor.actor.goal_dim, **f32)
+        if self._dec is not None:
+            dec = self._dec
+            self.P = dec.latent_plan_dim
+            self.H = dec.rnn.hidden_size
+            self.E = dec.rnn.input_size - self.P
+            if self.P % 4 or self.E % 4 or self.H % 8:
+                raise ValueError(f"decoder sizes plan {self.P} / embedding {self.E} / hidden {self.H} are not supported")
+            self.plan = torch.zeros(n, self.P, **f32)
+            self.hidden = torch.zeros(2, n, self.H, **f32)
+            self.logits = torch.zeros(n, 182, **f32)
+            self.ws = torch.zeros(int(L.query("tacorl_rollout_ws_bytes", n, self.H)), dtype=torch.uint8, device=dev)
+        else:
+            self.plan = self.hidden = None
+        self.goal_emb = torch.zeros(n, self._net.goal_dim, **f32)
         self.restart = torch.zeros(n, device=dev, dtype=torch.int32)
         self.env_id = torch.tensor(env_ids, device=dev, dtype=torch.int32)
         self.t = torch.zeros(n, device=dev, dtype=torch.int64)
         self.actions = torch.zeros(n, 7, **f32)
-        self.logits = torch.zeros(n, 182, **f32)
-        self.ws = torch.zeros(int(L.query("tacorl_rollout_ws_bytes", n, self.H)), dtype=torch.uint8, device=dev)
         self.static_obs = None
         self._replan = np.zeros(n, dtype=np.int32)
         self._has_goal = np.zeros(n, dtype=bool)
         self._graphs = {}
         self._pool = None
         self.launches = {}            # (replan, precision) -> library launches recorded in that graph
-        self._tensors = [x for mod in (module.perceptual_encoder, actor, dec)
-                         for x in list(mod.parameters()) + list(mod.buffers())]
+        self._tensors = [x for mod in nets for x in list(mod.parameters()) + list(mod.buffers())]
         self.captures = 0
 
     # ------------------------------------------------------------------------------------------------ validation
@@ -165,14 +237,14 @@ class RolloutPolicy:
     def _set_goal(self, rows, goal):
         rows = _rows_list(rows, self.n)
         self._check_images(goal, self.goal_mods, len(rows), "goal")
-        actor = self.module.actor
         g = {m: goal[m].to(self.device) for m in self.goal_mods}
-        emb = actor.encoder.get_state_from_observation(observation=g, modalities=self.goal_mods).reshape(len(rows), -1)
-        if actor.goal_encoder is not None:
-            emb = actor.goal_encoder(emb)
+        emb = self._enc.get_state_from_observation(observation=g, modalities=self.goal_mods).reshape(len(rows), -1)
+        if self._goal_enc is not None:
+            emb = self._goal_enc(emb)
         self.goal_emb[rows] = emb.reshape(len(rows), -1)
         self._has_goal[rows] = True
-        self._replan[rows] = 1
+        if self._dec is not None:
+            self._replan[rows] = 1
         return rows
 
     def reset(self, rows, goal):
@@ -186,24 +258,51 @@ class RolloutPolicy:
 
     def replan(self, rows):
         """New plan and zero hidden state for `rows` at the next step."""
+        if self._dec is None:
+            raise ValueError("flat CQL has no plan: every step already runs the actor")
         rows = _rows_list(rows, self.n)
         self._replan[rows] = 1
 
     # ------------------------------------------------------------------------------------------------ stepping
+    def _embed(self, enc, mods):
+        return enc.get_state_from_observation(observation=self.static_obs, modalities=mods).reshape(self.n, -1)
+
     def _run(self, replan):
         """The work of one step on the static buffers (what a graph captures)."""
-        m = self.module
         with torch.no_grad():
-            emb = m.perceptual_encoder.get_state_from_observation(observation=self.static_obs,
-                                                                  modalities=self.dec_mods).reshape(self.n, -1)
+            if self._dec is None:
+                self._act(self._embed(self._enc, self.env_mods))
+                return
+            if self.kind == "play_lmp":       # plan proposal and decoder read the same encoder: each view once
+                per = self._enc.get_state_from_observation(observation=self.static_obs, modalities=self.obs_mods,
+                                                           cat_output=False)
+                per = {k: v.reshape(self.n, -1) for k, v in per.items()}
+                emb = _cat([per[k] for k in self.dec_mods])
+                e = _cat([per[k] for k in self.env_mods]) if replan else None
+            else:
+                emb = self._embed(self.module.perceptual_encoder, self.dec_mods)
+                e = self._embed(self._enc, self.env_mods) if replan else None
             if replan:
-                actor = m.actor
-                e = actor.encoder.get_state_from_observation(observation=self.static_obs,
-                                                             modalities=actor.env_modalities).reshape(self.n, -1)
-                new_plan = torch.tanh(actor.actor(e, self.goal_emb)[0])
-                self.plan.copy_(torch.where(self.restart.unsqueeze(1) != 0, new_plan, self.plan))
-            decoder_step(m.action_decoder, self.plan, emb.contiguous(), self.hidden, self.restart, self.seed,
+                out = self._net(e, self.goal_emb)
+                if self.deterministic:
+                    new_plan = torch.tanh(out[0])
+                    self.plan.copy_(torch.where(self.restart.unsqueeze(1) != 0, new_plan, self.plan))
+                else:         # the flagged rows' plans, drawn at the t their first decoder step reads
+                    policy_sample(out[0], out[1], None, self.restart, self.seed, self.env_id, self.t, self.plan)
+            decoder_step(self._dec, self.plan, emb.contiguous(), self.hidden, self.restart, self.seed,
                          self.env_id, self.t, self.actions, self.logits, self.ws)
+
+    def _act(self, e):
+        """Flat CQL: the actor on cat(e, goal embedding) -> actions, then t += 1."""
+        mean, std, logits = self._net(e, self.goal_emb)
+        if self.deterministic:            # Actor.get_actions(deterministic=True)
+            A = mean.shape[1]
+            self.actions[:, :A].copy_(torch.tanh(mean))
+            grip = torch.argmax(torch.softmax(logits, dim=-1), dim=-1).to(torch.float32) * 2.0 - 1
+            self.actions[:, A].copy_(grip)
+            self.t.add_(1)
+        else:
+            policy_sample(mean, std, logits, None, self.seed, self.env_id, self.t, self.actions, advance_t=True)
 
     def _signature(self):
         """What decides the device addresses a captured step reads.  A graph bakes them in: an optimiser built later
@@ -216,8 +315,8 @@ class RolloutPolicy:
                 frozenset(id(v[2]) for v in ops._FROZEN_SHADOWS.values()))
 
     def _operands(self):
-        """The tensors a graph reads: every parameter and buffer of the encoders, the actor and the decoder, and the
-        bf16 shadow of each parameter.  A graph keeps them alive for as long as it exists."""
+        """The tensors a graph reads: every parameter and buffer of the encoders, the actor (plan proposal) and the
+        decoder, and the bf16 shadow of each parameter.  A graph keeps them alive for as long as it exists."""
         keep = []
         for x in self._tensors:
             keep.append(x.detach())
@@ -227,7 +326,8 @@ class RolloutPolicy:
 
     def _capture(self, replan):
         # warm-up on a side stream against copies of the state the step mutates, then restore it
-        saved = [x.clone() for x in (self.plan, self.hidden, self.t)]
+        state = [x for x in (self.plan, self.hidden, self.t) if x is not None]
+        saved = [x.clone() for x in state]
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
@@ -242,7 +342,7 @@ class RolloutPolicy:
             self._run(replan)
         launches = L.launch_count() - n0
         with torch.no_grad():
-            for x, s in zip((self.plan, self.hidden, self.t), saved):
+            for x, s in zip(state, saved):
                 x.copy_(s)
         torch.cuda.synchronize(self.device)
         return graph, launches
