@@ -7,7 +7,7 @@
 //                   fenced into the async proxy and handed to the MMA warp through an mbarrier ring
 //   B operand     = the layer's packed bf16 weights, TMA-loaded ONCE per CTA and kept resident in shared memory
 //   accumulator   = TMEM, double-buffered so the epilogue of tile i overlaps the MMAs of tile i+1
-//   epilogue      = tcgen05.ld -> bias + ReLU (forward) or ReLU gate of the saved activation (dgrad) -> NHWC bf16/fp32
+//   epilogue      = TMEM load -> bias + ReLU (forward) or ReLU gate of the saved activation (dgrad) -> NHWC bf16/fp32
 //
 // The same kernel runs conv1 (as a 2x2/stride-1 conv over a space-to-depth(4) copy of the image), conv2, conv3 forward,
 // conv3 dgrad and the four stride-parity classes of conv2 dgrad.  conv_tc_wgrad_kernel computes the weight gradients
@@ -15,7 +15,7 @@
 // Reference semantics: nn.Conv2d x3 + ReLU of /root/reference/src/tacorl/networks/visual_encoders/encoder.py:369-390.
 #include "common.cuh"
 #include "internal.h"
-#include <cuda.h>
+#include "sm100.cuh"
 #include <cuda_bf16.h>
 #include <algorithm>
 
@@ -43,43 +43,7 @@ struct ConvEpi {
   float* out_f32;                   // (N, OH, OW, BN) or null
 };
 
-// ---- PTX helpers (same conventions as gemm_tc.cu)
-__device__ __forceinline__ uint32_t cv_smem(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void cv_mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void cv_mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void cv_mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void cv_tma_2d(uint32_t dst, const CUtensorMap* tm, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-      ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_tma_4d(uint32_t dst, const CUtensorMap* tm, int c0, int c1, int c2, int c3, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-      ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_tma_5d(uint32_t dst, const CUtensorMap* tm, int c0, int c1, int c2, int c3, int c4,
-                                          uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
-      ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(bar) : "memory");
-}
+// ---- cp.async gathers and wide stores (the TMA / tcgen05 primitives are in sm100.cuh)
 __device__ __forceinline__ void cv_cp16(uint32_t dst, const void* src, uint32_t src_bytes) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
 }
@@ -106,43 +70,6 @@ __device__ __forceinline__ void cv_wait_group_dyn(int n) {   // n in [0, 4]
   }
 }
 __device__ __forceinline__ void cv_fence_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void cv_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void cv_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void cv_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void cv_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void cv_ld16_nowait(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void cv_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint64_t cv_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
 
 // ------------------------------------------------------------------------------------------ forward / dgrad
 // One tile = a BW x BH patch of output pixels of one frame (row r = a_l*BW + b_l, BW*BH <= 128).  For filter tap t
@@ -160,15 +87,15 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
   constexpr uint32_t TMEM_COLS = 2 * ACC_COLS;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  const uint32_t w_base = cv_smem(smem);
+  const uint32_t w_base = smem_u32(smem);
   const uint32_t a_base = w_base + g.ntaps * W_TAP_BYTES;            // multiple of 1024 (BN*128 with BN >= 32: 4096)
   uint64_t* bars = (uint64_t*)(smem + g.ntaps * W_TAP_BYTES + CV_STAGES * A_BYTES);
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * CV_STAGES + 5);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + CV_STAGES + s); };
-  auto tfull_bar = [&](int a) { return cv_smem(bars + 2 * CV_STAGES + a); };
-  auto tempty_bar = [&](int a) { return cv_smem(bars + 2 * CV_STAGES + 2 + a); };
-  const uint32_t w_bar = cv_smem(bars + 2 * CV_STAGES + 4);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + CV_STAGES + s); };
+  auto tfull_bar = [&](int a) { return smem_u32(bars + 2 * CV_STAGES + a); };
+  auto tempty_bar = [&](int a) { return smem_u32(bars + 2 * CV_STAGES + 2 + a); };
+  const uint32_t w_bar = smem_u32(bars + 2 * CV_STAGES + 4);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tiles_per_frame = g.tiles_x * g.tiles_y;
@@ -176,26 +103,22 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
   if (threadIdx.x < BN) s_bias[threadIdx.x] = ep.bias ? ep.bias[threadIdx.x] : 0.f;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < CV_STAGES; ++s) { cv_mbar_init(full_bar(s), 1); cv_mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < 2; ++a) { cv_mbar_init(tfull_bar(a), 1); cv_mbar_init(tempty_bar(a), 4); }
-    cv_mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < CV_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
+    mbar_init(w_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  cv_fence_before();
+  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
       // ===== TMA producer: resident weights (one box per tap), then one activation box per (tile, tap)
-      cv_mbar_expect_tx(w_bar, g.ntaps * W_TAP_BYTES);
-      for (int t = 0; t < g.ntaps; ++t) cv_tma_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * BN, w_bar);
+      mbar_expect_tx(w_bar, g.ntaps * W_TAP_BYTES);
+      for (int t = 0; t < g.ntaps; ++t) tma_load_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * BN, w_bar);
       const uint32_t box_bytes = (uint32_t)(g.BW * g.BH) * 128;
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x) {
@@ -204,39 +127,39 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
         const int x0 = tx * g.BW, y0 = ty * g.BH;
         for (int t = 0; t < g.ntaps; ++t, ++it) {
           const int s = it % CV_STAGES;
-          cv_mbar_wait(empty_bar(s), ((it / CV_STAGES) & 1) ^ 1);
-          cv_mbar_expect_tx(full_bar(s), box_bytes);
-          cv_tma_5d(a_base + s * A_BYTES, &tmA, 0, x0 + g.tap_x[t], g.tap_p[t], y0 + g.tap_y[t], n, full_bar(s));
+          mbar_wait(empty_bar(s), ((it / CV_STAGES) & 1) ^ 1);
+          mbar_expect_tx(full_bar(s), box_bytes);
+          tma_load_5d(a_base + s * A_BYTES, &tmA, 0, x0 + g.tap_x[t], g.tap_p[t], y0 + g.tap_y[t], n, full_bar(s));
         }
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      cv_mbar_wait(w_bar, 0);
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      mbar_wait(w_bar, 0);
+      constexpr uint32_t idesc = idesc_bf16(128, BN);
       // one thread of scalar code issues every MMA: descriptors are precomputed (weights: per tap and K step; stages:
       // base + stage * size), leaving one 64-bit add per operand per instruction
       uint64_t bdesc[NTAPS * 4];
 #pragma unroll
-      for (int i = 0; i < NTAPS * 4; ++i) bdesc[i] = cv_desc(w_base + (i >> 2) * W_TAP_BYTES + (i & 3) * 32, 16, 1024);
-      const uint64_t adesc0 = cv_desc(a_base, 16, 1024);
+      for (int i = 0; i < NTAPS * 4; ++i) bdesc[i] = smem_desc(w_base + (i >> 2) * W_TAP_BYTES + (i & 3) * 32, 16, 1024);
+      const uint64_t adesc0 = smem_desc(a_base, 16, 1024);
       uint32_t it = 0, lt = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++lt) {
         const uint32_t acc = lt & 1;
-        cv_mbar_wait(tempty_bar(acc), ((lt >> 1) & 1) ^ 1);
-        cv_fence_after();
+        mbar_wait(tempty_bar(acc), ((lt >> 1) & 1) ^ 1);
+        tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * ACC_COLS;
 #pragma unroll
         for (int t = 0; t < NTAPS; ++t, ++it) {
           const int s = it % CV_STAGES;
-          cv_mbar_wait(full_bar(s), (it / CV_STAGES) & 1);
-          cv_fence_after();
+          mbar_wait(full_bar(s), (it / CV_STAGES) & 1);
+          tc_fence_after();
           const uint64_t adesc = adesc0 + (uint64_t)(s * (A_BYTES >> 4));
 #pragma unroll
-          for (int k = 0; k < 4; ++k) cv_mma(tmem_d, adesc + 2 * k, bdesc[t * 4 + k], idesc, (t > 0 || k > 0) ? 1u : 0u);
-          cv_commit(empty_bar(s));
+          for (int k = 0; k < 4; ++k) tc_mma_bf16(tmem_d, adesc + 2 * k, bdesc[t * 4 + k], idesc, (t > 0 || k > 0) ? 1u : 0u);
+          tc_commit(empty_bar(s));
         }
-        cv_commit(tfull_bar(acc));
+        tc_commit(tfull_bar(acc));
       }
     }
   } else {
@@ -259,12 +182,12 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
 #pragma unroll
         for (int j = 0; j < BN / 8; ++j) gate[j] = __ldg(gp + j);
       }
-      cv_mbar_wait(tfull_bar(acc), (lt >> 1) & 1);
-      cv_fence_after();
+      mbar_wait(tfull_bar(acc), (lt >> 1) & 1);
+      tc_fence_after();
 #pragma unroll
       for (int c0 = 0; c0 < BN; c0 += 16) {
         uint32_t rr[16];
-        cv_ld16(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + c0, rr);
+        tc_ld16(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + c0, rr);
         if (!row_ok) continue;
         float v[16];
 #pragma unroll
@@ -303,16 +226,16 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
           cv_st32(ep.out_f32 + opix * BN + c0 + 8, hi);
         }
       }
-      cv_fence_before();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) cv_mbar_arrive(tempty_bar(acc));
+      if (lane == 0) mbar_arrive(tempty_bar(acc));
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -350,53 +273,49 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const uint32_t stage_bytes = ((uint32_t)g.load_rows * 128 + 1023) & ~1023u;
-  const uint32_t w_base = cv_smem(smem);
+  const uint32_t w_base = smem_u32(smem);
   const uint32_t a_base = w_base + g.ntaps * W_TAP_BYTES;
   uint64_t* bars = (uint64_t*)(smem + g.ntaps * W_TAP_BYTES + g.stages * stage_bytes);
   const int CL_STAGES = g.stages;
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * CL_MAX_STAGES + 2 * NACC + 1);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + CL_MAX_STAGES + s); };
-  auto tfull_bar = [&](int a) { return cv_smem(bars + 2 * CL_MAX_STAGES + a); };
-  auto tempty_bar = [&](int a) { return cv_smem(bars + 2 * CL_MAX_STAGES + NACC + a); };
-  const uint32_t w_bar = cv_smem(bars + 2 * CL_MAX_STAGES + 2 * NACC);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + CL_MAX_STAGES + s); };
+  auto tfull_bar = [&](int a) { return smem_u32(bars + 2 * CL_MAX_STAGES + a); };
+  auto tempty_bar = [&](int a) { return smem_u32(bars + 2 * CL_MAX_STAGES + NACC + a); };
+  const uint32_t w_bar = smem_u32(bars + 2 * CL_MAX_STAGES + 2 * NACC);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   __shared__ float s_bias[BN];
   if (threadIdx.x < BN) s_bias[threadIdx.x] = ep.bias ? ep.bias[threadIdx.x] : 0.f;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < CL_STAGES; ++s) { cv_mbar_init(full_bar(s), 1); cv_mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < NACC; ++a) { cv_mbar_init(tfull_bar(a), 1); cv_mbar_init(tempty_bar(a), 4); }
-    cv_mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < CL_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int a = 0; a < NACC; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
+    mbar_init(w_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  cv_fence_before();
+  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
-      cv_mbar_expect_tx(w_bar, g.ntaps * W_TAP_BYTES);
-      for (int t = 0; t < g.ntaps; ++t) cv_tma_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * BN, w_bar);
+      mbar_expect_tx(w_bar, g.ntaps * W_TAP_BYTES);
+      for (int t = 0; t < g.ntaps; ++t) tma_load_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * BN, w_bar);
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++it) {
         const int n = tile / g.tiles_per_frame, k = tile - n * g.tiles_per_frame;
         const int s = it % CL_STAGES;
-        cv_mbar_wait(empty_bar(s), ((it / CL_STAGES) & 1) ^ 1);
-        cv_mbar_expect_tx(full_bar(s), (uint32_t)g.load_rows * 128);
-        cv_tma_2d(a_base + s * stage_bytes, &tmA, 0, n * g.frame_rows + k * 128, full_bar(s));
+        mbar_wait(empty_bar(s), ((it / CL_STAGES) & 1) ^ 1);
+        mbar_expect_tx(full_bar(s), (uint32_t)g.load_rows * 128);
+        tma_load_2d(a_base + s * stage_bytes, &tmA, 0, n * g.frame_rows + k * 128, full_bar(s));
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      cv_mbar_wait(w_bar, 0);
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      mbar_wait(w_bar, 0);
+      constexpr uint32_t idesc = idesc_bf16(128, BN);
       // The issue loop is one thread of scalar code: keep it to one 64-bit add per operand per MMA.  Descriptor =
       // (constant high word, start address >> 4 in the low 14 bits); offsets below never carry out of that field
       // (shared memory is < 256 KB = 2^14 x 16 B).
@@ -407,23 +326,23 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
 #pragma unroll
         for (int k = 0; k < KSTEPS; ++k) {
           aoff[t * KSTEPS + k] = ((uint32_t)g.shift[t] * 128 + k * 32) >> 4;
-          bdesc[t * KSTEPS + k] = cv_desc(w_base + t * W_TAP_BYTES + k * 32, 16, 1024);
+          bdesc[t * KSTEPS + k] = smem_desc(w_base + t * W_TAP_BYTES + k * 32, 16, 1024);
         }
-      const uint64_t adesc0 = cv_desc(a_base, 16, 1024);
+      const uint64_t adesc0 = smem_desc(a_base, 16, 1024);
       const uint32_t stage16 = stage_bytes >> 4;
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++it) {
         const uint32_t acc = it % NACC;
         const int s = it % CL_STAGES;
-        cv_mbar_wait(tempty_bar(acc), ((it / NACC) & 1) ^ 1);
-        cv_mbar_wait(full_bar(s), (it / CL_STAGES) & 1);
-        cv_fence_after();
+        mbar_wait(tempty_bar(acc), ((it / NACC) & 1) ^ 1);
+        mbar_wait(full_bar(s), (it / CL_STAGES) & 1);
+        tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * ACC_COLS;
         const uint64_t adesc = adesc0 + (uint64_t)(s * stage16);
 #pragma unroll
-        for (int i = 0; i < NTAPS * KSTEPS; ++i) cv_mma(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
-        cv_commit(empty_bar(s));
-        cv_commit(tfull_bar(acc));
+        for (int i = 0; i < NTAPS * KSTEPS; ++i) tc_mma_bf16(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
+        tc_commit(empty_bar(s));
+        tc_commit(tfull_bar(acc));
       }
     }
   } else {
@@ -442,12 +361,12 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
 #pragma unroll
         for (int j = 0; j < BN / 8; ++j) gate[j] = __ldg(gp + j);
       }
-      cv_mbar_wait(tfull_bar(acc), (lt / NACC) & 1);
-      cv_fence_after();
+      mbar_wait(tfull_bar(acc), (lt / NACC) & 1);
+      tc_fence_after();
 #pragma unroll
       for (int c0 = 0; c0 < BN; c0 += 16) {
         uint32_t rr[16];
-        cv_ld16(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + c0, rr);
+        tc_ld16(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + c0, rr);
         if (!row_ok) continue;
         float v[16];
 #pragma unroll
@@ -486,16 +405,16 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
           cv_st32(ep.out_f32 + opix * BN + c0 + 8, hi);
         }
       }
-      cv_fence_before();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) cv_mbar_arrive(tempty_bar(acc));
+      if (lane == 0) mbar_arrive(tempty_bar(acc));
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -526,53 +445,49 @@ conv_dgrad2_kernel(const __grid_constant__ Dgrad2Geom g, const __grid_constant__
   constexpr uint32_t A_BYTES = 128 * 128, W_TAP_BYTES = 128 * 128, ACC_COLS = 128, TMEM_COLS = 256;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  const uint32_t w_base = cv_smem(smem);
+  const uint32_t w_base = smem_u32(smem);
   const uint32_t a_base = w_base + 4 * W_TAP_BYTES;
   // (one spare tile after the ring: the shifted reads of the halo rows run up to 17 rows past the last stage)
   uint64_t* bars = (uint64_t*)(smem + 4 * W_TAP_BYTES + (DG_STAGES + 1) * A_BYTES);
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * DG_STAGES + 5);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + DG_STAGES + s); };
-  auto tfull_bar = [&](int a) { return cv_smem(bars + 2 * DG_STAGES + a); };
-  auto tempty_bar = [&](int a) { return cv_smem(bars + 2 * DG_STAGES + 2 + a); };
-  const uint32_t w_bar = cv_smem(bars + 2 * DG_STAGES + 4);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + DG_STAGES + s); };
+  auto tfull_bar = [&](int a) { return smem_u32(bars + 2 * DG_STAGES + a); };
+  auto tempty_bar = [&](int a) { return smem_u32(bars + 2 * DG_STAGES + 2 + a); };
+  const uint32_t w_bar = smem_u32(bars + 2 * DG_STAGES + 4);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tiles_per_frame = g.tiles_x * g.tiles_y;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < DG_STAGES; ++s) { cv_mbar_init(full_bar(s), 1); cv_mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < 2; ++a) { cv_mbar_init(tfull_bar(a), 1); cv_mbar_init(tempty_bar(a), 8); }
-    cv_mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < DG_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 8); }
+    mbar_init(w_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  cv_fence_before();
+  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
-      cv_mbar_expect_tx(w_bar, 4 * W_TAP_BYTES);
-      for (int t = 0; t < 4; ++t) cv_tma_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * 128, w_bar);
+      mbar_expect_tx(w_bar, 4 * W_TAP_BYTES);
+      for (int t = 0; t < 4; ++t) tma_load_2d(w_base + t * W_TAP_BYTES, &tmW, 0, t * 128, w_bar);
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++it) {
         const int n = tile / tiles_per_frame, rem = tile - n * tiles_per_frame;
         const int ty = rem / g.tiles_x, tx = rem - ty * g.tiles_x;
         const int s = it % DG_STAGES;
-        cv_mbar_wait(empty_bar(s), ((it / DG_STAGES) & 1) ^ 1);
-        cv_mbar_expect_tx(full_bar(s), A_BYTES);
-        cv_tma_4d(a_base + s * A_BYTES, &tmA, 0, tx * (DG_PW - 1) - 1, ty * (DG_PH - 1) - 1, n, full_bar(s));
+        mbar_wait(empty_bar(s), ((it / DG_STAGES) & 1) ^ 1);
+        mbar_expect_tx(full_bar(s), A_BYTES);
+        tma_load_4d(a_base + s * A_BYTES, &tmA, 0, tx * (DG_PW - 1) - 1, ty * (DG_PH - 1) - 1, n, full_bar(s));
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      cv_mbar_wait(w_bar, 0);
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      mbar_wait(w_bar, 0);
+      constexpr uint32_t idesc = idesc_bf16(128, 128);
       uint32_t aoff[16];
       uint64_t bdesc[16];
 #pragma unroll
@@ -581,22 +496,22 @@ conv_dgrad2_kernel(const __grid_constant__ Dgrad2Geom g, const __grid_constant__
         for (int k = 0; k < 4; ++k) {
           const int j = t >> 1, i = t & 1;
           aoff[t * 4 + k] = (uint32_t)(((1 - j) * DG_PW + (1 - i)) * 128 + k * 32) >> 4;
-          bdesc[t * 4 + k] = cv_desc(w_base + t * W_TAP_BYTES + k * 32, 16, 1024);
+          bdesc[t * 4 + k] = smem_desc(w_base + t * W_TAP_BYTES + k * 32, 16, 1024);
         }
-      const uint64_t adesc0 = cv_desc(a_base, 16, 1024);
+      const uint64_t adesc0 = smem_desc(a_base, 16, 1024);
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < g.num_tiles; tile += gridDim.x, ++it) {
         const uint32_t acc = it & 1;
         const int s = it % DG_STAGES;
-        cv_mbar_wait(tempty_bar(acc), ((it >> 1) & 1) ^ 1);
-        cv_mbar_wait(full_bar(s), (it / DG_STAGES) & 1);
-        cv_fence_after();
+        mbar_wait(tempty_bar(acc), ((it >> 1) & 1) ^ 1);
+        mbar_wait(full_bar(s), (it / DG_STAGES) & 1);
+        tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * ACC_COLS;
         const uint64_t adesc = adesc0 + (uint64_t)(s * (A_BYTES >> 4));
 #pragma unroll
-        for (int i = 0; i < 16; ++i) cv_mma(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
-        cv_commit(empty_bar(s));
-        cv_commit(tfull_bar(acc));
+        for (int i = 0; i < 16; ++i) tc_mma_bf16(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
+        tc_commit(empty_bar(s));
+        tc_commit(tfull_bar(acc));
       }
     }
   } else {
@@ -625,17 +540,17 @@ conv_dgrad2_kernel(const __grid_constant__ Dgrad2Geom g, const __grid_constant__
 #pragma unroll
         for (int j = 0; j < 4; ++j) gate[c2][j] = __ldg(gp + j);
       }
-      cv_mbar_wait(tfull_bar(acc), (lt >> 1) & 1);
-      cv_fence_after();
+      mbar_wait(tfull_bar(acc), (lt >> 1) & 1);
+      tc_fence_after();
 #pragma unroll
       for (int c2 = 0; c2 < 2; ++c2) {
         const int cls = 2 * half + c2;
         const bool ok = okc[c2];
         const long long opix = dpixc[c2];
         uint32_t r2[2][16];                  // both 16-column halves of the class in flight before the one wait
-        cv_ld16_nowait(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + cls * 32, r2[0]);
-        cv_ld16_nowait(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + cls * 32 + 16, r2[1]);
-        cv_ld_wait();
+        tc_ld16_nowait(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + cls * 32, r2[0]);
+        tc_ld16_nowait(tmem_base + acc * ACC_COLS + ((uint32_t)(q * 32) << 16) + cls * 32 + 16, r2[1]);
+        tc_ld_wait();
 #pragma unroll
         for (int c0 = 0; c0 < 32; c0 += 16) {
           const uint32_t (&rr)[16] = r2[c0 / 16];
@@ -663,49 +578,26 @@ conv_dgrad2_kernel(const __grid_constant__ Dgrad2Geom g, const __grid_constant__
           cv_st32(dy1 + opix * 32 + c0, pk);
         }
       }
-      cv_fence_before();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) cv_mbar_arrive(tempty_bar(acc));
+      if (lane == 0) mbar_arrive(tempty_bar(acc));
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*CvEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                               const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                               CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static CvEncodeFn cv_encode_fn() {
-  static CvEncodeFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = (CvEncodeFn)p;
-  }
-  return fn;
-}
-
 // packed weights: [ntaps * BN rows][64] bf16, K-major; one [64][BN] box per tap
 static int cv_weight_tmap(CUtensorMap* tm, const void* wp, int ntaps, int BN) {
-  CvEncodeFn fn = cv_encode_fn();
-  TACORL_REQUIRE(fn, "conv_tc: cuTensorMapEncodeTiled is not available");
   TACORL_REQUIRE(((uintptr_t)wp & 15) == 0, "conv_tc: packed weights must be 16-byte aligned");
-  cuuint64_t dims[2] = {64, (cuuint64_t)ntaps * BN};
-  cuuint64_t strides[1] = {128};
-  cuuint32_t box[2] = {64, (cuuint32_t)BN};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(wp), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_tc: cuTensorMapEncodeTiled(weights) failed (%d)", (int)r);
-  return 0;
+  const cuuint64_t dims[2] = {64, (cuuint64_t)ntaps * BN}, strides[1] = {128};
+  const cuuint32_t box[2] = {64, (cuuint32_t)BN};
+  return encode_tmap_bf16(tm, "conv_tc(weights)", 2, wp, dims, strides, box);
 }
 
 // 5-D view of an NHWC bf16 activation for the patch boxes: (64 channels, x, p, y, n); strides in bytes.
@@ -715,20 +607,12 @@ struct ActView {
   long long sx, sp, sy, sn;
 };
 static int cv_act_tmap(CUtensorMap* tm, const ActView& v, int BW, int BH) {
-  CvEncodeFn fn = cv_encode_fn();
-  TACORL_REQUIRE(fn, "conv_tc: cuTensorMapEncodeTiled is not available");
   TACORL_REQUIRE(((uintptr_t)v.base & 15) == 0 && v.sx % 16 == 0 && v.sp % 16 == 0 && v.sy % 16 == 0 && v.sn % 16 == 0,
                  "conv_tc: activation view must be 16-byte aligned (strides %lld %lld %lld %lld)", v.sx, v.sp, v.sy, v.sn);
-  cuuint64_t dims[5] = {64, (cuuint64_t)v.nx, (cuuint64_t)v.np, (cuuint64_t)v.ny, (cuuint64_t)v.nn};
-  cuuint64_t strides[4] = {(cuuint64_t)v.sx, (cuuint64_t)v.sp, (cuuint64_t)v.sy, (cuuint64_t)v.sn};
-  cuuint32_t box[5] = {64, (cuuint32_t)BW, 1, (cuuint32_t)BH, 1};
-  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(v.base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_tc: cuTensorMapEncodeTiled(activation) failed (%d): dims %lld %lld %lld %lld box %dx%d",
-                 (int)r, v.nx, v.np, v.ny, v.nn, BW, BH);
-  return 0;
+  const cuuint64_t dims[5] = {64, (cuuint64_t)v.nx, (cuuint64_t)v.np, (cuuint64_t)v.ny, (cuuint64_t)v.nn};
+  const cuuint64_t strides[4] = {(cuuint64_t)v.sx, (cuuint64_t)v.sp, (cuuint64_t)v.sy, (cuuint64_t)v.sn};
+  const cuuint32_t box[5] = {64, (cuuint32_t)BW, 1, (cuuint32_t)BH, 1};
+  return encode_tmap_bf16(tm, "conv_tc(activation)", 5, v.base, dims, strides, box);
 }
 
 // patch shape with the fewest wasted accumulator rows: maximise RA*RB / (tiles * 128)
@@ -781,8 +665,6 @@ static int conv_tc_run(ConvGeom g, int N, const ActView& view, int BN, const voi
 // Linear-shift launch: src is an NHWC bf16 activation with 128-byte pixels, frame_rows pixel rows per frame.
 template <int BN, int NTAPS, int KSTEPS>
 static int cl_launch(ConvLinGeom g, int N, const void* src, const void* wpacked, const ConvEpi& ep, cudaStream_t st) {
-  CvEncodeFn fn = cv_encode_fn();
-  TACORL_REQUIRE(fn, "conv_lin: cuTensorMapEncodeTiled is not available");
   int max_shift = 0;
   for (int t = 0; t < g.ntaps; ++t) max_shift = g.shift[t] > max_shift ? g.shift[t] : max_shift;
   g.load_rows = (128 + max_shift + 7) & ~7;
@@ -793,17 +675,10 @@ static int cl_launch(ConvLinGeom g, int N, const void* src, const void* wpacked,
   CUtensorMap tw, ta;
   int rc = cv_weight_tmap(&tw, wpacked, g.ntaps, BN);
   if (rc) return rc;
-  {
-    TACORL_REQUIRE(((uintptr_t)src & 15) == 0, "conv_lin: activation must be 16-byte aligned");
-    cuuint64_t dims[2] = {64, (cuuint64_t)N * g.frame_rows};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)g.load_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(&ta, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(src), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_lin: cuTensorMapEncodeTiled(activation) failed (%d)", (int)r);
-  }
+  TACORL_REQUIRE(((uintptr_t)src & 15) == 0, "conv_lin: activation must be 16-byte aligned");
+  const cuuint64_t dims[2] = {64, (cuuint64_t)N * g.frame_rows}, strides[1] = {128};
+  const cuuint32_t box[2] = {64, (cuuint32_t)g.load_rows};
+  if ((rc = encode_tmap_bf16(&ta, "conv_lin(activation)", 2, src, dims, strides, box))) return rc;
   const size_t stage = ((size_t)g.load_rows * 128 + 1023) & ~(size_t)1023;
   const size_t fixed = (size_t)g.ntaps * BN * 128 + (2 * CL_MAX_STAGES + 12) * 8 + 16 + 1024 + 256;
   g.stages = (int)std::min<size_t>(CL_MAX_STAGES, (227 * 1024 - fixed) / stage);
@@ -865,8 +740,14 @@ __global__ void cv_zero_margin_kernel(uint4* __restrict__ t, int N, int H, int W
 int conv_dgrad2_fused(const void* dy2b, int N, int H1, int W1, int H2, int W2, const void* wp5, const void* y1b, void* dy1b,
                       int out_pad, cudaStream_t st) {
   if (N == 0) return 0;
-  CvEncodeFn fn = cv_encode_fn();
-  TACORL_REQUIRE(fn, "conv_dgrad2: cuTensorMapEncodeTiled is not available");
+  CUtensorMap tw, ta;
+  int rc = cv_weight_tmap(&tw, wp5, 4, 128);
+  if (rc) return rc;
+  TACORL_REQUIRE(((uintptr_t)dy2b & 15) == 0, "conv_dgrad2: dy2 must be 16-byte aligned");
+  const cuuint64_t dims[4] = {64, (cuuint64_t)W2, (cuuint64_t)H2, (cuuint64_t)N};
+  const cuuint64_t strides[3] = {128, (cuuint64_t)W2 * 128, (cuuint64_t)H2 * W2 * 128};
+  const cuuint32_t box[4] = {64, DG_PW, DG_PH, 1};
+  if ((rc = encode_tmap_bf16(&ta, "conv_dgrad2(dy2)", 4, dy2b, dims, strides, box))) return rc;
   Dgrad2Geom g = {};
   g.H1 = H1; g.W1 = W1; g.H2 = H2; g.W2 = W2; g.RA = (H1 + 1) / 2; g.RB = (W1 + 1) / 2;
   g.tiles_x = cdiv(g.RB, DG_PW - 1); g.tiles_y = cdiv(g.RA, DG_PH - 1);
@@ -876,20 +757,6 @@ int conv_dgrad2_fused(const void* dy2b, int N, int H1, int W1, int H2, int W2, c
     const long long total = (long long)N * (H1 * out_pad + out_pad * g.OWp) * 4;
     cv_zero_margin_kernel<<<(int)min((long long)592, (total + 255) / 256), 256, 0, st>>>((uint4*)dy1b, N, H1, W1, g.OHp, g.OWp, 4);
     TACORL_LAUNCH_CHECK();
-  }
-  CUtensorMap tw, ta;
-  int rc = cv_weight_tmap(&tw, wp5, 4, 128);
-  if (rc) return rc;
-  {
-    TACORL_REQUIRE(((uintptr_t)dy2b & 15) == 0, "conv_dgrad2: dy2 must be 16-byte aligned");
-    cuuint64_t dims[4] = {64, (cuuint64_t)W2, (cuuint64_t)H2, (cuuint64_t)N};
-    cuuint64_t strides[3] = {128, (cuuint64_t)W2 * 128, (cuuint64_t)H2 * W2 * 128};
-    cuuint32_t box[4] = {64, DG_PW, DG_PH, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fn(&ta, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(dy2b), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_dgrad2: cuTensorMapEncodeTiled(dy2) failed (%d)", (int)r);
   }
   const size_t smem = 4 * 128 * 128 + (size_t)(DG_STAGES + 1) * 128 * 128 + (2 * DG_STAGES + 5) * 8 + 16 + 1024;
   static bool configured = false;
@@ -1160,7 +1027,6 @@ int conv_tc_conv2_dgrad(const void* dy2b, int N, int H1, int W1, int H2, int W2,
 namespace tacorl {
 
 constexpr int WG_STAGES = 5;
-constexpr int WG_LAG = 3;
 constexpr int WG_PL = 4;              // producer lanes per pixel row (chunks j = c*WG_PL + h: whole 32-byte sectors per warp instruction)
 constexpr int WG_PROD = 64 * WG_PL;   // producer threads; warps 0..3 also drain TMEM at the end
 constexpr int WG_THREADS = WG_PROD + 32;   // + the MMA warp
@@ -1185,14 +1051,14 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_tc_wgrad_kernel(const __gr
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const uint32_t stage_bytes = (1 + g.NT) * TILE;
-  const uint32_t base = cv_smem(smem);
+  const uint32_t base = smem_u32(smem);
   const uint32_t zero_tile = base + WG_STAGES * stage_bytes;
   const uint32_t ones_tile = zero_tile + TILE;          // all-ones B operand: dY^T x 1 = bias gradient
   uint64_t* bars = (uint64_t*)(smem + WG_STAGES * stage_bytes + 2 * TILE);
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * WG_STAGES + 1);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + WG_STAGES + s); };
-  const uint32_t done_bar = cv_smem(bars + 2 * WG_STAGES);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + WG_STAGES + s); };
+  const uint32_t done_bar = smem_u32(bars + 2 * WG_STAGES);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int NCOLS = g.NT * 64;
   const bool with_bias = g.bias_partial != nullptr && blockIdx.y == 0;
@@ -1212,19 +1078,15 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_tc_wgrad_kernel(const __gr
         make_uint4(0x3F803F80u, 0x3F803F80u, 0x3F803F80u, 0x3F803F80u);          // bf16 1.0 pairs
   }
   if (threadIdx.x == 0) {
-    for (int s = 0; s < WG_STAGES; ++s) { cv_mbar_init(full_bar(s), WG_PROD); cv_mbar_init(empty_bar(s), 1); }
-    cv_mbar_init(done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < WG_STAGES; ++s) { mbar_init(full_bar(s), WG_PROD); mbar_init(empty_bar(s), 1); }
+    mbar_init(done_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == WG_PROD / 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == WG_PROD / 32) tmem_alloc(tmem_slot, tmem_cols);
   cv_fence_async();          // the generic-proxy zero fill must be visible to the tensor core (async proxy)
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp < WG_PROD / 32) {
@@ -1234,7 +1096,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_tc_wgrad_kernel(const __gr
     for (int i = 0; i < nkb; ++i) {
       const int s = i % WG_STAGES;
       const uint32_t ph = (i / WG_STAGES) & 1;
-      cv_mbar_wait(empty_bar(s), ph ^ 1);
+      mbar_wait(empty_bar(s), ph ^ 1);
       const uint32_t st = base + s * stage_bytes;
       const int m = m_begin + i * 64 + p;
       const bool ok = m < m_end;
@@ -1261,42 +1123,39 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_tc_wgrad_kernel(const __gr
     }
   } else if (warp == WG_PROD / 32) {
     if (lane == 0 && nkb > 0) {
-      // A and B MN-major (bits 15, 16), D = f32, bf16 inputs, M = 128, N = NT*64
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
-                             ((uint32_t)(NCOLS >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-      const uint32_t idesc_b = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
-                               ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      const uint32_t idesc = idesc_bf16(128, NCOLS, true, true);
+      constexpr uint32_t idesc_b = idesc_bf16(128, 16, true, true);
       for (int i = 0; i < nkb; ++i) {
         const int s = i % WG_STAGES;
         const uint32_t ph = (i / WG_STAGES) & 1;
-        cv_mbar_wait(full_bar(s), ph);
+        mbar_wait(full_bar(s), ph);
         cv_fence_async();
-        cv_fence_after();
+        tc_fence_after();
         const uint32_t a_src = base + s * stage_bytes, b_src = a_src + TILE;
 #pragma unroll
         for (int k = 0; k < 4; ++k)     // 16 pixel rows (2048 B) per UMMA K step
-          cv_mma(tmem_base, cv_desc(a_src + k * 2048, zero_tile - a_src, 1024), cv_desc(b_src + k * 2048, TILE, 1024),
-                 idesc, (i > 0 || k > 0) ? 1u : 0u);
+          tc_mma_bf16(tmem_base, smem_desc(a_src + k * 2048, zero_tile - a_src, 1024), smem_desc(b_src + k * 2048, TILE, 1024),
+                      idesc, (i > 0 || k > 0) ? 1u : 0u);
         if (with_bias) {
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            cv_mma(tmem_base + NCOLS, cv_desc(a_src + k * 2048, zero_tile - a_src, 1024), cv_desc(ones_tile, TILE, 1024),
-                   idesc_b, (i > 0 || k > 0) ? 1u : 0u);
+            tc_mma_bf16(tmem_base + NCOLS, smem_desc(a_src + k * 2048, zero_tile - a_src, 1024),
+                        smem_desc(ones_tile, TILE, 1024), idesc_b, (i > 0 || k > 0) ? 1u : 0u);
         }
-        cv_commit(empty_bar(s));
+        tc_commit(empty_bar(s));
       }
-      cv_commit(done_bar);
+      tc_commit(done_bar);
     }
   }
   if (warp < 4) {   // the producer warps drain the accumulator: TMEM lane quarter = warp index
     const int q = warp;
     const int oc = q * 32 + lane;
-    if (nkb > 0) { cv_mbar_wait(done_bar, 0); cv_fence_after(); }
+    if (nkb > 0) { mbar_wait(done_bar, 0); tc_fence_after(); }
     float* P = g.partial + (((long long)blockIdx.x * g.groups + grp) * g.OC + oc) * NCOLS;
     if (q * 32 < g.OC) {
       for (int c0 = 0; c0 < NCOLS; c0 += 16) {
         uint32_t r[16];
-        if (nkb > 0) cv_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
+        if (nkb > 0) tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
         else {
 #pragma unroll
           for (int j = 0; j < 16; ++j) r[j] = 0;
@@ -1310,17 +1169,17 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_tc_wgrad_kernel(const __gr
       }
       if (with_bias) {
         uint32_t r[16];
-        if (nkb > 0) cv_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + NCOLS, r);
+        if (nkb > 0) tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + NCOLS, r);
         else r[0] = 0;
         if (oc < g.OC) g.bias_partial[(long long)blockIdx.x * g.OC + oc] = __uint_as_float(r[0]);
       }
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == WG_PROD / 32) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, tmem_cols);
   }
 }
 
@@ -1448,14 +1307,14 @@ conv_wgrad_lin_kernel(const __grid_constant__ WgradLinGeom g, const __grid_const
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const uint32_t src_bytes = (uint32_t)g.src_rows * 128, dy_bytes = (uint32_t)g.dy_rows * 128;   // multiples of 1024
   const uint32_t stage_bytes = src_bytes + dy_bytes;
-  const uint32_t base = cv_smem(smem);
+  const uint32_t base = smem_u32(smem);
   const int WL_STAGES = g.stages;
   const uint32_t ones_tile = base + WL_STAGES * stage_bytes;       // 16 K rows x 128 B of bf16 1.0 (N = 16 uses 32 B of each)
   uint64_t* bars = (uint64_t*)(smem + WL_STAGES * stage_bytes + 2048);
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * WL_MAX_STAGES + 1);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + WL_MAX_STAGES + s); };
-  const uint32_t done_bar = cv_smem(bars + 2 * WL_MAX_STAGES);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + WL_MAX_STAGES + s); };
+  const uint32_t done_bar = smem_u32(bars + 2 * WL_MAX_STAGES);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int kb_begin = blockIdx.x * g.kb_per_cta;
   const int kb_end = min(g.nkb, kb_begin + g.kb_per_cta);
@@ -1464,68 +1323,61 @@ conv_wgrad_lin_kernel(const __grid_constant__ WgradLinGeom g, const __grid_const
   for (int i = threadIdx.x; i < 2048 / 16; i += blockDim.x)
     reinterpret_cast<uint4*>(smem + WL_STAGES * stage_bytes)[i] = make_uint4(0x3F803F80u, 0x3F803F80u, 0x3F803F80u, 0x3F803F80u);
   if (threadIdx.x == 0) {
-    for (int s = 0; s < WL_STAGES; ++s) { cv_mbar_init(full_bar(s), 1); cv_mbar_init(empty_bar(s), 1); }
-    cv_mbar_init(done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < WL_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    mbar_init(done_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, 512);
   cv_fence_async();          // the generic-proxy fill of the ones tile must be visible to the tensor core
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
       for (int i = 0; i < nkb; ++i) {
         const int s = i % WL_STAGES;
-        cv_mbar_wait(empty_bar(s), ((i / WL_STAGES) & 1) ^ 1);
+        mbar_wait(empty_bar(s), ((i / WL_STAGES) & 1) ^ 1);
         const uint32_t st = base + s * stage_bytes;
         const int row0 = (kb_begin + i) * WL_KB;                   // source window starts at pixel row p0 + W = row0
-        cv_mbar_expect_tx(full_bar(s), src_bytes + dy_bytes);
-        cv_tma_2d(st, &tmS, 0, row0, full_bar(s));                 // rows outside the tensor arrive as zeros
-        cv_tma_2d(st + src_bytes, &tmD, 0, row0 - g.W, full_bar(s));
+        mbar_expect_tx(full_bar(s), src_bytes + dy_bytes);
+        tma_load_2d(st, &tmS, 0, row0, full_bar(s));                 // rows outside the tensor arrive as zeros
+        tma_load_2d(st + src_bytes, &tmD, 0, row0 - g.W, full_bar(s));
       }
     }
   } else if (warp == 1) {
     if (lane == 0 && nkb > 0) {
-      // A and B MN-major (bits 15, 16), D = f32, bf16 inputs, M = 128
-      const uint32_t idesc_hi = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(128 >> 4) << 24);
-      const uint32_t idesc = idesc_hi | ((uint32_t)(192 >> 3) << 17);
-      const uint32_t idesc_b = idesc_hi | ((uint32_t)(16 >> 3) << 17);
-      const uint64_t ones_desc = cv_desc(ones_tile, 128, 1024);
+      constexpr uint32_t idesc = idesc_bf16(128, 192, true, true), idesc_b = idesc_bf16(128, 16, true, true);
+      const uint64_t ones_desc = smem_desc(ones_tile, 128, 1024);
       const uint32_t wrow = (uint32_t)g.W * 128;
-      const uint64_t b0 = cv_desc(base, 128, 1024);                       // N-atom stride: one pixel row
-      const uint64_t a0 = cv_desc(base + src_bytes, wrow, 1024);          // M-atom stride: one image row
+      const uint64_t b0 = smem_desc(base, 128, 1024);                       // N-atom stride: one pixel row
+      const uint64_t a0 = smem_desc(base + src_bytes, wrow, 1024);          // M-atom stride: one image row
       for (int i = 0; i < nkb; ++i) {
         const int s = i % WL_STAGES;
-        cv_mbar_wait(full_bar(s), (i / WL_STAGES) & 1);
-        cv_fence_after();
+        mbar_wait(full_bar(s), (i / WL_STAGES) & 1);
+        tc_fence_after();
         const uint64_t so = (uint64_t)((s * stage_bytes) >> 4);
 #pragma unroll
         for (int k = 0; k < WL_KB / 16; ++k) {      // 16 pixel rows (2048 B) per UMMA K step
           const uint32_t acc = (i > 0 || k > 0) ? 1u : 0u;
           const uint64_t ad = a0 + so + (uint64_t)(k * 128), bd = b0 + so + (uint64_t)(k * 128);
-          cv_mma(tmem_base, ad, bd, idesc, acc);
-          cv_mma(tmem_base + 192, ad, bd + (uint64_t)(wrow >> 4), idesc, acc);
-          cv_mma(tmem_base + 384, ad, ones_desc, idesc_b, acc);
+          tc_mma_bf16(tmem_base, ad, bd, idesc, acc);
+          tc_mma_bf16(tmem_base + 192, ad, bd + (uint64_t)(wrow >> 4), idesc, acc);
+          tc_mma_bf16(tmem_base + 384, ad, ones_desc, idesc_b, acc);
         }
-        cv_commit(empty_bar(s));
+        tc_commit(empty_bar(s));
       }
-      cv_commit(done_bar);
+      tc_commit(done_bar);
     }
   } else {
     const int q = warp & 3;                     // TMEM lane quarter this warp may read
-    if (nkb > 0) { cv_mbar_wait(done_bar, 0); cv_fence_after(); }
+    if (nkb > 0) { mbar_wait(done_bar, 0); tc_fence_after(); }
     float* P = g.partial + ((long long)blockIdx.x * 128 + (q * 32 + lane)) * WL_COLS;
 #pragma unroll 1
     for (int c0 = 0; c0 < WL_COLS; c0 += 16) {
       uint32_t r[16];
-      if (nkb > 0) cv_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
+      if (nkb > 0) tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
       else {
 #pragma unroll
         for (int x = 0; x < 16; ++x) r[x] = 0;
@@ -1536,11 +1388,11 @@ conv_wgrad_lin_kernel(const __grid_constant__ WgradLinGeom g, const __grid_const
                                                            __uint_as_float(r[4 * x + 2]), __uint_as_float(r[4 * x + 3]));
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 512);
   }
 }
 
@@ -1575,15 +1427,6 @@ __global__ void conv_wgrad_lin_reduce3_kernel(int ctas, const float* __restrict_
 //   A = source rows, M = 128 = the taps dx = 0, 1 (M-atom stride = 1 pixel row);
 //   B = dY rows,     N = 64 = two kernel rows: N-atom 0 = dY[p], N-atom 1 = dY[p + W] (stride = W pixel rows of 64 B).
 // With A shifted by W, ONE MMA per 16 pixel rows covers all four taps: columns 0-31 = taps dy = 1, columns 32-63 = dy = 0.
-__device__ __forceinline__ uint64_t cv_desc64(uint32_t saddr, uint32_t lbo, uint32_t sbo) {   // 64-byte swizzle
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)4 << 61;
-  return d;
-}
 constexpr int WL1_COLS = 64 + 32;         // accumulator columns: D | bias
 
 __global__ void __launch_bounds__(WL_THREADS, 1)
@@ -1593,14 +1436,14 @@ conv_wgrad_lin1_kernel(const __grid_constant__ WgradLinGeom g, const __grid_cons
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const uint32_t src_bytes = (uint32_t)g.src_rows * 128, dy_bytes = (uint32_t)g.dy_rows * 64;   // multiples of 1024
   const uint32_t stage_bytes = src_bytes + dy_bytes;
-  const uint32_t base = cv_smem(smem);
+  const uint32_t base = smem_u32(smem);
   const int NST = g.stages;
   const uint32_t ones_tile = base + NST * stage_bytes;             // 2 M-atoms x 16 K rows x 128 B of bf16 1.0
   uint64_t* bars = (uint64_t*)(smem + NST * stage_bytes + 4096);
   uint32_t* tmem_slot = (uint32_t*)(bars + 2 * WL_MAX_STAGES + 1);
-  auto full_bar = [&](int s) { return cv_smem(bars + s); };
-  auto empty_bar = [&](int s) { return cv_smem(bars + WL_MAX_STAGES + s); };
-  const uint32_t done_bar = cv_smem(bars + 2 * WL_MAX_STAGES);
+  auto full_bar = [&](int s) { return smem_u32(bars + s); };
+  auto empty_bar = [&](int s) { return smem_u32(bars + WL_MAX_STAGES + s); };
+  const uint32_t done_bar = smem_u32(bars + 2 * WL_MAX_STAGES);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int kb_begin = blockIdx.x * g.kb_per_cta;
   const int kb_end = min(g.nkb, kb_begin + g.kb_per_cta);
@@ -1609,65 +1452,59 @@ conv_wgrad_lin1_kernel(const __grid_constant__ WgradLinGeom g, const __grid_cons
   for (int i = threadIdx.x; i < 4096 / 16; i += blockDim.x)
     reinterpret_cast<uint4*>(smem + NST * stage_bytes)[i] = make_uint4(0x3F803F80u, 0x3F803F80u, 0x3F803F80u, 0x3F803F80u);
   if (threadIdx.x == 0) {
-    for (int s = 0; s < NST; ++s) { cv_mbar_init(full_bar(s), 1); cv_mbar_init(empty_bar(s), 1); }
-    cv_mbar_init(done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < NST; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    mbar_init(done_bar, 1);
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(cv_smem(tmem_slot)), "r"(128) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, 128);
   cv_fence_async();
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
-  cv_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
       for (int i = 0; i < nkb; ++i) {
         const int s = i % NST;
-        cv_mbar_wait(empty_bar(s), ((i / NST) & 1) ^ 1);
+        mbar_wait(empty_bar(s), ((i / NST) & 1) ^ 1);
         const uint32_t st = base + s * stage_bytes;
         const int row0 = (kb_begin + i) * WL_KB;
-        cv_mbar_expect_tx(full_bar(s), src_bytes + dy_bytes);
-        cv_tma_2d(st, &tmS, 0, row0, full_bar(s));
-        cv_tma_2d(st + src_bytes, &tmD, 0, row0 - g.W, full_bar(s));
+        mbar_expect_tx(full_bar(s), src_bytes + dy_bytes);
+        tma_load_2d(st, &tmS, 0, row0, full_bar(s));
+        tma_load_2d(st + src_bytes, &tmD, 0, row0 - g.W, full_bar(s));
       }
     }
   } else if (warp == 1) {
     if (lane == 0 && nkb > 0) {
-      const uint32_t idesc_hi = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(128 >> 4) << 24);
-      const uint32_t idesc = idesc_hi | ((uint32_t)(64 >> 3) << 17);
-      const uint32_t idesc_b = idesc_hi | ((uint32_t)(32 >> 3) << 17);
-      const uint64_t ones_desc = cv_desc(ones_tile, 2048, 1024);
-      const uint64_t a0 = cv_desc(base, 128, 1024);                               // M-atom stride: one pixel row
-      const uint64_t b0 = cv_desc64(base + src_bytes, (uint32_t)g.W * 64, 512);   // N-atom stride: one image row
+      constexpr uint32_t idesc = idesc_bf16(128, 64, true, true), idesc_b = idesc_bf16(128, 32, true, true);
+      const uint64_t ones_desc = smem_desc(ones_tile, 2048, 1024);
+      const uint64_t a0 = smem_desc(base, 128, 1024);                                  // M-atom stride: one pixel row
+      const uint64_t b0 = smem_desc(base + src_bytes, (uint32_t)g.W * 64, 512, UMMA_SW64);   // N-atom stride: one image row
       for (int i = 0; i < nkb; ++i) {
         const int s = i % NST;
-        cv_mbar_wait(full_bar(s), (i / NST) & 1);
-        cv_fence_after();
+        mbar_wait(full_bar(s), (i / NST) & 1);
+        tc_fence_after();
         const uint64_t so = (uint64_t)((s * stage_bytes) >> 4);
 #pragma unroll
         for (int k = 0; k < WL_KB / 16; ++k) {      // 16 pixel rows per UMMA K step: 2048 B of the source, 1024 B of dY
           const uint32_t acc = (i > 0 || k > 0) ? 1u : 0u;
           const uint64_t ad = a0 + so + (uint64_t)(k * 128), bd = b0 + so + (uint64_t)(k * 64);
-          cv_mma(tmem_base, ad, bd, idesc, acc);
-          cv_mma(tmem_base + 64, ones_desc, bd, idesc_b, acc);
+          tc_mma_bf16(tmem_base, ad, bd, idesc, acc);
+          tc_mma_bf16(tmem_base + 64, ones_desc, bd, idesc_b, acc);
         }
-        cv_commit(empty_bar(s));
+        tc_commit(empty_bar(s));
       }
-      cv_commit(done_bar);
+      tc_commit(done_bar);
     }
   } else {
     const int q = warp & 3;
-    if (nkb > 0) { cv_mbar_wait(done_bar, 0); cv_fence_after(); }
+    if (nkb > 0) { mbar_wait(done_bar, 0); tc_fence_after(); }
     float* P = g.partial + ((long long)blockIdx.x * 128 + (q * 32 + lane)) * WL1_COLS;
 #pragma unroll 1
     for (int c0 = 0; c0 < WL1_COLS; c0 += 16) {
       uint32_t r[16];
-      if (nkb > 0) cv_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
+      if (nkb > 0) tc_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, r);
       else {
 #pragma unroll
         for (int x = 0; x < 16; ++x) r[x] = 0;
@@ -1678,11 +1515,11 @@ conv_wgrad_lin1_kernel(const __grid_constant__ WgradLinGeom g, const __grid_cons
                                                            __uint_as_float(r[4 * x + 2]), __uint_as_float(r[4 * x + 3]));
     }
   }
-  cv_fence_before();
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    cv_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128) : "memory");
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 128);
   }
 }
 
@@ -1712,7 +1549,7 @@ __global__ void conv_wgrad_lin_reduce1_kernel(int ctas, const float* __restrict_
 }
 
 bool conv_lin_conv1_wgrad_ok(int Wp) {
-  return cv_encode_fn() != nullptr && ((WL_KB + Wp + 15) & ~15) <= 256;
+  return tmap_encoder_available() && ((WL_KB + Wp + 15) & ~15) <= 256;
 }
 
 // conv1: xs (N, Hp, Wp, 64) bf16 space-to-depth image, dy1p (N, Hp, Wp, 32) bf16 = the gradient w.r.t. conv1's
@@ -1720,8 +1557,7 @@ bool conv_lin_conv1_wgrad_ok(int Wp) {
 int conv_lin_conv1_wgrad(const void* dy1p, const void* xs, int N, int Hp, int Wp, float beta, float* dW, float* db,
                          float* ws, size_t ws_bytes, cudaStream_t st) {
   if (N == 0) return 0;
-  CvEncodeFn fn = cv_encode_fn();
-  if (!fn) return 1;
+  if (!tmap_encoder_available()) return 1;
   WgradLinGeom g = {};
   g.W = Wp;
   g.src_rows = (WL_KB + 1 + 7) & ~7;               // window rows 0 .. 127 + 1 (tap dx = 1)
@@ -1738,27 +1574,14 @@ int conv_lin_conv1_wgrad(const void* dy1p, const void* xs, int N, int Hp, int Wp
   ctas = (g.nkb + g.kb_per_cta - 1) / g.kb_per_cta;
   g.partial = ws;
   CUtensorMap ts, td;
+  int rc;
   TACORL_REQUIRE((((uintptr_t)xs | (uintptr_t)dy1p) & 15) == 0, "conv_lin_wgrad: tensors must be 16-byte aligned");
-  {
-    cuuint64_t dims[2] = {64, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)g.src_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(&ts, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(xs), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_lin_wgrad: cuTensorMapEncodeTiled(source) failed (%d)", (int)r);
-  }
-  {
-    cuuint64_t dims[2] = {32, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {64};
-    cuuint32_t box[2] = {32, (cuuint32_t)g.dy_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(&td, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(dy1p), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_lin_wgrad: cuTensorMapEncodeTiled(gradient) failed (%d)", (int)r);
-  }
+  const cuuint64_t s_dims[2] = {64, (cuuint64_t)rows}, s_strides[1] = {128};
+  const cuuint64_t d_dims[2] = {32, (cuuint64_t)rows}, d_strides[1] = {64};
+  const cuuint32_t s_box[2] = {64, (cuuint32_t)g.src_rows}, d_box[2] = {32, (cuuint32_t)g.dy_rows};
+  if ((rc = encode_tmap_bf16(&ts, "conv_lin_wgrad(source)", 2, xs, s_dims, s_strides, s_box))) return rc;
+  if ((rc = encode_tmap_bf16(&td, "conv_lin_wgrad(gradient)", 2, dy1p, d_dims, d_strides, d_box, CU_TENSOR_MAP_SWIZZLE_64B)))
+    return rc;
   const size_t stage = (size_t)g.src_rows * 128 + (size_t)g.dy_rows * 64;
   const size_t fixed = 4096 + (2 * WL_MAX_STAGES + 1) * 8 + 16 + 1024;
   g.stages = (int)std::min<size_t>(WL_MAX_STAGES, (227 * 1024 - fixed) / stage);
@@ -1777,14 +1600,13 @@ int conv_lin_conv1_wgrad(const void* dy1p, const void* xs, int N, int Hp, int Wp
 }
 
 bool conv_lin_conv3_wgrad_ok(int W2) {
-  return cv_encode_fn() != nullptr && ((WL_KB + W2 + 2 + 7) & ~7) <= 256;
+  return tmap_encoder_available() && ((WL_KB + W2 + 2 + 7) & ~7) <= 256;
 }
 
 int conv_lin_conv3_wgrad(const void* dy3p, const void* y2b, int N, int H2, int W2, float beta, float* dW, float* db,
                          float* ws, size_t ws_bytes, cudaStream_t st) {
   if (N == 0) return 0;
-  CvEncodeFn fn = cv_encode_fn();
-  if (!fn) return 1;
+  if (!tmap_encoder_available()) return 1;
   WgradLinGeom g = {};
   g.W = W2;
   g.src_rows = (WL_KB + W2 + 2 + 7) & ~7;          // window rows 0 .. 127 + W2 + 2 (D1, kx = 2)
@@ -1801,17 +1623,12 @@ int conv_lin_conv3_wgrad(const void* dy3p, const void* y2b, int N, int H2, int W
   ctas = (g.nkb + g.kb_per_cta - 1) / g.kb_per_cta;
   g.partial = ws;
   CUtensorMap ts, td;
+  int rc;
   TACORL_REQUIRE((((uintptr_t)y2b | (uintptr_t)dy3p) & 15) == 0, "conv_lin_wgrad: tensors must be 16-byte aligned");
-  for (int which = 0; which < 2; ++which) {
-    cuuint64_t dims[2] = {64, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)(which == 0 ? g.src_rows : g.dy_rows)};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(which == 0 ? &ts : &td, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                    const_cast<void*>(which == 0 ? y2b : dy3p), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "conv_lin_wgrad: cuTensorMapEncodeTiled failed (%d)", (int)r);
-  }
+  const cuuint64_t dims[2] = {64, (cuuint64_t)rows}, strides[1] = {128};
+  const cuuint32_t s_box[2] = {64, (cuuint32_t)g.src_rows}, d_box[2] = {64, (cuuint32_t)g.dy_rows};
+  if ((rc = encode_tmap_bf16(&ts, "conv_lin_wgrad(source)", 2, y2b, dims, strides, s_box))) return rc;
+  if ((rc = encode_tmap_bf16(&td, "conv_lin_wgrad(gradient)", 2, dy3p, dims, strides, d_box))) return rc;
   const size_t stage = (size_t)(g.src_rows + g.dy_rows) * 128;
   const size_t fixed = 2048 + (2 * WL_MAX_STAGES + 1) * 8 + 16 + 1024;
   g.stages = (int)std::min<size_t>(WL_MAX_STAGES, (227 * 1024 - fixed) / stage);

@@ -1,10 +1,10 @@
-// bf16 tensor-core GEMM for sm_100a: TMA (cp.async.bulk.tensor) -> 128B-swizzled shared memory ->
-// tcgen05.mma (single-thread issue, cta_group::1, UMMA 128 x BN x 16) with the fp32 accumulator in TMEM ->
-// tcgen05.ld epilogue (alpha/beta/bias/activation, fp32 and/or bf16 stores, or split-K partials).
+// bf16 tensor-core GEMM for sm_100a: TMA tensor loads -> 128B-swizzled shared memory ->
+// tcgen05 MMA (single-thread issue, cta_group::1, UMMA 128 x BN x 16) with the fp32 accumulator in TMEM ->
+// TMEM-load epilogue (alpha/beta/bias/activation, fp32 and/or bf16 stores, or split-K partials).
 //
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
 // warps 2..5 = epilogue (TMEM lane quarter = warp_idx % 4).  A kStages-deep mbarrier ring connects
-// producer and issuer; tcgen05.commit releases ring slots and finally signals the epilogue.
+// producer and issuer; tcgen05 commits release ring slots and finally signals the epilogue.
 //
 // Operand layouts: each operand is either K-major ([rows][K], K contiguous; one 64-wide K slab per
 // stage, canonical SW128 K-major atoms, SBO = 1024 B) or MN-major ([K][rows], rows contiguous; 64x64
@@ -12,7 +12,7 @@
 // 64-wide MN groups).  MN-major lets dX = dZ.W and dW = dZ^T.X run on the tensors as stored.
 #include "common.cuh"
 #include "internal.h"
-#include <cuda.h>
+#include "sm100.cuh"
 #include <cuda_bf16.h>
 #include <algorithm>
 
@@ -22,73 +22,6 @@ constexpr int TC_BM = 128;
 constexpr int TC_BK = 64;          // bf16 elements = 128 bytes = one swizzle row
 constexpr int TC_UMMA_K = 16;
 constexpr int TC_THREADS = 192;
-
-// ------------------------------------------------------------------------------------------ PTX helpers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tm, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-      ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tc_ld16_nowait(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tc_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// SM100 shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start>>4 [0,14), LBO>>4 [16,30),
-// SBO>>4 [32,46), version=1 [46,48), layout SWIZZLE_128B=2 [61,64).
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
 
 struct TcEpilogue {
   float alpha, beta;
@@ -100,10 +33,6 @@ struct TcEpilogue {
   float* partial;                       // split-K: raw accumulators [z][M][N]
   const float* gate; long long ldgate;  // optional ReLU gate: output forced to 0 where gate[row][col] <= 0
 };
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 
 // Epilogue math for one 16-column chunk of one output row, with 16-byte vector accesses when the row is
 // aligned and the chunk is fully inside the matrix (scalar guarded accesses otherwise).
@@ -232,13 +161,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -273,10 +198,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   } else if (warp == 1) {
     if (lane == 0 && nkb > 0) {
-      // instruction descriptor: D=f32 [4,6)=1, A=bf16 [7,10)=1, B=bf16 [10,13)=1, a_major bit15, b_major bit16,
-      // N>>3 at [17,23), M>>4 at [24,29)
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((A_MN ? 1u : 0u) << 15) | ((B_MN ? 1u : 0u) << 16) |
-                             ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
+      constexpr uint32_t idesc = idesc_bf16(TC_BM, BN, A_MN, B_MN);
       uint32_t it = 0, lt = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++lt) {
         const uint32_t acc = lt & 1;
@@ -292,8 +214,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k) {
             // K-major: advance 16 elements (32 B) inside the 128 B swizzle row; MN-major: 16 K-rows of 128 B
-            const uint64_t ad = A_MN ? make_smem_desc(a_src + k * 2048, 8192, 1024) : make_smem_desc(a_src + k * 32, 16, 1024);
-            const uint64_t bd = B_MN ? make_smem_desc(b_src + k * 2048, 8192, 1024) : make_smem_desc(b_src + k * 32, 16, 1024);
+            const uint64_t ad = A_MN ? smem_desc(a_src + k * 2048, 8192, 1024) : smem_desc(a_src + k * 32, 16, 1024);
+            const uint64_t bd = B_MN ? smem_desc(b_src + k * 2048, 8192, 1024) : smem_desc(b_src + k * 32, 16, 1024);
             tc_mma_bf16(tmem_d, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u);
           }
           tc_commit(empty_bar(s));          // slot reusable once these MMAs have read it
@@ -335,7 +257,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -422,13 +344,9 @@ skinny_cluster_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
   if (tid == RS_EPI) {
     for (int s = 0; s < kb_per_cta; ++s) mbar_init(smem_u32(bars + s), 1);
     mbar_init(done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == RS_EPI / 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == RS_EPI / 32) tmem_alloc(tmem_slot, tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -444,7 +362,7 @@ skinny_cluster_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
       tma_load_2d(dst + A_TILE, &tmW, k_begin + s * TC_BK, n0, bar);           // NT weight rows (rows >= N zero-filled)
     }
     // UMMA rows Mpad..127 read stale shared memory: those accumulator lanes are never drained
-    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    const uint32_t idesc = idesc_bf16(128, NT);
     RS_STAMP_T(2)
     for (int s = 0; s < kb_per_cta; ++s) {
       mbar_wait(smem_u32(bars + s), 0);
@@ -453,7 +371,7 @@ skinny_cluster_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
       const uint32_t a_src = smem_u32(smem + (size_t)s * STAGE), w_src = a_src + A_TILE;
 #pragma unroll
       for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
-        tc_mma_bf16(tmem_base, make_smem_desc(a_src + k * 32, 16, 1024), make_smem_desc(w_src + k * 32, 16, 1024), idesc,
+        tc_mma_bf16(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
                     (s > 0 || k > 0) ? 1u : 0u);
     }
     tc_commit(done_bar);
@@ -520,7 +438,7 @@ skinny_cluster_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
   RS_STAMP(7)
   if (tid >= RS_EPI) {                      // issuer warp: TMEM is drained; stay for the closing cluster barrier
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
+    tmem_dealloc(tmem_base, tmem_cols);
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.aligned;" ::: "memory");
     return;
@@ -637,11 +555,6 @@ __device__ long long g_seq_prof[16];
 #define SQ_STAMP(i)
 #endif
 
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* tm, int c0, int c1, int c2, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-      ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
 __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
   unsigned v;
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
@@ -684,13 +597,9 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     for (int s = 0; s < kb_per_cta; ++s) mbar_init(smem_u32(bars + s), 1);
     mbar_init(done_bar, 1);
     mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == RS_EPI / 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == RS_EPI / 32) tmem_alloc(tmem_slot, tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -726,7 +635,7 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       if (lane == 0) {
         SQ_STAMP(1)
         if (step == 0) mbar_wait(w_bar, 0);
-        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+        const uint32_t idesc = idesc_bf16(128, NT);
         SQ_STAMP(2)
         for (int s = 0; s < kb_per_cta; ++s) {
           mbar_wait(smem_u32(bars + s), ph);
@@ -735,7 +644,7 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const uint32_t a_src = smem_u32(a_smem + (size_t)s * A_TILE), w_src = smem_u32(w_smem + (size_t)s * W_STAGE);
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
-            tc_mma_bf16(tmem_base, make_smem_desc(a_src + k * 32, 16, 1024), make_smem_desc(w_src + k * 32, 16, 1024), idesc,
+            tc_mma_bf16(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
                         (s > 0 || k > 0) ? 1u : 0u);
         }
         tc_commit(done_bar);
@@ -863,7 +772,7 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   asm volatile("barrier.cluster.wait.aligned;" ::: "memory");
   if (warp == RS_EPI / 32) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
+    tmem_dealloc(tmem_base, tmem_cols);
   }
   rnn_launch_epilogue(tid);
 }
@@ -926,13 +835,9 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     for (int s = 0; s < kb_per_cta; ++s) mbar_init(smem_u32(bars + s), 1);
     mbar_init(done_bar, 1);
     mbar_init(w_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == RS_EPI / 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == RS_EPI / 32) tmem_alloc(tmem_slot, tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -972,7 +877,7 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       if (lane == 0) {
         WV_STAMP(2)
         if (step == 0) mbar_wait(w_bar, 0);
-        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+        const uint32_t idesc = idesc_bf16(128, NT);
         for (int s = 0; s < kb_per_cta; ++s) {
           mbar_wait(smem_u32(bars + s), ph);
           tc_fence_after();
@@ -980,7 +885,7 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           const uint32_t a_src = smem_u32(a_smem + (size_t)s * A_PITCH), w_src = smem_u32(w_smem + (size_t)s * W_STAGE);
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
-            tc_mma_bf16(tmem_base, make_smem_desc(a_src + k * 32, 16, 1024), make_smem_desc(w_src + k * 32, 16, 1024), idesc,
+            tc_mma_bf16(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
                         (s > 0 || k > 0) ? 1u : 0u);
         }
         tc_commit(done_bar);
@@ -1107,7 +1012,7 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   if (sa.n_steps > 0) asm volatile("barrier.cluster.wait.aligned;" ::: "memory");
   if (warp == RS_EPI / 32) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
+    tmem_dealloc(tmem_base, tmem_cols);
   }
   rnn_launch_epilogue(tid);
 }
@@ -1117,7 +1022,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static EncodeTiledFn get_encode_fn() {
+static EncodeTiledFn encode_tiled_fn() {
   static EncodeTiledFn fn = nullptr;
   if (!fn) {
     void* p = nullptr;
@@ -1129,23 +1034,37 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
+bool tmap_encoder_available() { return encode_tiled_fn() != nullptr; }
+
+int encode_tmap_bf16(CUtensorMap* tm, const char* what, int rank, const void* base, const cuuint64_t* dims,
+                     const cuuint64_t* byte_strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle) {
+  EncodeTiledFn fn = encode_tiled_fn();
+  TACORL_REQUIRE(fn, "%s: cuTensorMapEncodeTiled is not available from the driver", what);
+  const cuuint32_t elem_strides[5] = {1, 1, 1, 1, 1};
+  const CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, byte_strides,
+                        box, elem_strides, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char shape[512];
+    int n = 0;
+    for (int i = 0; i < rank; ++i)
+      n += snprintf(shape + n, sizeof(shape) - n, " %llu (box %u)", (unsigned long long)dims[i], box[i]);
+    for (int i = 0; i + 1 < rank; ++i)
+      n += snprintf(shape + n, sizeof(shape) - n, "%s %llu", i ? "" : ", byte strides", (unsigned long long)byte_strides[i]);
+    set_last_error("%s: cuTensorMapEncodeTiled failed (%d): dims%s", what, (int)r, shape);
+    return -1;
+  }
+  return 0;
+}
+
 // 2-D bf16 tensor map: inner dimension `inner` (contiguous), `outer` rows of pitch `ld` elements.
 static int make_tmap(CUtensorMap* tm, const void* base, long long inner, long long outer, long long ld,
                      int box_inner, int box_outer) {
-  EncodeTiledFn fn = get_encode_fn();
-  TACORL_REQUIRE(fn, "gemm_tc: cuTensorMapEncodeTiled is not available from the driver");
   TACORL_REQUIRE(((uintptr_t)base & 15) == 0 && (ld * 2) % 16 == 0,
                  "gemm_tc: TMA operand must be 16-byte aligned with a 16-byte multiple pitch (ld=%lld)", ld);
-  cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)outer};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)box_inner, (cuuint32_t)box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  TACORL_REQUIRE(r == CUDA_SUCCESS, "gemm_tc: cuTensorMapEncodeTiled failed (%d) inner=%lld outer=%lld ld=%lld", (int)r,
-                 inner, outer, ld);
-  return 0;
+  const cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)outer}, strides[1] = {(cuuint64_t)ld * 2};
+  const cuuint32_t box[2] = {(cuuint32_t)box_inner, (cuuint32_t)box_outer};
+  return encode_tmap_bf16(tm, "gemm_tc", 2, base, dims, strides, box);
 }
 
 template <int BN, bool A_MN, bool B_MN>
@@ -1301,19 +1220,11 @@ int rnn_seq_tc(const void* Ab, int T, const void* W, long long ldw, int M, int N
   }
   CUtensorMap ta, tw;
   int rc;
-  {
-    EncodeTiledFn fn = get_encode_fn();
-    TACORL_REQUIRE(fn, "rnn_seq: cuTensorMapEncodeTiled is not available from the driver");
-    TACORL_REQUIRE(((uintptr_t)Ab & 15) == 0, "rnn_seq: hidden-state buffer must be 16-byte aligned");
-    cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)M, (cuuint64_t)T};
-    cuuint64_t strides[2] = {(cuuint64_t)K * 2, (cuuint64_t)M * K * 2};
-    cuuint32_t box[3] = {64, (cuuint32_t)Mpad, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(&ta, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(Ab), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "rnn_seq: cuTensorMapEncodeTiled failed (%d) K=%d M=%d T=%d", (int)r, K, M, T);
-  }
+  TACORL_REQUIRE(((uintptr_t)Ab & 15) == 0, "rnn_seq: hidden-state buffer must be 16-byte aligned");
+  const cuuint64_t a_dims[3] = {(cuuint64_t)K, (cuuint64_t)M, (cuuint64_t)T};
+  const cuuint64_t a_strides[2] = {(cuuint64_t)K * 2, (cuuint64_t)M * K * 2};
+  const cuuint32_t a_box[3] = {64, (cuuint32_t)Mpad, 1};
+  if ((rc = encode_tmap_bf16(&ta, "rnn_seq", 3, Ab, a_dims, a_strides, a_box))) return rc;
   if ((rc = make_tmap(&tw, W, K, N, ldw, 64, NT))) return rc;
   SeqArgs sa;
   sa.n_steps = n_steps; sa.tau0 = tau0; sa.dtau = dtau; sa.beta = beta; sa.C = C; sa.ldc = ldc; sa.c_ts = c_ts;
@@ -1378,21 +1289,15 @@ int rnn_wave_tc(const WaveLaneHost* lanes, int n_lanes, int T, int M, int N, int
     }
     if (max_clusters < tiles * n_lanes) return 1;
   }
-  EncodeTiledFn fn = get_encode_fn();
-  TACORL_REQUIRE(fn, "rnn_wave: cuTensorMapEncodeTiled is not available from the driver");
   CUtensorMap ta[2], tw[2];
   WaveArgs wa;
   int rc;
   for (int l = 0; l < 2; ++l) {
     const WaveLaneHost& h = lanes[l < n_lanes ? l : 0];
-    cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)M, (cuuint64_t)T};
-    cuuint64_t strides[2] = {(cuuint64_t)h.lda * 2, (cuuint64_t)h.a_ts * 2};
-    cuuint32_t box[3] = {64, (cuuint32_t)Mpad, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(&ta[l], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(h.Ab), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    TACORL_REQUIRE(r == CUDA_SUCCESS, "rnn_wave: cuTensorMapEncodeTiled failed (%d) K=%d M=%d T=%d", (int)r, K, M, T);
+    const cuuint64_t a_dims[3] = {(cuuint64_t)K, (cuuint64_t)M, (cuuint64_t)T};
+    const cuuint64_t a_strides[2] = {(cuuint64_t)h.lda * 2, (cuuint64_t)h.a_ts * 2};
+    const cuuint32_t a_box[3] = {64, (cuuint32_t)Mpad, 1};
+    if ((rc = encode_tmap_bf16(&ta[l], "rnn_wave", 3, h.Ab, a_dims, a_strides, a_box))) return rc;
     if ((rc = make_tmap(&tw[l], h.W, K, N, h.ldw, 64, NT))) return rc;
     WaveLane& d = wa.lane[l];
     d.n_steps = l < n_lanes ? h.n_steps : 0; d.tau0 = h.tau0; d.dtau = h.dtau; d.act = h.act; d.beta = h.beta;

@@ -1,6 +1,7 @@
 // Internal (non-ABI) declarations shared between the .cu translation units.
 #pragma once
 #include "common.cuh"
+#include <cuda.h>
 
 namespace tacorl {
 
@@ -29,6 +30,15 @@ int softargmax_bwd_f32(const float* y, int N, int OH, int OW, int C, const float
 // because NCCL holds their SMs takes up to twice as long; leaving those SMs out of the grid costs only their share.
 int persistent_ctas();
 void set_sm_reserve(int n);
+
+// ---- TMA tensor maps of the tensor-core kernels (gemm_tc.cu)
+// Encodes a bf16 tensor map of `rank` dimensions: dims[0] is contiguous, byte_strides[i] is the stride of dimension
+// i + 1, box is the tile one TMA load copies.  No interleave, 256-byte L2 promotion, elements outside the tensor read as
+// zero.  On failure the library error names `what` (kernel and operand) and the shape; the caller checks alignment.
+bool tmap_encoder_available();
+int encode_tmap_bf16(CUtensorMap* tm, const char* what, int rank, const void* base, const cuuint64_t* dims,
+                     const cuuint64_t* byte_strides, const cuuint32_t* box,
+                     CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B);
 
 // ---- bf16 tcgen05 GEMM (gemm_tc.cu)
 struct TcArgs {
