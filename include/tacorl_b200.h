@@ -105,6 +105,18 @@ int tacorl_lmp_encoder_bwd(const void* x, int x_dtype, float x_scale, float x_sh
 int tacorl_conv_tc_debug(int op, const float* in0, const float* in1, const float* Wt, const float* bias, int N,
                          int H, int W, float* out, void* ws, size_t ws_bytes, void* stream);
 
+/* Diagnostic hook for the bf16 tcgen05 GEMM family behind tacorl_gemm* (PREC_BF16): runs the run-time dispatch on bf16
+ * operands already on the device, with no 2^24-multiply-add fp32 cut-off.  A: a_mn ? stored [K][M] : [M][K] (pitch lda),
+ * B: b_mn ? stored [K][N] : [N][K] (pitch ldb), both 16-byte aligned with 16-byte multiple pitches.  Epilogue per output
+ * element: pre = alpha * A.B + beta * C + bias -> Cpre; act; 0 where gate <= 0; -> C (may be NULL) and bf16 Cb (may be
+ * NULL).  split_k: 0 = automatic, else the K splits asked for (cut down to what ws holds).  ws: split-K partials.
+ * route (host int[4]): {0 = tiled kernel, 1 = skinny cluster kernel; tiled BN or skinny NT; z-slices (tiled: K splits
+ * used, skinny: K slabs per cluster); CTAs launched}. */
+int tacorl_gemm_tc_debug(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, int M, int N,
+                         int K, float alpha, float beta, float* C, long long ldc, void* Cb, long long ldcb,
+                         const float* bias, int act, float* Cpre, long long ldpre, int split_k, const float* gate,
+                         long long ldgate, void* ws, size_t ws_bytes, int* route, void* stream);
+
 /* ---- ReLU RNN layer, one direction, time-major (T*B rows): nn.RNN(nonlinearity="relu") at
  * rnn_models.py:5-16 (decoder) and plan_recognition_tanh_net.py:23-31 / plan_recognition_net.py:27-35
  * (BiRNN).  h0 may be NULL (zeros).  reverse: recurrence runs t = T-1 .. T-n_steps.

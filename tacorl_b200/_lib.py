@@ -33,6 +33,8 @@ _SIGS = {
     "tacorl_lmp_encoder_bwd": [_vp, _i, _f, _f, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i,
                                _vp, _vp, _sz, _i, _vp],
     "tacorl_conv_tc_debug": [_i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp],
+    "tacorl_gemm_tc_debug": [_vp, _ll, _i, _vp, _ll, _i, _i, _i, _i, _f, _f, _vp, _ll, _vp, _ll, _vp, _i, _vp, _ll, _i, _vp,
+                             _ll, _vp, _sz, _vp, _vp],
     "tacorl_rnn_layer_ws_bytes": [_i, _i, _i, _i],
     "tacorl_rnn_layer_fwd": [_i, _i, _i, _i, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _ll, _vp, _vp, _vp, _vp, _sz,
                              _i, _vp],

@@ -1069,7 +1069,7 @@ static int make_tmap(CUtensorMap* tm, const void* base, long long inner, long lo
 
 template <int BN, bool A_MN, bool B_MN>
 static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const TcEpilogue& ep, int M, int N, int K,
-                     int splits, cudaStream_t st) {
+                     int splits, cudaStream_t st, int* route) {
   constexpr int kStages = BN >= 128 ? 5 : 6;
   constexpr size_t smem = (size_t)kStages * (TC_BM * TC_BK * 2 + BN * TC_BK * 2) + (2 * kStages + 4) * 8 + 16 + 1024;
   static bool configured = false;
@@ -1086,6 +1086,7 @@ static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const TcEpilo
   dim3 grid(ctas, 1, zs);
   kern<<<grid, TC_THREADS, smem, st>>>(ta, tb, ep, M, N, K, per);
   TACORL_LAUNCH_CHECK();
+  if (route) { route[0] = 0; route[1] = BN; route[2] = zs; route[3] = ctas * zs; }
   return 0;
 }
 
@@ -1111,7 +1112,7 @@ __global__ void tc_splitk_reduce_kernel(int M, int N, int splits, const float* _
 // C[M][N] = epilogue(A[M][K] . W[N][K]^T) for M <= 128 through skinny_cluster_kernel; returns 1 when the shape is
 // outside what the kernel covers (the caller then uses the tiled kernel).
 static int launch_skinny_cluster(const void* A, long long lda, const void* W, long long ldw, int M, int N, int K,
-                                 const TcEpilogue& ep, cudaStream_t st) {
+                                 const TcEpilogue& ep, cudaStream_t st, int* route) {
   if (M < 1 || M > 128 || K % (TC_BK * RS_KS) != 0 || N % 4 != 0) return 1;
   auto al16 = [](const void* p, long long ld, int elt) { return p == nullptr || (((uintptr_t)p & 15) == 0 && (ld * elt) % 16 == 0); };
   if (!al16(ep.C, ep.ldc, 4) || !al16(ep.gate, ep.ldgate, 4) || !al16(ep.Cpre, ep.ldpre, 4) || !al16(ep.bias, 4, 4) ||
@@ -1135,6 +1136,7 @@ static int launch_skinny_cluster(const void* A, long long lda, const void* W, lo
   }
   skinny_cluster_kernel<<<dim3(RS_KS, tiles), RS_THREADS, smem, st>>>(ta, tw, ep, M, Mpad, N, NT, kb);
   TACORL_LAUNCH_CHECK();
+  if (route) { route[0] = 1; route[1] = NT; route[2] = RS_KS; route[3] = RS_KS * tiles; }
   return 0;
 }
 
@@ -1321,7 +1323,7 @@ unsigned rnn_seq_timeouts() {
 // Core entry: bf16 operands already in global memory.
 //   A: a_mn ? stored [K][M] (pitch lda) : stored [M][K];   B: b_mn ? stored [K][N] : stored [N][K].
 int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, int M, int N,
-                 int K, const TcArgs& e, float* ws, size_t ws_bytes, cudaStream_t st) {
+                 int K, const TcArgs& e, float* ws, size_t ws_bytes, cudaStream_t st, int* route) {
   if (M == 0 || N == 0) return 0;
   TACORL_REQUIRE(K > 0, "gemm_tc: K must be positive");
   int BN = N <= 32 ? 32 : (N <= 64 ? 64 : 128);
@@ -1335,7 +1337,7 @@ int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long lon
     ep.alpha = e.alpha; ep.beta = e.beta; ep.C = e.C; ep.ldc = e.ldc; ep.Cb = (__nv_bfloat16*)e.Cb; ep.ldcb = e.ldcb;
     ep.bias = e.bias; ep.act = e.act; ep.Cpre = e.Cpre; ep.ldpre = e.ldpre; ep.partial = nullptr;
     ep.gate = e.gate; ep.ldgate = e.ldgate;
-    rc = launch_skinny_cluster(A, lda, B, ldb, M, N, K, ep, st);
+    rc = launch_skinny_cluster(A, lda, B, ldb, M, N, K, ep, st, route);
     if (rc <= 0) return rc;
   }
   CUtensorMap ta, tb;
@@ -1359,10 +1361,10 @@ int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long lon
   ep.gate = e.gate; ep.ldgate = e.ldgate;
 #define TC_DISPATCH(BNV)                                                                                   \
   if (BN == BNV) {                                                                                         \
-    if (!a_mn && !b_mn) rc = launch_tc<BNV, false, false>(ta, tb, ep, M, N, K, splits, st);                \
-    else if (a_mn && !b_mn) rc = launch_tc<BNV, true, false>(ta, tb, ep, M, N, K, splits, st);             \
-    else if (!a_mn && b_mn) rc = launch_tc<(BNV < 64 ? 64 : BNV), false, true>(ta, tb, ep, M, N, K, splits, st); \
-    else rc = launch_tc<(BNV < 64 ? 64 : BNV), true, true>(ta, tb, ep, M, N, K, splits, st);               \
+    if (!a_mn && !b_mn) rc = launch_tc<BNV, false, false>(ta, tb, ep, M, N, K, splits, st, route);         \
+    else if (a_mn && !b_mn) rc = launch_tc<BNV, true, false>(ta, tb, ep, M, N, K, splits, st, route);      \
+    else if (!a_mn && b_mn) rc = launch_tc<(BNV < 64 ? 64 : BNV), false, true>(ta, tb, ep, M, N, K, splits, st, route); \
+    else rc = launch_tc<(BNV < 64 ? 64 : BNV), true, true>(ta, tb, ep, M, N, K, splits, st, route);        \
   }
   rc = -1;
   TC_DISPATCH(32) TC_DISPATCH(64) TC_DISPATCH(128)
@@ -1454,3 +1456,16 @@ int gemm_tc_from_f32(const GemmArgs& g, float* ws, size_t ws_bytes, cudaStream_t
 }
 
 }  // namespace tacorl
+
+extern "C" int tacorl_gemm_tc_debug(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, int M,
+                                    int N, int K, float alpha, float beta, float* C, long long ldc, void* Cb,
+                                    long long ldcb, const float* bias, int act, float* Cpre, long long ldpre, int split_k,
+                                    const float* gate, long long ldgate, void* ws, size_t ws_bytes, int* route,
+                                    void* stream) {
+  using namespace tacorl;
+  TcArgs e;
+  e.alpha = alpha; e.beta = beta; e.C = C; e.ldc = ldc; e.Cb = Cb; e.ldcb = ldcb; e.bias = bias; e.act = act;
+  e.Cpre = Cpre; e.ldpre = ldpre; e.split_k = split_k; e.gate = gate; e.ldgate = ldgate;
+  if (route) route[0] = route[1] = route[2] = route[3] = -1;
+  return gemm_tc_bf16(A, lda, a_mn, B, ldb, b_mn, M, N, K, e, (float*)ws, ws_bytes, (cudaStream_t)stream, route);
+}

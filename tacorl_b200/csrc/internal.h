@@ -51,9 +51,11 @@ struct TcArgs {
   int split_k = 0;                                // 0 = auto
   const float* gate = nullptr; long long ldgate = 0;   // optional ReLU gate applied to the output
 };
-// bf16 operands in place: a_mn/b_mn = operand stored [K][rows] (rows contiguous) instead of [rows][K]
+// bf16 operands in place: a_mn/b_mn = operand stored [K][rows] (rows contiguous) instead of [rows][K].
+// route (optional, host int[4]) receives the kernel that ran: {0 = tiled, 1 = skinny cluster; tiled BN or skinny NT;
+// z-slices (tiled: K splits used, skinny: the cluster's K slabs); CTAs launched}.
 int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, int M, int N,
-                 int K, const TcArgs& e, float* ws, size_t ws_bytes, cudaStream_t st);
+                 int K, const TcArgs& e, float* ws, size_t ws_bytes, cudaStream_t st, int* route = nullptr);
 // persistent recurrence (gemm_tc.cu): returns 1 if unsupported (caller launches step by step); flags: >= 16 unsigned
 int rnn_seq_tc(const void* Ab, int T, const void* W, long long ldw, int M, int N, int K, int tau0, int dtau, int n_steps,
                float beta, float* C, long long ldc, long long c_ts, const float* gate, long long ldgate, long long gate_ts,
