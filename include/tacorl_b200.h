@@ -170,6 +170,15 @@ int tacorl_rnn_layer2_bwd(int T, int B, int grad_rows, int I, int H, int D, cons
                           const float* out, long long ldo, const void* out_bf16, float* dout, long long lddo,
                           void* dpre_bf16, float* dx, long long lddx, float* const* dw, void* ws, size_t ws_bytes,
                           void* stream);
+/* The weight-gradient half of tacorl_rnn_layer2_bwd (dW_hh, dW_ih and the bias sums into dw), for a call of it made with
+ * every dw entry NULL once that call's recurrence has finished: dout / dpre_bf16 hold dpre.  Nothing on the dependent
+ * chain reads these gradients, so this may run on a second stream beside the next layer's backward, with its own
+ * workspace (tacorl_rnn_layer2_ws_bytes) and max_ctas > 0 capping the GEMMs' persistent grids to the SMs the
+ * concurrent recurrence leaves free (148 - 64 per lane); 0 = every SM.  The results do not depend on max_ctas. */
+int tacorl_rnn_layer2_wgrad(int T, int B, int I, int H, int D, const float* x, long long ldx, const void* x_bf16,
+                            long long ldxb, const int* n_steps, const void* out_bf16, long long ldo, const float* dout,
+                            long long lddo, const void* dpre_bf16, float* const* dw, void* ws, size_t ws_bytes,
+                            int max_ctas, void* stream);
 /* dst (cols x rows, bf16, dense) = transpose of src (rows x cols, fp32, dense) */
 int tacorl_cast_transpose_bf16(const float* src, int rows, int cols, void* dst, void* stream);
 

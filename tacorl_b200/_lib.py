@@ -44,6 +44,7 @@ _SIGS = {
     "tacorl_rnn_layer2_fwd": [_i, _i, _i, _i, _i, _vp, _ll, _vp, _ll, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _sz, _vp],
     "tacorl_rnn_layer2_bwd": [_i, _i, _i, _i, _i, _i, _vp, _ll, _vp, _ll, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _ll, _vp, _vp, _ll,
                               _vp, _vp, _sz, _vp],
+    "tacorl_rnn_layer2_wgrad": [_i, _i, _i, _i, _i, _vp, _ll, _vp, _ll, _vp, _vp, _ll, _vp, _ll, _vp, _vp, _vp, _sz, _i, _vp],
     "tacorl_cast_transpose_bf16": [_vp, _i, _i, _vp, _vp],
     "tacorl_dlm_nll": [_i, _i, _vp, _ll, _vp, _ll, _i, _f, _f, _f, _vp, _vp, _vp, _ll, _vp],
     "tacorl_dlm_sample": [_i, _i, _vp, _ll, _vp, _vp, _vp, _ll, _f, _f, _vp, _vp, _vp, _vp],

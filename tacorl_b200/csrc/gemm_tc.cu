@@ -1069,7 +1069,7 @@ static int make_tmap(CUtensorMap* tm, const void* base, long long inner, long lo
 
 template <int BN, bool A_MN, bool B_MN>
 static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const TcEpilogue& ep, int M, int N, int K,
-                     int splits, cudaStream_t st, int* route) {
+                     int splits, int max_ctas, cudaStream_t st, int* route) {
   constexpr int kStages = BN >= 128 ? 5 : 6;
   constexpr size_t smem = (size_t)kStages * (TC_BM * TC_BK * 2 + BN * TC_BK * 2) + (2 * kStages + 4) * 8 + 16 + 1024;
   static bool configured = false;
@@ -1082,7 +1082,8 @@ static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const TcEpilo
   const int per = cdiv(total_kb, splits);
   const int zs = cdiv(total_kb, per);
   const long long tiles = (long long)cdiv(N, BN) * cdiv(M, TC_BM);
-  const int ctas = (int)min(tiles, (long long)max(1, 148 / zs));   // persistent: ~one CTA per SM in total
+  const int cap = max_ctas > 0 && max_ctas < 148 ? max_ctas : 148;
+  const int ctas = (int)min(tiles, (long long)max(1, cap / zs));   // persistent: ~one CTA per SM in total
   dim3 grid(ctas, 1, zs);
   kern<<<grid, TC_THREADS, smem, st>>>(ta, tb, ep, M, N, K, per);
   TACORL_LAUNCH_CHECK();
@@ -1361,10 +1362,11 @@ int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long lon
   ep.gate = e.gate; ep.ldgate = e.ldgate;
 #define TC_DISPATCH(BNV)                                                                                   \
   if (BN == BNV) {                                                                                         \
-    if (!a_mn && !b_mn) rc = launch_tc<BNV, false, false>(ta, tb, ep, M, N, K, splits, st, route);         \
-    else if (a_mn && !b_mn) rc = launch_tc<BNV, true, false>(ta, tb, ep, M, N, K, splits, st, route);      \
-    else if (!a_mn && b_mn) rc = launch_tc<(BNV < 64 ? 64 : BNV), false, true>(ta, tb, ep, M, N, K, splits, st, route); \
-    else rc = launch_tc<(BNV < 64 ? 64 : BNV), true, true>(ta, tb, ep, M, N, K, splits, st, route);        \
+    if (!a_mn && !b_mn) rc = launch_tc<BNV, false, false>(ta, tb, ep, M, N, K, splits, e.max_ctas, st, route);  \
+    else if (a_mn && !b_mn) rc = launch_tc<BNV, true, false>(ta, tb, ep, M, N, K, splits, e.max_ctas, st, route); \
+    else if (!a_mn && b_mn)                                                                                \
+      rc = launch_tc<(BNV < 64 ? 64 : BNV), false, true>(ta, tb, ep, M, N, K, splits, e.max_ctas, st, route); \
+    else rc = launch_tc<(BNV < 64 ? 64 : BNV), true, true>(ta, tb, ep, M, N, K, splits, e.max_ctas, st, route); \
   }
   rc = -1;
   TC_DISPATCH(32) TC_DISPATCH(64) TC_DISPATCH(128)
@@ -1376,7 +1378,11 @@ int gemm_tc_bf16(const void* A, long long lda, int a_mn, const void* B, long lon
     const int used = cdiv(total_kb, per);
     ep.partial = nullptr;
     long long total = (long long)M * N;
-    tc_splitk_reduce_kernel<<<(int)min((long long)1184, (total + 255) / 256), 256, 0, st>>>(M, N, used, ws, ep);
+    // grid-stride, one thread per element summing the slices in order: the grid size does not change the result.  Its
+    // 64-register CTAs do not fit beside a recurrence CTA's register file, so it keeps to the GEMM's CTA cap too
+    long long rgrid = min((long long)1184, (total + 255) / 256);
+    if (e.max_ctas > 0) rgrid = min(rgrid, (long long)e.max_ctas);
+    tc_splitk_reduce_kernel<<<(int)rgrid, 256, 0, st>>>(M, N, used, ws, ep);
     TACORL_LAUNCH_CHECK();
   }
   return 0;

@@ -50,6 +50,10 @@ struct TcArgs {
   float* Cpre = nullptr; long long ldpre = 0;
   int split_k = 0;                                // 0 = auto
   const float* gate = nullptr; long long ldgate = 0;   // optional ReLU gate applied to the output
+  // tiled kernel: CTAs of the persistent grid (all z-slices together), 0 = one per SM.  Only which CTA computes a tile
+  // changes, not how a tile is summed; split-K counts do not depend on it.  Work issued beside a persistent recurrence
+  // keeps to the SMs that recurrence leaves free (ops.wgrad_cta_cap).
+  int max_ctas = 0;
 };
 // bf16 operands in place: a_mn/b_mn = operand stored [K][rows] (rows contiguous) instead of [rows][K].
 // route (optional, host int[4]) receives the kernel that ran: {0 = tiled, 1 = skinny cluster; tiled BN or skinny NT;

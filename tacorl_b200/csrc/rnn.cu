@@ -474,6 +474,64 @@ static int layer2_fwd_bf16(int T, int B, int I, int H, int D, const float* x, lo
   return 0;
 }
 
+// Weight gradients of one layer2 backward, once its recurrence has written dpre (fp32 in dout, bf16 twin in dpre_bf16):
+// dW_hh = dpre[pairs]^T h[prev], dW_ih = dpre^T x, db_ih = db_hh = column sums of dpre.  Nothing on the dependent chain
+// (the next layer's BPTT) reads them, so tacorl_rnn_layer2_wgrad issues them on a second stream beside that chain; the
+// one-call backward runs the same code on its own stream.  max_ctas caps the GEMMs' persistent grids (TcArgs::max_ctas).
+static int layer2_wgrad_bf16(int T, int B, int I, int H, int D, const float* x, long long ldx, const void* x_bf16,
+                             long long ldxb, const int* n_steps, const void* out_bf16, long long ldo, const float* dout,
+                             long long lddo, const void* dpre_bf16, float* const* dw, void* ws, size_t ws_bytes,
+                             int max_ctas, cudaStream_t st) {
+  const long long Ip = (I + 7) & ~7LL;
+  Arena ar(ws, ws_bytes);
+  int rc;
+  bool need_x = false;
+  for (int d = 0; d < D; ++d) need_x = need_x || dw[4 * d];
+  const __nv_bfloat16* xb = nullptr; long long ldb_x = 0;
+  const bool x_ready = x_bf16 && ldxb % 8 == 0 && ldxb >= I && ((uintptr_t)x_bf16 & 15) == 0 && (I % 8 == 0);
+  if (x_ready) { xb = (const __nv_bfloat16*)x_bf16; ldb_x = ldxb; }
+  else if (need_x) {
+    __nv_bfloat16* xc = ar.take<__nv_bfloat16>((size_t)T * B * Ip);
+    TACORL_REQUIRE(xc, "rnn_layer2_bwd: workspace too small");
+    if ((rc = cast_bf16_2d(x, ldx, (long long)T * B, I, xc, Ip, st))) return rc;
+    xb = xc; ldb_x = Ip;
+  }
+  float* sk = (float*)(ar.base + ar.off);
+  const size_t sk_bytes = ar.left();
+  const __nv_bfloat16* hb = (const __nv_bfloat16*)out_bf16;
+  const __nv_bfloat16* dpb = (const __nv_bfloat16*)dpre_bf16;
+  for (int d = 0; d < D; ++d) {
+    const int n = n_steps[d], t_lo = d ? T - n : 0;
+    const long long col = (long long)d * H, rows = (long long)n * B;
+    const float* dpre = dout + (long long)t_lo * B * lddo + col;
+    const __nv_bfloat16* dp = dpb + (long long)t_lo * B * lddo + col;
+    float *dw_ih = dw[4 * d], *dw_hh = dw[4 * d + 1], *db_ih = dw[4 * d + 2], *db_hh = dw[4 * d + 3];
+    if (dw_hh) {
+      if (n > 1) {   // dW_hh = dpre[pairs]^T h[prev]: both operands stored [K = rows][H]: MN-major
+        const __nv_bfloat16 *a, *b;
+        if (d == 0) { a = dp + (long long)B * lddo; b = hb + col; }
+        else { a = dp; b = hb + (long long)(t_lo + 1) * B * ldo + col; }
+        TcArgs g;
+        g.C = dw_hh; g.ldc = H; g.split_k = 0; g.max_ctas = max_ctas;
+        if ((rc = gemm_tc_bf16(a, lddo, 1, b, ldo, 1, H, H, (n - 1) * B, g, sk, sk_bytes, st))) return rc;
+      } else {
+        TACORL_CHECK_CUDA(cudaMemsetAsync(dw_hh, 0, (size_t)H * H * 4, st));
+      }
+    }
+    if (dw_ih) {
+      TcArgs g;
+      g.C = dw_ih; g.ldc = I; g.split_k = 0; g.max_ctas = max_ctas;
+      if ((rc = gemm_tc_bf16(dp, lddo, 1, xb + (long long)t_lo * B * ldb_x, ldb_x, 1, H, I, (int)rows, g, sk, sk_bytes, st))) return rc;
+    }
+    if (db_ih || db_hh) {   // db_ih == db_hh == column sums of dpre: reduce once, reuse
+      float* first = db_ih ? db_ih : db_hh;
+      if ((rc = colsum2_f32((int)rows, H, dpre, lddo, first, 0, sk, sk_bytes, st))) return rc;
+      if (db_ih && db_hh) TACORL_CHECK_CUDA(cudaMemcpyAsync(db_hh, db_ih, (size_t)H * 4, cudaMemcpyDeviceToDevice, st));
+    }
+  }
+  return 0;
+}
+
 static int layer2_bwd_bf16(int T, int B, int Bg, int I, int H, int D, const float* x, long long ldx, const void* x_bf16,
                            long long ldxb, const float* const* w, const void* const* w_bf16, const int* n_steps,
                            const float* out, long long ldo, const void* out_bf16, float* dout, long long lddo,
@@ -505,20 +563,10 @@ static int layer2_bwd_bf16(int T, int B, int Bg, int I, int H, int D, const floa
     wih[d] = ih_ready ? (const __nv_bfloat16*)tih : cih;
     whht[d] = ht_ready ? (const __nv_bfloat16*)tht : cht;
   }
-  const bool x_ready = x_bf16 && ldxb % 8 == 0 && ldxb >= I && ((uintptr_t)x_bf16 & 15) == 0 && (I % 8 == 0);
-  const __nv_bfloat16* xb; long long ldb_x;
-  if (x_ready) { xb = (const __nv_bfloat16*)x_bf16; ldb_x = ldxb; }
-  else {
-    __nv_bfloat16* xc = ar.take<__nv_bfloat16>((size_t)T * B * Ip);
-    TACORL_REQUIRE(xc, "rnn_layer2_bwd: workspace too small");
-    if ((rc = cast_bf16_2d(x, ldx, (long long)T * B, I, xc, Ip, st))) return rc;
-    xb = xc; ldb_x = Ip;
-  }
   unsigned* flags = ar.take<unsigned>(128);
   TACORL_REQUIRE(flags, "rnn_layer2_bwd: workspace too small");
   float* sk = (float*)(ar.base + ar.off);
   const size_t sk_bytes = ar.left();
-  const __nv_bfloat16* hb = (const __nv_bfloat16*)out_bf16;
   __nv_bfloat16* dpb = (__nv_bfloat16*)dpre_bf16;
   WaveLaneHost lanes[2];
   int n_lanes = 0;
@@ -567,38 +615,17 @@ static int layer2_bwd_bf16(int T, int B, int Bg, int I, int H, int D, const floa
       }
     }
   }
-  for (int d = 0; d < D; ++d) {
-    const int n = n_steps[d], t_lo = d ? T - n : 0;
-    const long long col = (long long)d * H, rows = (long long)n * B;
-    float* dpre = dout + (long long)t_lo * B * lddo + col;
-    const __nv_bfloat16* dp = dpb + (long long)t_lo * B * lddo + col;
-    float *dw_ih = dw[4 * d], *dw_hh = dw[4 * d + 1], *db_ih = dw[4 * d + 2], *db_hh = dw[4 * d + 3];
-    if (dw_hh) {
-      if (n > 1) {   // dW_hh = dpre[pairs]^T h[prev]: both operands stored [K = rows][H]: MN-major
-        const __nv_bfloat16 *a, *b;
-        if (d == 0) { a = dp + (long long)B * lddo; b = hb + col; }
-        else { a = dp; b = hb + (long long)(t_lo + 1) * B * ldo + col; }
-        TcArgs g;
-        g.C = dw_hh; g.ldc = H; g.split_k = 0;
-        if ((rc = gemm_tc_bf16(a, lddo, 1, b, ldo, 1, H, H, (n - 1) * B, g, sk, sk_bytes, st))) return rc;
-      } else {
-        TACORL_CHECK_CUDA(cudaMemsetAsync(dw_hh, 0, (size_t)H * H * 4, st));
-      }
-    }
-    if (dw_ih) {
-      TcArgs g;
-      g.C = dw_ih; g.ldc = I; g.split_k = 0;
-      if ((rc = gemm_tc_bf16(dp, lddo, 1, xb + (long long)t_lo * B * ldb_x, ldb_x, 1, H, I, (int)rows, g, sk, sk_bytes, st))) return rc;
-    }
-    if (db_ih || db_hh) {   // db_ih == db_hh == column sums of dpre: reduce once, reuse
-      float* first = db_ih ? db_ih : db_hh;
-      if ((rc = colsum2_f32((int)rows, H, dpre, lddo, first, 0, sk, sk_bytes, st))) return rc;
-      if (db_ih && db_hh) TACORL_CHECK_CUDA(cudaMemcpyAsync(db_hh, db_ih, (size_t)H * 4, cudaMemcpyDeviceToDevice, st));
-    }
-    if (dx) {   // dx (+)= dpre_d W_ih_d  (B operand = W_ih as stored [K = H][N = I]: MN-major)
+  if ((rc = layer2_wgrad_bf16(T, B, I, H, D, x, ldx, x_bf16, ldxb, n_steps, out_bf16, ldo, dout, lddo, dpre_bf16, dw, sk,
+                              sk_bytes, 0, st)))
+    return rc;
+  if (dx) {   // dx (+)= dpre_d W_ih_d  (B operand = W_ih as stored [K = H][N = I]: MN-major)
+    for (int d = 0; d < D; ++d) {
+      const int n = n_steps[d], t_lo = d ? T - n : 0;
       TcArgs g;
       g.C = dx + (long long)t_lo * B * lddx; g.ldc = lddx; g.beta = d ? 1.f : 0.f; g.split_k = 1;
-      if ((rc = gemm_tc_bf16(dp, lddo, 0, wih[d], Ip, 1, (int)rows, I, H, g, sk, sk_bytes, st))) return rc;
+      if ((rc = gemm_tc_bf16(dpb + (long long)t_lo * B * lddo + (long long)d * H, lddo, 0, wih[d], Ip, 1, n * B, I, H, g, sk,
+                             sk_bytes, st)))
+        return rc;
     }
   }
   return 0;
@@ -645,6 +672,23 @@ int tacorl_rnn_layer2_bwd(int T, int B, int grad_rows, int I, int H, int D, cons
                           void* stream) {
   return layer2_bwd_bf16(T, B, grad_rows, I, H, D, x, ldx, x_bf16, ldxb, w, w_bf16, n_steps, out, ldo, out_bf16, dout, lddo, dpre_bf16,
                          dx, lddx, dw, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int tacorl_rnn_layer2_wgrad(int T, int B, int I, int H, int D, const float* x, long long ldx, const void* x_bf16,
+                            long long ldxb, const int* n_steps, const void* out_bf16, long long ldo, const float* dout,
+                            long long lddo, const void* dpre_bf16, float* const* dw, void* ws, size_t ws_bytes,
+                            int max_ctas, void* stream) {
+  TACORL_REQUIRE(x && n_steps && out_bf16 && dout && dpre_bf16 && dw && ws, "rnn_layer2_wgrad: null pointer");
+  TACORL_REQUIRE(D == 1 || D == 2, "rnn_layer2_wgrad: D must be 1 or 2");
+  TACORL_REQUIRE(H % 8 == 0 && ldo % 8 == 0 && lddo % 8 == 0 && ((uintptr_t)out_bf16 & 15) == 0 && ((uintptr_t)dpre_bf16 & 15) == 0,
+                 "rnn_layer2_wgrad: pitches must be multiples of 8 and the bf16 twins 16-byte aligned");
+  TACORL_REQUIRE(n_steps[0] == T, "rnn_layer2_wgrad: the forward direction must cover every step");
+  TACORL_REQUIRE(max_ctas >= 0, "rnn_layer2_wgrad: max_ctas must be >= 0");
+  for (int d = 0; d < D; ++d)
+    TACORL_REQUIRE(n_steps[d] >= 1 && n_steps[d] <= T, "rnn_layer2_wgrad: n_steps out of range");
+  if (B == 0) return 0;
+  return layer2_wgrad_bf16(T, B, I, H, D, x, ldx, x_bf16, ldxb, n_steps, out_bf16, ldo, dout, lddo, dpre_bf16, dw, ws,
+                           ws_bytes, max_ctas, (cudaStream_t)stream);
 }
 
 int tacorl_cast_transpose_bf16(const float* src, int rows, int cols, void* dst, void* stream) {

@@ -104,18 +104,23 @@ class PlayLMP(LightningModule):
         self._overlap_grad_sync(emb_states)
         pp_state = self._cat([emb_states[k][:, 0] for k in self.plan_proposal_obs_modalities])
         pp_goal = self._cat([emb_states[k][:, -1] for k in self.plan_proposal_goal_modalities])
-        pp_goal = self.goal_encoder(pp_goal)
-        pp_dist = self.plan_proposal.get_dist(pp_state, pp_goal)
         pr_states = self._cat([emb_states[k] for k in self.plan_recognition_modalities])
         if self.early_subnet_sync and self._sync_active():
             pr_states = pr_states.view_as(pr_states)      # own autograd node: its gradient = "the recogniser's BPTT is done"
             self._sync_when_grad_of(pr_states, [self.plan_recognition])
         pr_dist = self.plan_recognition(pr_states)
+
+        # Goal encoder and plan proposal on a forked stream, so that autograd runs their backward there too: it then waits
+        # only on the KL gradient and runs beside the decoder's BPTT instead of after the recogniser's.  Forked after the
+        # recogniser, whose two-lane layer-0 recurrence leaves no room for the chains' 32 CTAs.
+        def proposal():
+            goal = self.goal_encoder(pp_goal)
+            return goal, self.plan_proposal.get_dist(pp_state, goal)
+        pp_goal, pp_dist = ops.forked(proposal, pp_state.device) if torch.is_grad_enabled() else proposal()
         return emb_states, pp_dist, pr_dist, pp_goal
 
     def compute_loss(self, batch, stage: str = "train"):                          # :221-257
         emb_states, pp_dist, pr_dist, lat_goal = self.process_batch(batch)
-        kl_loss = self.compute_kl_loss(pr_dist=pr_dist, pp_dist=pp_dist, stage=stage)
         ad_states = self._cat([emb_states[k] for k in self.action_decoder_modalities])
         latent_plan = pr_dist.rsample()
         self._sync_when_grad_of(latent_plan, [self.action_decoder])       # decoder BPTT done -> its slice can go
@@ -141,6 +146,9 @@ class PlayLMP(LightningModule):
             for prefix, l_, a_ in (("", action_loss, acc), ("random_plan_", rp_loss, acc_rp)):
                 self.log(f"{stage}/{prefix}action_loss", l_, on_step=True, on_epoch=True, sync_dist=True)
                 self.log(f"{stage}/{prefix}gripper_accuracy", a_, on_step=True, on_epoch=True, sync_dist=True)
+        # after the decoder: autograd orders a pass's backward by creation, latest first, so the KL gradient (all the plan
+        # proposal's backward waits on) is issued before the decoder's BPTT
+        kl_loss = self.compute_kl_loss(pr_dist=pr_dist, pp_dist=pp_dist, stage=stage)
         total_loss = kl_loss + action_loss
         if self.add_random_plan_loss:
             total_loss = total_loss - rp_loss

@@ -42,6 +42,108 @@ def _prep_stream(dev):
     return _SIDE[key]
 
 
+def _wgrad_stream(dev):
+    key = ("wgrad", dev.index if dev.index is not None else torch.cuda.current_device())
+    if key not in _SIDE:
+        _SIDE[key] = torch.cuda.Stream(device=dev)
+    return _SIDE[key]
+
+
+def _plan_stream(dev):
+    key = ("plan", dev.index if dev.index is not None else torch.cuda.current_device())
+    if key not in _SIDE:
+        _SIDE[key] = torch.cuda.Stream(device=dev)
+    return _SIDE[key]
+
+
+def _ws_tag(dev, base="main"):
+    """Scratch buffers are stream-ordered: work on the plan stream (forked) must not share the main stream's."""
+    dev = torch.device(dev)
+    if dev.type != "cuda":
+        return base                                    # (L.workspace refuses it)
+    key = ("plan", dev.index if dev.index is not None else torch.cuda.current_device())
+    side = _SIDE.get(key)
+    return base + "@plan" if side is not None and torch.cuda.current_stream(dev) == side else base
+
+
+def _tensors_in(obj, depth=0):
+    if torch.is_tensor(obj):
+        yield obj
+    elif depth < 3 and isinstance(obj, (tuple, list)):
+        for o in obj:
+            yield from _tensors_in(o, depth + 1)
+    elif depth < 3 and hasattr(obj, "__dict__"):
+        for o in vars(obj).values():
+            yield from _tensors_in(o, depth + 1)
+
+
+def forked(fn, device):
+    """fn() on the plan stream, forked from the current stream and joined back into it; returns fn()'s result.  Autograd
+    runs the backward of what fn() recorded on that stream too, where it waits only on its own input gradients, not on
+    everything issued before it: the backward of a small sub-network that hangs off the loss early (PlayLMP's plan
+    proposal and goal encoder) then runs beside the recurrences of the main chain.  The result's tensors are marked as
+    used by the current stream, so the caching allocator does not hand their memory to later plan-stream work while the
+    current stream may still read them."""
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        return fn()
+    main, side = torch.cuda.current_stream(dev), _plan_stream(dev)
+    side.wait_stream(main)
+    with torch.cuda.stream(side):
+        out = fn()
+    main.wait_stream(side)
+    for t in _tensors_in(out):
+        if t.is_cuda:
+            t.record_stream(main)
+    return out
+
+
+def wgrad_cta_cap(lanes):
+    """CTAs a weight-gradient GEMM issued beside a persistent recurrence of `lanes` lanes may use: each lane holds 64
+    SMs, and a recurrence CTA (~200 KB of shared memory) cannot share an SM with a GEMM CTA (>= 160 KB), so a GEMM that
+    took every SM would keep the recurrence's clusters from becoming resident until its own CTAs retire."""
+    return 148 if lanes <= 0 else max(1, 148 - 64 * lanes)
+
+
+# ---- weight gradients still being computed on the wgrad stream.  ReluRNN2Fn.backward leaves each layer's weight
+# gradients running beside the next layer's BPTT and returns without waiting when they all went into optimiser grad
+# slots; (done event, every buffer that work reads) stays here so that the caching allocator cannot hand those buffers
+# to later work on the main stream.  The backward pass ends by joining them into the caller's stream (a captured graph
+# must end with every side stream joined), and whatever reads the flat gradient before that waits on them first.
+_PENDING = {}                 # device index -> [(event, refs)]
+
+
+def _dev_key(device):
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    return device.index if device.index is not None else torch.cuda.current_device()
+
+
+def wait_pending_grads(stream, device=None):
+    """Make `stream` wait for every pending weight gradient of `device` (the buffers stay held)."""
+    for ev, _ in _PENDING.get(_dev_key(device), ()):
+        stream.wait_event(ev)
+
+
+def join_pending_grads(device=None):
+    """Make the current stream wait for every pending weight gradient of `device` and release what they read."""
+    key = _dev_key(device)
+    pend = _PENDING.pop(key, None)
+    if pend:
+        main = torch.cuda.current_stream(torch.device("cuda", key))
+        for ev, _ in pend:
+            main.wait_event(ev)
+
+
+def _join_all_pending():
+    for key in list(_PENDING):
+        join_pending_grads(torch.device("cuda", key))
+
+
+def _defer_join(device, event, refs):
+    _PENDING.setdefault(_dev_key(device), []).append((event, refs))
+    torch.autograd.Variable._execution_engine.queue_callback(_join_all_pending)    # runs when the backward pass ends
+
+
 def _off(t, elems):
     return ctypes.c_void_p(t.data_ptr() + 4 * elems)
 
@@ -191,7 +293,7 @@ def gemm(A, B, C, transA=False, transB=False, alpha=1.0, beta=0.0, bias=None, ac
     K = A.shape[0] if transA else A.shape[1]
     assert (A.shape[1] if transA else A.shape[0]) == M, (A.shape, C.shape, transA)
     assert (B.shape[0] if transB else B.shape[1]) == N and (B.shape[1] if transB else B.shape[0]) == K
-    ws = L.workspace(_GEMM_WS, C.device)
+    ws = L.workspace(_GEMM_WS, C.device, _ws_tag(C.device))
     L.call("tacorl_gemm_ex", int(transA), int(transB), M, N, K, float(alpha), L.ptr(A), _ld(A), L.ptr(B), _ld(B),
            float(beta), L.ptr(C), _ld(C), L.ptr(bias), int(act), L.ptr(Cpre), _ld(Cpre) if Cpre is not None else 0,
            L.ptr_any(A_bf16), L.ptr_any(B_bf16), ctypes.c_void_p(ws.data_ptr()), ws.numel(),
@@ -320,7 +422,7 @@ class MlpChainFn(Function):
         dx1 = torch.empty_like(x1) if (x1 is not None and need[2]) else None
         nl = len(ctx.spec[1])
         nbytes = L.query("tacorl_mlp_chain_ws_bytes", nl, rows, ctypes.byref(arr))
-        ws = L.workspace(nbytes, x0.device, "mlp_chain")
+        ws = L.workspace(nbytes, x0.device, _ws_tag(x0.device, "mlp_chain"))
         L.call("tacorl_mlp_chain_bwd", nl, rows, ctypes.byref(arr), L.ptr(x0), x0.shape[1], x0.shape[1],
                L.ptr(x1), x1.shape[1] if x1 is not None else 0, x1.shape[1] if x1 is not None else 0,
                L.ptr(z), z.shape[1], L.ptr(d_out), d_out.shape[1], L.ptr(dx0), x0.shape[1],
@@ -643,9 +745,15 @@ class ReluRNN2Fn(Function):
             dbuf[T - 1].copy_(d_out)
         else:
             dbuf = d_out.contiguous().clone()
+        main = torch.cuda.current_stream(dev)
         if prep_done is not None:
-            torch.cuda.current_stream(dev).wait_event(prep_done)
+            main.wait_event(prep_done)
+        # each layer's weight gradients go to the wgrad stream once its recurrence and dx are done: nothing on the chain
+        # reads them, so they run beside the next layer's BPTT (and, after the bottom layer, beside whatever backward
+        # follows), on the SMs that recurrence leaves free
+        side = _wgrad_stream(dev)
         wgrads = [None] * len(weights)
+        refs, all_slots = [x, outs, outbs], True
         for l in range(num_layers - 1, -1, -1):
             inp, inp_b = (x, None) if l == 0 else (outs[l - 1], outbs[l - 1])
             Il = inp.shape[2]
@@ -660,14 +768,34 @@ class ReluRNN2Fn(Function):
                 tw += [shadow_of(wl[4 * d]), whts[l * D + d]]
                 for j in range(4):   # straight into the optimiser's flat gradient when this is the parameter's first use
                     slot = grad_slot_of(wl[4 * d + j])
+                    all_slots = all_slots and slot is not None
                     g.append(slot if slot is not None else torch.empty_like(wl[4 * d + j]))
             nst = [T] + ([1 if (last_only and l == num_layers - 1) else T] if D == 2 else [])
-            ws = L.workspace(L.query("tacorl_rnn_layer2_ws_bytes", T, B, Il, H, D), dev, "main")
+            nbytes = L.query("tacorl_rnn_layer2_ws_bytes", T, B, Il, H, D)
+            ws = L.workspace(nbytes, dev, "main")
             L.call("tacorl_rnn_layer2_bwd", T, B, Bg, Il, H, D, L.ptr(inp), Il, L.ptr_any(inp_b), Il, L.ptr_array(w2),
                    L.ptr_array(tw), L.int_array(nst), L.ptr(outs[l]), D * H, L.ptr_any(outbs[l]), L.ptr(dbuf), D * H,
-                   L.ptr_any(dpb), L.ptr(dx), Il, L.ptr_array(g), ctypes.c_void_p(ws.data_ptr()), ws.numel(), L.stream())
+                   L.ptr_any(dpb), L.ptr(dx), Il, L.ptr_array([None] * (4 * D)), ctypes.c_void_p(ws.data_ptr()),
+                   ws.numel(), L.stream())
+            # the next recurrence: the layer below (every direction runs all T steps), or, below the bottom layer, the
+            # next network's; in this project that is at most one lane (the action decoder hands over to the plan
+            # recogniser's last_only top layer, the recogniser to the vision encoders)
+            cap = wgrad_cta_cap(D if l > 0 else 1)
+            side.wait_stream(main)
+            with torch.cuda.stream(side):
+                wsw = L.workspace(nbytes, dev, "wgrad")
+                L.call("tacorl_rnn_layer2_wgrad", T, B, Il, H, D, L.ptr(inp), Il, L.ptr_any(inp_b), Il, L.int_array(nst),
+                       L.ptr_any(outbs[l]), D * H, L.ptr(dbuf), D * H, L.ptr_any(dpb), L.ptr_array(g),
+                       ctypes.c_void_p(wsw.data_ptr()), wsw.numel(), cap, L.stream())
+            refs += [dbuf, dpb, wsw]
             wgrads[l * D * 4:(l + 1) * D * 4] = g
             dbuf = dx
+        done = torch.cuda.Event()
+        done.record(side)
+        if all_slots:    # the flat gradient is read only after the join (see _defer_join)
+            _defer_join(dev, done, refs)
+        else:            # temporaries autograd accumulates into .grad right after this returns
+            main.wait_event(done)
         return (dbuf if ctx.needs_input_grad[0] else None, None, None, None, None, *wgrads)
 
 

@@ -100,6 +100,7 @@ class FlatAdam(torch.optim.Optimizer):
         lo, hi, e0, e1 = r
         if any(not (hi <= a or b <= lo) for a, b, _, _ in self._ranges + self._pre):
             return
+        ops.join_pending_grads(self.pbuf.flat.device)    # the exchange reads the slice in the current stream's order
         self.gather_grads(lo, hi)
         if self.sm_reserve:
             _lib.lib().tacorl_set_sm_reserve(int(self.sm_reserve))
@@ -122,6 +123,8 @@ class FlatAdam(torch.optim.Optimizer):
         lo, hi, e0, e1 = r
         if any(not (hi <= a or b <= lo) for a, b, _, _ in self._ranges):
             return                                     # (already handled this step)
+        if self.grad_sync is not None:     # the exchange reads the slice in the current stream's order
+            ops.join_pending_grads(self.pbuf.flat.device)
         # sub-runs whose exchange was started earlier (begin_exchange_only): gathered and on the wire already
         pre = sorted(q for q in self._pre if lo <= q[0] and q[1] <= hi)
         self._pre = [q for q in self._pre if q not in pre]
@@ -152,6 +155,7 @@ class FlatAdam(torch.optim.Optimizer):
         stream = self._early_stream
         # the update runs on its own stream (later exchanges must not queue behind it), after the gather ...
         stream.wait_stream(torch.cuda.current_stream(dev))
+        ops.wait_pending_grads(stream, dev)            # ... and after weight gradients still running beside the BPTT
         if first:
             self.step_count += 1
         # ... and, with data parallelism, bucket by bucket behind the all-reduce: the update of bucket i overlaps the
@@ -292,6 +296,8 @@ class FlatAdam(torch.optim.Optimizer):
     @torch.no_grad()
     def step(self, closure=None, gathered=False):
         loss = closure() if closure is not None else None
+        if self.pbuf.flat.is_cuda:
+            ops.join_pending_grads(self.pbuf.flat.device)
         self._slots_taken.clear()
         if self._reserved:                         # the kernels that ran under the overlapped exchange are all launched
             _lib.lib().tacorl_set_sm_reserve(0)
