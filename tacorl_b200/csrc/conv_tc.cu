@@ -134,11 +134,13 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
       }
     }
   } else if (warp == 1) {
-    if (lane == 0) {
+    {
       mbar_wait(w_bar, 0);
       constexpr uint32_t idesc = idesc_bf16(128, BN);
-      // one thread of scalar code issues every MMA: descriptors are precomputed (weights: per tap and K step; stages:
-      // base + stage * size), leaving one 64-bit add per operand per instruction
+      // the whole warp runs the issue loop (warp-uniform descriptors in uniform registers), one elected lane issues; its
+      // lanes wait through every ring phase in order and meet at each elect.sync, so each ring still has one in-order
+      // waiter.  Descriptors are precomputed (weights: per tap and K step; stages: base + stage * size), leaving one 64-bit add
+      // per operand per instruction
       uint64_t bdesc[NTAPS * 4];
 #pragma unroll
       for (int i = 0; i < NTAPS * 4; ++i) bdesc[i] = smem_desc(w_base + (i >> 2) * W_TAP_BYTES + (i & 3) * 32, 16, 1024);
@@ -156,10 +158,10 @@ conv_tc_kernel(const __grid_constant__ ConvGeom g, const __grid_constant__ CUten
           tc_fence_after();
           const uint64_t adesc = adesc0 + (uint64_t)(s * (A_BYTES >> 4));
 #pragma unroll
-          for (int k = 0; k < 4; ++k) tc_mma_bf16(tmem_d, adesc + 2 * k, bdesc[t * 4 + k], idesc, (t > 0 || k > 0) ? 1u : 0u);
-          tc_commit(empty_bar(s));
+          for (int k = 0; k < 4; ++k) tc_mma_bf16_warp(tmem_d, adesc + 2 * k, bdesc[t * 4 + k], idesc, (t > 0 || k > 0) ? 1u : 0u);
+          tc_commit_warp(empty_bar(s));
         }
-        tc_commit(tfull_bar(acc));
+        tc_commit_warp(tfull_bar(acc));
       }
     }
   } else {
@@ -313,10 +315,11 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
       }
     }
   } else if (warp == 1) {
-    if (lane == 0) {
+    {
       mbar_wait(w_bar, 0);
       constexpr uint32_t idesc = idesc_bf16(128, BN);
-      // The issue loop is one thread of scalar code: keep it to one 64-bit add per operand per MMA.  Descriptor =
+      // The issue loop is warp-uniform scalar code (one elected lane issues): keep it to one 64-bit add per operand per
+      // MMA.  Descriptor =
       // (constant high word, start address >> 4 in the low 14 bits); offsets below never carry out of that field
       // (shared memory is < 256 KB = 2^14 x 16 B).
       uint32_t aoff[NTAPS * KSTEPS];
@@ -340,9 +343,9 @@ conv_lin_kernel(const __grid_constant__ ConvLinGeom g, const __grid_constant__ C
         const uint32_t tmem_d = tmem_base + acc * ACC_COLS;
         const uint64_t adesc = adesc0 + (uint64_t)(s * stage16);
 #pragma unroll
-        for (int i = 0; i < NTAPS * KSTEPS; ++i) tc_mma_bf16(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
-        tc_commit(empty_bar(s));
-        tc_commit(tfull_bar(acc));
+        for (int i = 0; i < NTAPS * KSTEPS; ++i) tc_mma_bf16_warp(tmem_d, adesc + aoff[i], bdesc[i], idesc, i > 0 ? 1u : 0u);
+        tc_commit_warp(empty_bar(s));
+        tc_commit_warp(tfull_bar(acc));
       }
     }
   } else {

@@ -197,7 +197,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
     }
   } else if (warp == 1) {
-    if (lane == 0 && nkb > 0) {
+    if (nkb > 0) {            // the whole warp runs the issue loop (warp-uniform descriptors), one elected lane issues
       constexpr uint32_t idesc = idesc_bf16(TC_BM, BN, A_MN, B_MN);
       uint32_t it = 0, lt = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++lt) {
@@ -216,11 +216,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             // K-major: advance 16 elements (32 B) inside the 128 B swizzle row; MN-major: 16 K-rows of 128 B
             const uint64_t ad = A_MN ? smem_desc(a_src + k * 2048, 8192, 1024) : smem_desc(a_src + k * 32, 16, 1024);
             const uint64_t bd = B_MN ? smem_desc(b_src + k * 2048, 8192, 1024) : smem_desc(b_src + k * 32, 16, 1024);
-            tc_mma_bf16(tmem_d, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u);
+            tc_mma_bf16_warp(tmem_d, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u);
           }
-          tc_commit(empty_bar(s));          // slot reusable once these MMAs have read it
+          tc_commit_warp(empty_bar(s));     // slot reusable once these MMAs have read it
         }
-        tc_commit(tfull_bar(acc));          // accumulator complete
+        tc_commit_warp(tfull_bar(acc));     // accumulator complete
       }
     }
   } else {
@@ -632,23 +632,23 @@ rnn_seq_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         tma_load_3d(smem_u32(a_smem + (size_t)lane * A_TILE), &tmA, k0, 0, tau - sa.dtau, bar);
       }
       if (__any_sync(0xffffffffu, bad)) dead = true;
-      if (lane == 0) {
-        SQ_STAMP(1)
+      {                       // the whole warp issues (warp-uniform descriptors), one elected lane per MMA
+        if (lane == 0) { SQ_STAMP(1) }
         if (step == 0) mbar_wait(w_bar, 0);
         const uint32_t idesc = idesc_bf16(128, NT);
-        SQ_STAMP(2)
+        if (lane == 0) { SQ_STAMP(2) }
         for (int s = 0; s < kb_per_cta; ++s) {
           mbar_wait(smem_u32(bars + s), ph);
           tc_fence_after();
-          if (s == 0) { SQ_STAMP(3) }
+          if (s == 0 && lane == 0) { SQ_STAMP(3) }
           const uint32_t a_src = smem_u32(a_smem + (size_t)s * A_TILE), w_src = smem_u32(w_smem + (size_t)s * W_STAGE);
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
-            tc_mma_bf16(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
-                        (s > 0 || k > 0) ? 1u : 0u);
+            tc_mma_bf16_warp(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
+                             (s > 0 || k > 0) ? 1u : 0u);
         }
-        tc_commit(done_bar);
-        SQ_STAMP(4)
+        tc_commit_warp(done_bar);
+        if (lane == 0) { SQ_STAMP(4) }
       }
       __syncwarp();
     } else {
@@ -874,22 +874,22 @@ rnn_wave_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         WV_STAMP(32 + lane)
       }
       if (__any_sync(0xffffffffu, bad)) dead = true;
-      if (lane == 0) {
-        WV_STAMP(2)
+      {                       // the whole warp issues (warp-uniform descriptors), one elected lane per MMA
+        if (lane == 0) { WV_STAMP(2) }
         if (step == 0) mbar_wait(w_bar, 0);
         const uint32_t idesc = idesc_bf16(128, NT);
         for (int s = 0; s < kb_per_cta; ++s) {
           mbar_wait(smem_u32(bars + s), ph);
           tc_fence_after();
-          WV_STAMP(16 + s)
+          if (lane == 0) { WV_STAMP(16 + s) }
           const uint32_t a_src = smem_u32(a_smem + (size_t)s * A_PITCH), w_src = smem_u32(w_smem + (size_t)s * W_STAGE);
 #pragma unroll
           for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
-            tc_mma_bf16(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
-                        (s > 0 || k > 0) ? 1u : 0u);
+            tc_mma_bf16_warp(tmem_base, smem_desc(a_src + k * 32, 16, 1024), smem_desc(w_src + k * 32, 16, 1024), idesc,
+                             (s > 0 || k > 0) ? 1u : 0u);
         }
-        tc_commit(done_bar);
-        WV_STAMP(4)
+        tc_commit_warp(done_bar);
+        if (lane == 0) { WV_STAMP(4) }
       }
       __syncwarp();
     } else {

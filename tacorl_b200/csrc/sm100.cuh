@@ -84,6 +84,24 @@ __device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t adesc, uin
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// The same two for an issue loop run by a whole converged warp instead of one lane: the descriptors are then warp-uniform,
+// so ptxas keeps them in uniform registers, and one elected lane issues.  From a single lane every tcgen05.mma compiles to
+// descriptor moves into uniform registers inside an ELECT / BRA.U.ANY loop, which slows a loop of short MMAs.
+__device__ __forceinline__ void tc_mma_bf16_warp(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                                 uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p, e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "@e tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void tc_commit_warp(uint32_t bar) {
+  asm volatile(
+      "{\n\t.reg .pred e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "@e tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar) : "memory");
+}
 // 16 consecutive fp32 columns of this thread's TMEM lane (taddr = lane << 16 | column); tc_ld16 also waits for them
 __device__ __forceinline__ void tc_ld16_nowait(uint32_t taddr, uint32_t (&r)[16]) {
   asm volatile(
