@@ -456,6 +456,41 @@ int tacorl_rollout_decoder_step(int n, int P, int E, int H, const float* plan, c
 int tacorl_rollout_policy_sample(int n, int A, const float* mean, const float* std, const float* grip_logits,
                                  const int* mask, unsigned long long seed, const int* env_id, long long* t, int advance_t,
                                  float* out, long long ldo, void* stream);
+/* ---- critic-guided plan search of the rollout policy (tacorl_b200/rollout.py PlanSearch, DESIGN.md section 16.2): a
+ * cross-entropy-method search over the pre-tanh latent plan z of n (1..64) environments, K candidates each (a multiple
+ * of 32 in 32..512), scored by min(Q1, Q2) of two MLPQNetwork critics of L SiLU layers of width H (a multiple of 32 in
+ * 32..1024) on (e | tanh z).  One iteration k is sample_l0, hidden for layers 1..L-1, then select; all launches are
+ * graph-capturable.  ws: tacorl_plan_search_ws_bytes(n, K, P, H) bytes, 16-byte aligned, shared by the three calls of
+ * a search (the critics' hidden activations); calls sharing a ws must be stream-ordered.
+ * sample_l0: z (n K, P) row i K + c: candidate c of environment i, z = mu + sigma eps with eps = sqrt(-2 ln(1 - u_a))
+ *   cos(2 pi u_b) from words 0 / 1 of Philox4x32-10 draw 256 + (k K + c) P + d (key (lo32(seed), hi32(seed)), counter
+ *   (lo32(t[i]), hi32(t[i]), env_id[i], draw)), as (w >> 8) 2^-24; candidate (0, 0) of iteration 0 is mu itself.
+ *   mu, sigma (n, P).  Critic j's input is cat(eo_j (n, Do), eg_j (n, Dg), tanh z); W0_j (H, Do + Dg + P), b0_j (H):
+ *   h0 = silu(W0_j[:, :Do + Dg] e_j + b0_j + W0_j[:, Do + Dg:] tanh z), the first part once per environment.
+ *   u_out: NULL or (n K, P, 2) receives (u_a, u_b) of every element.  PREC_BF16 also writes the bf16 copy the next
+ *   layer reads.
+ * hidden: layer `layer` >= 1 of both critics, h = silu(h_prev W^T + b), W (H, H); PREC_BF16: tcgen05 bf16 GEMM reading
+ *   W_bf16 (NULL or not 16-byte aligned: W is cast into ws
+ *   first, one extra launch), PREC_F32: fp32 FFMA.  Split-K is 1 in both.
+ * select: critic j's output Linear(H, 1) (w_out_j (H), b_out_j (1)) on the last hidden layer (fp32), score
+ *   s = min(Q1, Q2) (NaN -> -inf) into scores (n, K); the E best candidates (ties: lower c) refit mu = mean(z_elite),
+ *   sigma = max(population std(z_elite), min_std), fp32 sums in ascending c; best_z (n, P) / best_s (n) keep the best
+ *   candidate of iterations 0..k (ties: the earliest (k, c)); k == 0 starts them.  last = 1: rows whose restart is
+ *   non-zero (all rows when restart is NULL) get plan = tanh(best_z) and plan_value = best_s.
+ * A row's results depend neither on n nor on the other rows. */
+size_t tacorl_plan_search_ws_bytes(int n, int K, int P, int H);
+int tacorl_plan_search_sample_l0(int n, int K, int P, int Do, int Dg, int H, int k, const float* mu, const float* sigma,
+                                 const float* eo1, const float* eg1, const float* W0_1, const float* b0_1,
+                                 const float* eo2, const float* eg2, const float* W0_2, const float* b0_2,
+                                 unsigned long long seed, const int* env_id, const long long* t, float* z,
+                                 float* u_out, void* ws, size_t ws_bytes, int prec, void* stream);
+int tacorl_plan_search_hidden(int n, int K, int H, int layer, const float* W1, const void* W1_bf16, const float* b1,
+                              const float* W2, const void* W2_bf16, const float* b2, void* ws, size_t ws_bytes, int prec,
+                              void* stream);
+int tacorl_plan_search_select(int n, int K, int P, int H, int L, int E, int k, int last, float min_std, const float* z,
+                              const float* w_out1, const float* b_out1, const float* w_out2, const float* b_out2,
+                              float* scores, float* mu, float* sigma, float* best_z, float* best_s, const int* restart,
+                              float* plan, float* plan_value, const void* ws, size_t ws_bytes, void* stream);
 int tacorl_polyak_update(long long n, float* target, const float* source, float tau, void* stream);
 int tacorl_sqnorm(long long n, const float* x, float* out, float* ws, void* stream);
 

@@ -90,6 +90,12 @@ _SIGS = {
     "tacorl_rollout_decoder_step": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp, _f, _f,
                                     _vp, _vp, _vp, _sz, _i, _vp],
     "tacorl_rollout_policy_sample": [_i, _i, _vp, _vp, _vp, _vp, ctypes.c_ulonglong, _vp, _vp, _i, _vp, _ll, _vp],
+    "tacorl_plan_search_ws_bytes": [_i, _i, _i, _i],
+    "tacorl_plan_search_sample_l0": [_i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                     ctypes.c_ulonglong, _vp, _vp, _vp, _vp, _vp, _sz, _i, _vp],
+    "tacorl_plan_search_hidden": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i, _vp],
+    "tacorl_plan_search_select": [_i, _i, _i, _i, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                  _vp, _vp, _vp, _vp, _sz, _vp],
     "tacorl_metrics_accumulate": [_vp, _vp, _vp],
     "tacorl_metrics_record": [_vp, _vp, _i, _vp, _vp, _vp],
     "tacorl_mlp_chain_ws_bytes": [_i, _i, _vp],
@@ -109,6 +115,7 @@ _SIGS = {
 _RESTYPES = {
     "tacorl_lmp_encoder_ws_bytes": _sz, "tacorl_rnn_layer_ws_bytes": _sz, "tacorl_rnn_layer2_ws_bytes": _sz,
     "tacorl_mlp_chain_ws_bytes": _sz, "tacorl_rollout_ws_bytes": _sz,
+    "tacorl_plan_search_ws_bytes": _sz,
     "tacorl_last_error": ctypes.c_char_p, "tacorl_launch_count": ctypes.c_ulonglong,
     "tacorl_rnn_seq_timeouts": ctypes.c_uint,
 }

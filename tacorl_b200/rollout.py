@@ -15,7 +15,11 @@ share the batch, and the decoder step is batch-invariant.  DESIGN.md section 16 
 
 The decoder step is `tacorl_rollout_decoder_step` and sampled plans and flat-CQL actions are drawn by
 `tacorl_rollout_policy_sample` (csrc/rollout.cu); the encoders and the actor run through the same library kernels as
-training.  Nothing here changes the module: `act()`, `clear_hidden_state()` and training are untouched."""
+training.  Nothing here changes the module: `act()`, `clear_hidden_state()` and training are untouched.
+
+A TACO-RL policy built with `plan_search=PlanSearch(...)` replans by a cross-entropy-method search over the latent plan
+scored by the module's twin critics (`tacorl_plan_search_*`, csrc/plan_search.cu, DESIGN.md section 16.2) instead of
+taking the actor's tanh(mean); `policy.plan_value` holds min(Q1, Q2) of each row's current plan."""
 import ctypes
 
 import numpy as np
@@ -96,6 +100,118 @@ def policy_sample(mean, std, logits, mask, seed, env_id, t, out, advance_t=False
     return out
 
 
+class PlanSearch:
+    """Settings of the critic-guided plan search (DESIGN.md section 16.2): `iterations` rounds of `samples` candidate
+    pre-tanh plans per replanning environment, drawn from a diagonal Gaussian that starts at the actor's head and is
+    refitted to the `elites` best candidates by min(Q1, Q2), its std floored at `min_std`.  The plan is tanh of the
+    best candidate of all rounds; candidate 0 of round 0 is the actor's deterministic plan."""
+
+    def __init__(self, samples=128, elites=16, iterations=3, min_std=1e-3):
+        for name, v in (("samples", samples), ("elites", elites), ("iterations", iterations)):
+            if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer)):
+                raise ValueError(f"PlanSearch: {name} must be an integer (got {v!r})")
+        samples, elites, iterations = int(samples), int(elites), int(iterations)
+        if not 32 <= samples <= 512 or samples % 32:
+            raise ValueError(f"PlanSearch: samples must be a multiple of 32 in 32..512 (got {samples})")
+        if not 1 <= elites <= samples:
+            raise ValueError(f"PlanSearch: elites must be in 1..samples = {samples} (got {elites})")
+        if not 1 <= iterations <= 8:
+            raise ValueError(f"PlanSearch: iterations must be in 1..8 (got {iterations})")
+        if (isinstance(min_std, (bool, np.bool_)) or not isinstance(min_std, (int, float, np.integer, np.floating))
+                or not np.isfinite(min_std) or not np.float32(min_std) > 0):
+            raise ValueError(f"PlanSearch: min_std must be a finite number > 0 (got {min_std!r})")
+        self.samples, self.elites, self.iterations, self.min_std = samples, elites, iterations, float(min_std)
+
+    def __repr__(self):
+        return (f"PlanSearch(samples={self.samples}, elites={self.elites}, iterations={self.iterations}, "
+                f"min_std={self.min_std})")
+
+
+def critic_layers(qnet):
+    """The fp32 (W, b) pairs of an MLPQNetwork: its SiLU layers, then the output layer (W (1, H), b (1))."""
+    if not hasattr(qnet, "fc_layers") or not hasattr(qnet, "out"):
+        raise ValueError("the plan search scores plans with MLPQNetwork critics")
+    layers = [(fc.weight.detach(), fc.bias.detach()) for fc in qnet.fc_layers] + [(qnet.out.weight.detach(),
+                                                                                   qnet.out.bias.detach())]
+    H = layers[0][0].shape[0]
+    for W, b in layers[1:-1]:
+        if W.shape != (H, H):
+            raise ValueError(f"the plan search needs equal hidden widths (got {tuple(W.shape)} after width {H})")
+    if layers[-1][0].shape != (1, H):
+        raise ValueError("the critic's output layer must be Linear(hidden, 1)")
+    for W, b in layers:
+        if not (W.is_contiguous() and b.is_contiguous()):
+            raise ValueError("critic weights must be contiguous")
+    return layers
+
+
+class SearchBuffers:
+    """Device buffers of a plan search over n environments and K samples: the workspace of tacorl_plan_search_*, the
+    candidates z (n K, P) and their scores (n, K) of the latest round, the refitted (mu, sigma) (n, P) and the best
+    candidate so far, best_z (n, P) and best_s (n)."""
+
+    def __init__(self, n, K, P, H, device):
+        f32 = dict(device=device, dtype=torch.float32)
+        self.n, self.K, self.P, self.H = n, K, P, H
+        self.ws = torch.empty(int(L.query("tacorl_plan_search_ws_bytes", n, K, P, H)), dtype=torch.uint8, device=device)
+        self.z = torch.empty(n * K, P, **f32)
+        self.scores = torch.empty(n, K, **f32)
+        self.mu, self.sigma, self.best_z = (torch.empty(n, P, **f32) for _ in range(3))
+        self.best_s = torch.empty(n, **f32)
+
+
+def plan_search(critics, eo, eg, mean, std, search, seed, env_id, t, restart, plan, plan_value, bufs, trace=None,
+                uniforms=None):
+    """The critic-guided plan search of n = mean.shape[0] environments in the current precision mode (DESIGN.md
+    section 16.2).  critics: the two MLPQNetworks; eo / eg: per critic its (n, Do) observation and (n, Dg) goal
+    embeddings; mean, std (n, P): the actor's head (ops.gauss_head); restart: None or (n,) int32, rows whose flag is 0
+    keep their plan (n, P) and plan_value (n,).  bufs: SearchBuffers(n, K, P, H).  trace: None or a list that receives,
+    after every round, copies of that round's candidates, scores, refit and best-so-far (tests; not graph-capturable).
+    uniforms: None or a list that receives each round's (n K, P, 2) Philox uniforms (tests)."""
+    n, P = mean.shape
+    K, E, I = search.samples, search.elites, search.iterations
+    q = [critic_layers(c) for c in critics]
+    H, nl = q[0][0][0].shape[0], len(q[0]) - 1
+    if len(q[1]) != len(q[0]) or q[1][0][0].shape != q[0][0][0].shape:
+        raise ValueError("the two critics must have the same shapes")
+    Do, Dg = eo[0].shape[1], eg[0].shape[1]
+    for j in range(2):
+        if eo[j].shape != (n, Do) or eg[j].shape != (n, Dg) or q[j][0][0].shape[1] != Do + Dg + P:
+            raise ValueError(f"plan_search: critic {j + 1} takes {q[j][0][0].shape[1]} inputs, embeddings "
+                             f"{tuple(eo[j].shape)} + {tuple(eg[j].shape)} + plan {P}")
+    if (bufs.n, bufs.K, bufs.P, bufs.H) != (n, K, P, H):
+        raise ValueError("plan_search: buffers of another shape")
+    if env_id.dtype != torch.int32 or t.dtype != torch.int64 or (restart is not None and restart.dtype != torch.int32):
+        raise ValueError("plan_search: env_id and restart are int32, t is int64")
+    eo = [x.contiguous() for x in eo]
+    eg = [x.contiguous() for x in eg]
+    mean, std = mean.contiguous(), std.contiguous()
+    prec = ops._STATE["prec"]
+    sd = ctypes.c_ulonglong(int(seed) & 0xFFFFFFFFFFFFFFFF)
+    ws = ctypes.c_void_p(bufs.ws.data_ptr())
+    (W1, b1), (W2, b2) = q[0][-1], q[1][-1]
+    for k in range(I):
+        mu, sg = (mean, std) if k == 0 else (bufs.mu, bufs.sigma)
+        u = torch.empty(n * K, P, 2, device=mean.device) if uniforms is not None else None
+        L.call("tacorl_plan_search_sample_l0", n, K, P, Do, Dg, H, k, L.ptr(mu), L.ptr(sg),
+               L.ptr(eo[0]), L.ptr(eg[0]), L.ptr(q[0][0][0]), L.ptr(q[0][0][1]),
+               L.ptr(eo[1]), L.ptr(eg[1]), L.ptr(q[1][0][0]), L.ptr(q[1][0][1]),
+               sd, L.ptr_any(env_id), L.ptr_any(t), L.ptr(bufs.z), L.ptr(u), ws, bufs.ws.numel(), prec, L.stream())
+        for l in range(1, nl):
+            (Wa, ba), (Wb, bb) = q[0][l], q[1][l]
+            L.call("tacorl_plan_search_hidden", n, K, H, l, L.ptr(Wa), L.ptr_any(ops.shadow_of(Wa)), L.ptr(ba),
+                   L.ptr(Wb), L.ptr_any(ops.shadow_of(Wb)), L.ptr(bb), ws, bufs.ws.numel(), prec, L.stream())
+        L.call("tacorl_plan_search_select", n, K, P, H, nl, E, k, int(k == I - 1), float(search.min_std),
+               L.ptr(bufs.z), L.ptr(W1), L.ptr(b1), L.ptr(W2), L.ptr(b2), L.ptr(bufs.scores), L.ptr(bufs.mu),
+               L.ptr(bufs.sigma), L.ptr(bufs.best_z), L.ptr(bufs.best_s), L.ptr_any(restart), L.ptr(plan),
+               L.ptr(plan_value), ws, bufs.ws.numel(), L.stream())
+        if uniforms is not None:
+            uniforms.append(u)
+        if trace is not None:
+            trace.append({k2: getattr(bufs, k2).clone() for k2 in ("z", "scores", "mu", "sigma", "best_z", "best_s")})
+    return plan
+
+
 def _module_kind(module):
     """"play_lmp", "cql" (flat CQL: a CQL_Offline without an action decoder) or "tacorl" (everything else, checked as
     a TACO-RL module)."""
@@ -134,6 +250,10 @@ class RolloutPolicy:
     plan proposal reads the same encoder, so each modality is encoded once per step.
     Flat CQL: every step is the actor on cat(encoder(obs), goal embedding): Actor.get_actions(deterministic=True)
     (tanh(mean), argmax gripper), or with deterministic=False a TanhNormal arm and GumbelSoftmax gripper sample.
+    plan_search=PlanSearch(...) (TACO-RL, deterministic=True only): a replanning row's plan comes from a cross-entropy
+    search scored by min(Q1, Q2) of the module's critics, started at the actor's head (DESIGN.md section 16.2);
+    reset / set_goal also cache each critic's goal embedding, the replan step adds one pass of each critic's encoder,
+    and `plan_value` (n,) holds each row's min(Q1, Q2) of its current plan (NaN before its first replan).
 
     Each step is one CUDA-graph replay of one of two graphs, with and without a replan (the replan graph runs the actor
     for every row and keeps the plan of the flagged rows only; flat CQL has one graph); the host picks it from its own
@@ -144,8 +264,16 @@ class RolloutPolicy:
     next step, and a step whose parameters or bf16 shadows moved since the capture (an optimiser built or dropped
     since) captures its graphs again."""
 
-    def __init__(self, module, n_envs, seed=0, env_ids=None, use_graphs=True, deterministic=True):
+    def __init__(self, module, n_envs, seed=0, env_ids=None, use_graphs=True, deterministic=True, plan_search=None):
         kind = _module_kind(module)
+        if plan_search is not None:
+            if not isinstance(plan_search, PlanSearch):
+                raise ValueError(f"plan_search must be a PlanSearch or None (got {type(plan_search).__name__})")
+            if kind != "tacorl" or not all(hasattr(module, a) for a in ("q1", "q2", "actor")):
+                raise ValueError("the plan search needs a TACO-RL module: PlayLMP has no critic and flat CQL no plan")
+            if deterministic is not True:
+                raise ValueError("the plan search replaces the actor's plan: it cannot be combined with "
+                                 "deterministic=False")
         if kind == "tacorl":
             for attr in ("actor", "action_decoder", "perceptual_encoder", "action_decoder_modalities"):
                 if not hasattr(module, attr):
@@ -174,6 +302,7 @@ class RolloutPolicy:
             raise L.TacorlLibraryError("RolloutPolicy runs on a CUDA device (there is no CPU path)")
         self.module, self.n, self.seed, self.device = module, n, int(seed), dev
         self.kind, self.deterministic = kind, deterministic
+        self.search = plan_search
         self.use_graphs = bool(use_graphs)
         # what the step reads: the encoder of the actor's (plan proposal's) input, its goal encoder and policy, and the
         # decoder with its encoder (None for flat CQL)
@@ -216,6 +345,22 @@ class RolloutPolicy:
         self._graphs = {}
         self._pool = None
         self.launches = {}            # (replan, precision) -> library launches recorded in that graph
+        self.plan_value = None
+        self._critics = []
+        if plan_search is not None:
+            self._critics = [module.q1, module.q2]
+            for q in self._critics:
+                critic_layers(q.critic.Q)
+                if not set(q.env_modalities) <= set(self.obs_mods) or not set(q.goal_modalities) <= set(self.goal_mods):
+                    raise ValueError("the critics must read the actor's observation and goal modalities")
+            H = module.q1.critic.Q.fc_layers[0].weight.shape[0]
+            if self.P > 64 or H % 32 or not 32 <= H <= 1024:
+                raise ValueError(f"the plan search covers plans of <= 64 dimensions and critic widths that are "
+                                 f"multiples of 32 in 32..1024 (plan {self.P}, critic {H})")
+            self.plan_value = torch.full((n,), float("nan"), **f32)
+            self.q_goal_emb = [None, None]
+            self._search_bufs = SearchBuffers(n, plan_search.samples, self.P, H, dev)
+            nets = nets + (module.q1, module.q2)
         self._tensors = [x for mod in nets for x in list(mod.parameters()) + list(mod.buffers())]
         self.captures = 0
 
@@ -242,6 +387,14 @@ class RolloutPolicy:
         if self._goal_enc is not None:
             emb = self._goal_enc(emb)
         self.goal_emb[rows] = emb.reshape(len(rows), -1)
+        for j, q in enumerate(self._critics):        # goal_encoder_qj(encoder_qj(goal)), the critics' goal embedding
+            ge = q.encoder.get_state_from_observation(observation=g, modalities=q.goal_modalities).reshape(len(rows), -1)
+            if q.goal_encoder is not None:
+                ge = q.goal_encoder(ge)
+            ge = ge.reshape(len(rows), -1)
+            if self.q_goal_emb[j] is None:
+                self.q_goal_emb[j] = torch.zeros(self.n, ge.shape[1], device=self.device, dtype=torch.float32)
+            self.q_goal_emb[j][rows] = ge
         self._has_goal[rows] = True
         if self._dec is not None:
             self._replan[rows] = 1
@@ -284,7 +437,12 @@ class RolloutPolicy:
                 e = self._embed(self._enc, self.env_mods) if replan else None
             if replan:
                 out = self._net(e, self.goal_emb)
-                if self.deterministic:
+                if self.search is not None:     # the flagged rows' plans and values from the critic-guided search
+                    eo = [self._embed(q.encoder, q.env_modalities) for q in self._critics]
+                    plan_search([q.critic.Q for q in self._critics], eo, self.q_goal_emb, out[0], out[1], self.search,
+                                self.seed, self.env_id, self.t, self.restart, self.plan, self.plan_value,
+                                self._search_bufs)
+                elif self.deterministic:
                     new_plan = torch.tanh(out[0])
                     self.plan.copy_(torch.where(self.restart.unsqueeze(1) != 0, new_plan, self.plan))
                 else:         # the flagged rows' plans, drawn at the t their first decoder step reads
@@ -326,7 +484,7 @@ class RolloutPolicy:
 
     def _capture(self, replan):
         # warm-up on a side stream against copies of the state the step mutates, then restore it
-        state = [x for x in (self.plan, self.hidden, self.t) if x is not None]
+        state = [x for x in (self.plan, self.hidden, self.t, self.plan_value) if x is not None]
         saved = [x.clone() for x in state]
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
